@@ -2,6 +2,7 @@
 """bags/sec of one full adversarial G+D train step (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--precision bf16|tf32x3|tf32|fp32] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): AdvMIL-ABMIL, synthetic bags of 16,384 x 1024 features, 16 bags per optimiser
 step and per GPU (bp_every_batch, config/cfg_nlst.yaml:71) = 512 MiB (bf16) / 1 GiB (fp32) of features per step per GPU
@@ -24,6 +25,8 @@ Printed JSON line
   gpu_eager_baseline    the same unmodified handler around the reference's own modules `.cuda()` on the same B200
   cpu_baseline          ... and on this box's host cores (kind "reference" when oracle/_ref is staged, else the oracle port)
 `--impl reference` times only that CPU path (the reference arm of the driver).
+`--dump-outputs DIR` writes what the last timed step produced as DIR/<name>.npy (see dump_outputs); the inputs, weights,
+noise and dropout seeds depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import contextlib
@@ -382,6 +385,17 @@ def local_counts(st):
     return (float(((st.e == 1) & (st.visible != 0)).sum()), float(len(st.lengths)), float(st.visible.sum()))
 
 
+def dump_outputs(out_dir, out, engine):
+    """`--dump-outputs`: the tensors the engine's step returned (losses, per-bag predictions and discriminator outputs, the
+    real-pair mask) and the flat G / D parameters that step left behind after both Adam updates, as out_dir/<name>.npy in
+    float32 (about 5 MB for the ABMIL networks).  Call it after the timed region and before anything else steps the engine."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v for k, v in out.items() if isinstance(v, torch.Tensor)}
+    arrays.update(params_G=engine.G.flat, params_D=engine.D.flat)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def leg_mode(ctx, precision, res_bf16, counts, steps, warmup):
     """configs[1] in another precision mode: the same bags (the bf16 values widened to fp32 on the device -- exactly
     representable), a fresh pair of networks and engine."""
@@ -555,10 +569,12 @@ def run_esat(args, rank, world, local_rank):
     ev0.record()
     th0 = time.perf_counter()
     for i in range(args.steps):
-        one_step(args.warmup + i)
+        out = one_step(args.warmup + i)
     ev1.record()
     ctx.barrier()
     clocks = sampler.stop(th0, time.perf_counter()) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, eng)
     launches = int(lib.advmil_launch_count(0))
     ms_dev = ctx.max_over_ranks(ev0.elapsed_time(ev1))
     value = args.bags * world * args.steps / (ms_dev / 1e3)
@@ -685,6 +701,8 @@ def run_main(args, rank, world, local_rank):
     ev1.record()
     ctx.barrier()
     clocks = sampler.stop(th0, time.perf_counter()) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, engine)
     ms = ev0.elapsed_time(ev1)
     launches = int(lib.advmil_launch_count(0))
     # per-kernel-class CUDA-event timing in a SEPARATE pass (the event records perturb the step, so they stay out of the
@@ -880,7 +898,11 @@ def main():
                     help="generator backbone: abmil (the benchmark's workload, C-fused AdvStep) or patch (ESAT, C-fused EsatAdvStep)")
     ap.add_argument("--ragged", action="store_true",
                     help="main line on configs[2] instead of configs[1]: bag lengths log-uniform in [1024, 100000]")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step and the parameters it left as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the timed GPU step; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -11,8 +11,8 @@ next to the built `.so`.  Consumers (all of them checkers / baselines, never the
   * `bench.py --impl reference` and the `cpu_baseline` leg: the reference's own modules, losses, optimiser factory and
     `MyHandler._update_disc/_update_gen` on the box's host cores (`cpu_baseline.kind = "reference"`);
   * `bench.py`'s `gpu_eager_baseline`: the same unmodified handler methods with the modules `.cuda()` on the same B200;
-  * `tests/test_gpu_handler.py`: the unmodified `MyHandler._train_each_epoch` around the reference modules and around
-    the advmil_b200 modules (four-import swap of INTEGRATION.md §1).
+  * `bench.py`'s `dropin_handler`: the unmodified handler methods around the advmil_b200 modules (four-import swap of
+    INTEGRATION.md §1).
 
 Nothing under advmil_b200/ imports it (tests/test_host_cpu.py enforces that).
 """

@@ -1,6 +1,6 @@
 """TEST / BASELINE INFRASTRUCTURE -- drives the reference's UNMODIFIED `MyHandler` (model/model_handler.py).
 
-Only tests/, bench.py's baseline legs and __graft_entry__ use this file; the product path never imports it.
+Only bench.py's baseline legs use this file; the product path never imports it.
 
 What it offers
   * `load_cfg(**over)`        the reference's own config/cfg_nlst.yaml with overrides (bcb_mode, paths, ...);
