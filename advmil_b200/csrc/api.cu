@@ -19,10 +19,6 @@ void set_error(const char* fmt, ...) {
   va_end(ap);
 }
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-bool pdl_enabled() {
-  static const int on = [] { const char* e = getenv("ADVMIL_PDL"); return (e && atoi(e) == 0) ? 0 : 1; }();
-  return on != 0;
-}
 
 // ---- per-stage event profiling ------------------------------------------------------------------
 struct ProfRec { int tag; cudaEvent_t a, b; };

@@ -51,25 +51,20 @@ void count_launch(int n = 1);
 // with cudaLaunchAttributeProgrammaticStreamSerialization and starts with pdl_prologue(): it lets ITS dependents be
 // scheduled right away (their CTAs become resident while this grid still runs) and then waits until the grid(s) it
 // depends on have completed and flushed, so no kernel touches memory before its predecessor in the stream is done.  The
-// gain is the launch/scheduling latency between dependent kernels.  ADVMIL_PDL=0 launches without the attribute (the
-// two instructions are then no-ops).
+// gain is the launch/scheduling latency between dependent kernels.
 __device__ __forceinline__ void pdl_prologue() {
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   asm volatile("griddepcontrol.wait;" ::: "memory");
 }
-bool pdl_enabled();
 template <typename... Exp, typename... Act>
 static inline void launch_kc(void (*kern)(Exp...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, unsigned cluster_x,
                              Act&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
   cudaLaunchAttribute at[2];
-  unsigned n = 0;
-  if (pdl_enabled()) {
-    at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  unsigned n = 1;
   if (cluster_x > 1) {
     at[n].id = cudaLaunchAttributeClusterDimension;
     at[n].val.clusterDim.x = cluster_x; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;

@@ -3,7 +3,6 @@
 // The N-row projection runs on the GEMM engines in the caller's precision mode; everything after the region mean works
 // on rows/16 region rows in fp32 (contractions on tcgen05 kind::tf32 outside the exact-fp32 mode, like the RLIP head).
 #include <mutex>
-#include <stdlib.h>
 #include <vector>
 #include "stages.cuh"
 
@@ -26,7 +25,7 @@ __global__ void region_offsets_kernel(const int32_t* __restrict__ offs, int n, i
 // (advmil_adv_step_esat_gen) requests it: 3.40 -> 3.32 ms per step.  The module path does not: the generator's forward +
 // backward alone gains 4 % (2.22 -> 2.13 ms), but the Python-composed ModuleAdvStep is within a few percent of being
 // host-bound and the six extra event record / wait pairs per backward cost it more host time than the overlap saves
-// (4.42 -> 4.60 ms per step).  ADVMIL_ESAT_OVERLAP=1 / 0 forces it on / off everywhere.
+// (4.42 -> 4.60 ms per step).
 struct EsatSide {
   cudaStream_t st = nullptr;
   cudaEvent_t fork = nullptr, join = nullptr;
@@ -37,10 +36,7 @@ static thread_local int g_esat_overlap_request = 0;      // set by the C-fused s
 void esat_request_overlap(int on) { g_esat_overlap_request = on; }
 static int esat_side_get(EsatSide** out) {
   *out = nullptr;
-  static int env = -2;                                    // ADVMIL_ESAT_OVERLAP: 1 = always, 0 = never, unset = only where requested
-  if (env == -2) { const char* e = getenv("ADVMIL_ESAT_OVERLAP"); env = e ? (atoi(e) != 0 ? 1 : 0) : -1; }
-  const int enabled = env >= 0 ? env : g_esat_overlap_request;
-  if (!enabled) return ADVMIL_OK;
+  if (!g_esat_overlap_request) return ADVMIL_OK;
   int dev = 0;
   ADVMIL_CHECK_CUDA(cudaGetDevice(&dev));
   if (dev < 0 || dev >= 64) return ADVMIL_OK;

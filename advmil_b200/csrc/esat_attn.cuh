@@ -1,4 +1,4 @@
-// Shared between the warp-level (esat_kernels.cu) and the tcgen05 (esat_attn_tc.cu) attention kernels.
+// Shared between the FFMA (esat_kernels.cu) and the tcgen05 (esat_attn_tc.cu, esat_attn_bwd_tc.cu) attention kernels.
 #pragma once
 #include "common.cuh"
 

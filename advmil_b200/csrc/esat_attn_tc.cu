@@ -16,9 +16,8 @@
 // query row exchange the row maximum inside the group; one group computes while the other waits for its MMAs; the two
 // partial results are merged at the end), warp 16 MMA issuer, warp 17 TMA producer of q and the k tiles, warp 18 TMA producer of the v tiles (a k slot is free as soon as its S has
 // retired, a v slot only after P V: separate rings keep the next S from waiting behind a P V plus a TMA round trip).
-// Dropout keep bits: the same counter generator and indices as the warp-level kernels (esat_kernels.cu), so the backward
+// Dropout keep bits: the same counter generator and indices as the FFMA kernels (esat_kernels.cu), so the backward
 // pass regenerates them.
-#include <stdlib.h>
 #include "stages.cuh"
 #include "tc_ptx.cuh"
 #include "esat_attn.cuh"
@@ -377,9 +376,7 @@ mha_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmK /*q, k: K-major*/
 }  // namespace
 
 bool mha_tcgen05_supported(int hd, int d) {
-  static int enabled = -1;
-  if (enabled < 0) { const char* e = getenv("ADVMIL_ATTN_TCGEN05"); enabled = (e && atoi(e) == 0) ? 0 : 1; }
-  return enabled && (hd == 16 || hd == 32 || hd == 48 || hd == 64) && (3 * (long long)d * 4) % 16 == 0;
+  return (hd == 16 || hd == 32 || hd == 48 || hd == 64) && (3 * (long long)d * 4) % 16 == 0;
 }
 
 template <int HD>

@@ -3,7 +3,6 @@
 // and multi-head self-attention over the regions of each bag (forward and backward).  Everything here works on
 // rows/16 "region" rows; the N-row contraction of the embedding runs on the GEMM engines (gemm_stages.cu).
 #include <limits.h>
-#include <stdlib.h>
 #include "stages.cuh"
 #include "esat_attn.cuh"
 
@@ -497,374 +496,6 @@ __global__ void __launch_bounds__(ATT_BQ) mha_bwd_kv_kernel(const float* __restr
   }
 }
 
-// =============================================================================================
-// Tensor-core variants of the three attention kernels for the tf32 / bf16 modes (the exact-fp32 mode keeps the FFMA
-// kernels above): warp-level mma.sync m16n8k8 tf32 with fp32 accumulation, flash-style.  One warp owns 16 "row"
-// items (queries in forward / dQ, keys in dK/dV), the "column" items stream through shared memory in tiles.
-//
-// The probabilities (C fragments: row g / g+8, columns 2t, 2t+1 of an 8-wide tile) feed the second contraction as A
-// fragments without any shuffle: A's k-slot t takes column 2t and k-slot t+4 takes column 2t+1, and the B operand reads
-// its rows in the same permuted order (row 2t for b0, row 2t+1 for b1) -- a sum over the contracted index does not
-// care about its order.  Shared-memory rows are HD + 4 floats so that both B access patterns are bank-conflict free.
-// =============================================================================================
-__device__ __forceinline__ uint32_t f2tf32(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return r;
-}
-__device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-constexpr int TCA_WARPS = 4;                 // 64 row items per CTA
-constexpr int TCA_ROWS = 16 * TCA_WARPS;
-
-// A fragments (HD/8 k-steps) of 16 rows [row0 + g, row0 + g + 8] x HD columns of a row-major matrix with stride ld;
-// rows >= nrows read as zero; values are multiplied by `mul` before the tf32 rounding
-template <int HD>
-__device__ __forceinline__ void load_a_frags(const float* __restrict__ base, size_t ld, int row0, int nrows, int lane, float mul,
-                                             uint32_t (&a)[HD / 8][4]) {
-  const int g = lane >> 2, t = lane & 3;
-  const bool v0 = row0 + g < nrows, v1 = row0 + g + 8 < nrows;
-  const float* p0 = base + (size_t)(row0 + g) * ld;
-  const float* p1 = base + (size_t)(row0 + g + 8) * ld;
-#pragma unroll
-  for (int ks = 0; ks < HD / 8; ++ks) {
-    a[ks][0] = f2tf32(v0 ? p0[ks * 8 + t] * mul : 0.f);
-    a[ks][1] = f2tf32(v1 ? p1[ks * 8 + t] * mul : 0.f);
-    a[ks][2] = f2tf32(v0 ? p0[ks * 8 + t + 4] * mul : 0.f);
-    a[ks][3] = f2tf32(v1 ? p1[ks * 8 + t + 4] * mul : 0.f);
-  }
-}
-// asynchronous copy of N rows x HD columns (row stride ld floats, zero beyond nvalid) into S[N][HD + 4]: 16-byte cp.async
-// chunks, raw fp32 bits (the tensor core reads the top 19 bits of each word: tf32 by truncation).  The caller commits
-// and waits for the group.
-template <int HD, int N>
-__device__ __forceinline__ void tile_copy_async(const float* __restrict__ base, size_t ld, int nvalid, uint32_t (*S)[HD + 4]) {
-  for (int i = threadIdx.x; i < N * (HD / 4); i += blockDim.x) {
-    const int j = i / (HD / 4), c4 = i % (HD / 4);
-    const uint32_t dst = (uint32_t)__cvta_generic_to_shared(&S[j][4 * c4]);
-    if (j < nvalid) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(base + (size_t)j * ld + 4 * c4) : "memory");
-    else *reinterpret_cast<uint4*>(&S[j][4 * c4]) = make_uint4(0u, 0u, 0u, 0u);
-  }
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-// C[nt] (16 x 8 per tile, NT tiles) += A (16 x HD) . B^T where B rows are the column items: B(k = c, n = item)
-template <int HD, int NT>
-__device__ __forceinline__ void mma_rows_x_items(float (&c)[NT][4], const uint32_t (&a)[HD / 8][4], const uint32_t (*S)[HD + 4], int lane) {
-  const int g = lane >> 2, t = lane & 3;
-#pragma unroll
-  for (int ks = 0; ks < HD / 8; ++ks)
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) mma_tf32(c[nt], a[ks], S[nt * 8 + g][ks * 8 + t], S[nt * 8 + g][ks * 8 + t + 4]);
-}
-// O[no] (16 x 8 per tile, HD/8 tiles) += P (16 x 8 NT, C-fragment layout, permuted k order) . V (items x HD)
-template <int HD, int NT>
-__device__ __forceinline__ void mma_probs_x_values(float (&o)[HD / 8][4], const float (&p)[NT][4], const uint32_t (*S)[HD + 4], int lane) {
-  const int g = lane >> 2, t = lane & 3;
-#pragma unroll
-  for (int nt = 0; nt < NT; ++nt) {
-    const uint32_t a[4] = {f2tf32(p[nt][0]), f2tf32(p[nt][2]), f2tf32(p[nt][1]), f2tf32(p[nt][3])};
-#pragma unroll
-    for (int no = 0; no < HD / 8; ++no) mma_tf32(o[no], a, S[nt * 8 + 2 * t][no * 8 + g], S[nt * 8 + 2 * t + 1][no * 8 + g]);
-  }
-}
-// 2^x on the SFU; the attention kernels keep their logits in log2 units (q is pre-scaled by log2(e) / sqrt(hd))
-__device__ __forceinline__ float ex2f(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-constexpr float kLog2e = 1.4426950408889634f, kLn2 = 0.6931471805599453f;
-__device__ __forceinline__ float quad_max(float v) {
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1));
-  return fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
-}
-__device__ __forceinline__ float quad_sum(float v) {
-  v += __shfl_xor_sync(0xffffffffu, v, 1);
-  return v + __shfl_xor_sync(0xffffffffu, v, 2);
-}
-
-constexpr int TCF_KT = 64;   // keys per shared-memory tile, forward
-template <int HD> constexpr size_t mha_fwd_tc_smem() { return (size_t)2 * 2 * TCF_KT * (HD + 4) * sizeof(uint32_t); }
-template <int HD>
-__global__ void __launch_bounds__(32 * TCA_WARPS, 4) mha_fwd_tc_kernel(const float* __restrict__ qkv, const int32_t* __restrict__ ro, int d,
-                                                                   float scale, AttDrop ad, float* __restrict__ ctx,
-                                                                   float* __restrict__ lse, int Rtot) {
-  pdl_prologue();
-  extern __shared__ __align__(16) uint32_t tca_smem[];
-  typedef uint32_t (*Tile)[HD + 4];
-  auto Kt = [&](int i) { return reinterpret_cast<Tile>(tca_smem + (size_t)i * 2 * TCF_KT * (HD + 4)); };   // [K tile | V tile] per buffer
-  auto Vt = [&](int i) { return Kt(i) + TCF_KT; };
-  constexpr int NT = TCF_KT / 8;
-  const int b = blockIdx.y, head = blockIdx.z, r0 = ro[b], Rb = ro[b + 1] - r0;
-  if ((int)blockIdx.x * TCA_ROWS >= Rb) return;
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, g = lane >> 2, t = lane & 3;
-  const int q0 = blockIdx.x * TCA_ROWS + wid * 16;
-  const size_t ld = 3 * (size_t)d;
-  const float* Q = qkv + (size_t)r0 * ld + head * HD;
-  tile_copy_async<HD, TCF_KT>(Q + d, ld, min(TCF_KT, Rb), Kt(0));
-  tile_copy_async<HD, TCF_KT>(Q + 2 * d, ld, min(TCF_KT, Rb), Vt(0));
-  cp_async_commit();
-  uint32_t qa[HD / 8][4];
-  load_a_frags<HD>(Q, ld, q0, Rb, lane, scale * kLog2e, qa);      // logits in log2 units
-  float o[HD / 8][4];
-#pragma unroll
-  for (int no = 0; no < HD / 8; ++no) o[no][0] = o[no][1] = o[no][2] = o[no][3] = 0.f;
-  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-  const int qi0 = q0 + g, qi1 = q0 + g + 8;
-  int buf = 0;
-  for (int k0 = 0; k0 < Rb; k0 += TCF_KT, buf ^= 1) {
-    const int nk = min(TCF_KT, Rb - k0);
-    if (k0 + TCF_KT < Rb) {            // prefetch the next tile into the other buffer
-      const int nn = min(TCF_KT, Rb - k0 - TCF_KT);
-      tile_copy_async<HD, TCF_KT>(Q + (size_t)(k0 + TCF_KT) * ld + d, ld, nn, Kt(buf ^ 1));
-      tile_copy_async<HD, TCF_KT>(Q + (size_t)(k0 + TCF_KT) * ld + 2 * d, ld, nn, Vt(buf ^ 1));
-      cp_async_commit();
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncthreads();
-    float s[NT][4];
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f;
-    mma_rows_x_items<HD, NT>(s, qa, Kt(buf), lane);
-    float mx0 = -INFINITY, mx1 = -INFINITY;
-    if (nk < TCF_KT) {                 // only the last tile of a bag has keys to mask
-#pragma unroll
-      for (int nt = 0; nt < NT; ++nt) {
-        const int kc = nt * 8 + 2 * t;
-        if (kc >= nk) s[nt][0] = s[nt][2] = -INFINITY;
-        if (kc + 1 >= nk) s[nt][1] = s[nt][3] = -INFINITY;
-      }
-    }
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      mx0 = fmaxf(mx0, fmaxf(s[nt][0], s[nt][1]));
-      mx1 = fmaxf(mx1, fmaxf(s[nt][2], s[nt][3]));
-    }
-    const float mn0 = fmaxf(m0, quad_max(mx0)), mn1 = fmaxf(m1, quad_max(mx1));
-    const float c0 = ex2f(m0 - mn0), c1 = ex2f(m1 - mn1);
-    l0 *= c0; l1 *= c1;
-#pragma unroll
-    for (int no = 0; no < HD / 8; ++no) { o[no][0] *= c0; o[no][1] *= c0; o[no][2] *= c1; o[no][3] *= c1; }
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      const int kc = k0 + nt * 8 + 2 * t;
-      float p0 = ex2f(s[nt][0] - mn0), p1 = ex2f(s[nt][1] - mn0), p2 = ex2f(s[nt][2] - mn1), p3 = ex2f(s[nt][3] - mn1);
-      l0 += p0 + p1; l1 += p2 + p3;
-      if (ad.drop.active) {
-        if (ad.mask) {
-          if (!ad.keep(b, head, min(qi0, Rb - 1), min(kc, Rb - 1), Rb, 0)) p0 = 0.f;
-          if (!ad.keep(b, head, min(qi0, Rb - 1), min(kc + 1, Rb - 1), Rb, 0)) p1 = 0.f;
-          if (!ad.keep(b, head, min(qi1, Rb - 1), min(kc, Rb - 1), Rb, 0)) p2 = 0.f;
-          if (!ad.keep(b, head, min(qi1, Rb - 1), min(kc + 1, Rb - 1), Rb, 0)) p3 = 0.f;
-        } else {
-          bool ka, kb;
-          ad.drop.keep2((uint32_t)(r0 + qi0) * (uint32_t)ad.heads + (uint32_t)head, (uint32_t)kc, ka, kb);
-          if (!ka) p0 = 0.f;
-          if (!kb) p1 = 0.f;
-          ad.drop.keep2((uint32_t)(r0 + qi1) * (uint32_t)ad.heads + (uint32_t)head, (uint32_t)kc, ka, kb);
-          if (!ka) p2 = 0.f;
-          if (!kb) p3 = 0.f;
-        }
-      }
-      s[nt][0] = p0; s[nt][1] = p1; s[nt][2] = p2; s[nt][3] = p3;
-    }
-    mma_probs_x_values<HD, NT>(o, s, Vt(buf), lane);
-    m0 = mn0; m1 = mn1;
-    __syncthreads();                   // this buffer is refilled by the prefetch of the iteration after next
-  }
-  l0 = quad_sum(l0); l1 = quad_sum(l1);
-  const float i0 = ad.drop.inv_keep / l0, i1 = ad.drop.inv_keep / l1;
-#pragma unroll
-  for (int no = 0; no < HD / 8; ++no) {
-    if (qi0 < Rb) *reinterpret_cast<float2*>(ctx + (size_t)(r0 + qi0) * d + head * HD + no * 8 + 2 * t) = make_float2(o[no][0] * i0, o[no][1] * i0);
-    if (qi1 < Rb) *reinterpret_cast<float2*>(ctx + (size_t)(r0 + qi1) * d + head * HD + no * 8 + 2 * t) = make_float2(o[no][2] * i1, o[no][3] * i1);
-  }
-  if (t == 0) {
-    if (qi0 < Rb) lse[(size_t)head * Rtot + r0 + qi0] = m0 * kLn2 + __logf(l0);      // back to natural units
-    if (qi1 < Rb) lse[(size_t)head * Rtot + r0 + qi1] = m1 * kLn2 + __logf(l1);
-  }
-}
-
-// probabilities and their gradients of one 16 x (8 NT) tile: s holds the logits on entry, P (dropped, scaled) or dS on exit
-//   rows: the warp's row items (r_lo = g, r_hi = g + 8), columns: tile items 2t, 2t+1 of each 8-wide block
-constexpr int TCB_T = 32;    // column items per shared-memory tile, backward
-template <int HD>
-__global__ void __launch_bounds__(32 * TCA_WARPS, 3) mha_bwd_q_tc_kernel(const float* __restrict__ qkv, const float* __restrict__ ctx,
-                                                                     const float* __restrict__ d_ctx, const float* __restrict__ lse,
-                                                                     const int32_t* __restrict__ ro, int d, float scale, AttDrop ad,
-                                                                     float* __restrict__ d_qkv, float* __restrict__ Dq, int Rtot) {
-  pdl_prologue();
-  __shared__ __align__(16) uint32_t Ks[2][TCB_T][HD + 4];
-  __shared__ __align__(16) uint32_t Vs[2][TCB_T][HD + 4];
-  constexpr int NT = TCB_T / 8;
-  const int b = blockIdx.y, head = blockIdx.z, r0 = ro[b], Rb = ro[b + 1] - r0;
-  if ((int)blockIdx.x * TCA_ROWS >= Rb) return;
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, g = lane >> 2, t = lane & 3;
-  const int q0 = blockIdx.x * TCA_ROWS + wid * 16;
-  const size_t ld = 3 * (size_t)d;
-  const float* Q = qkv + (size_t)r0 * ld + head * HD;
-  const float* G = d_ctx + (size_t)r0 * d + head * HD;
-  const float* O = ctx + (size_t)r0 * d + head * HD;
-  tile_copy_async<HD, TCB_T>(Q + d, ld, min(TCB_T, Rb), Ks[0]);
-  tile_copy_async<HD, TCB_T>(Q + 2 * d, ld, min(TCB_T, Rb), Vs[0]);
-  cp_async_commit();
-  const int qi0 = q0 + g, qi1 = q0 + g + 8;
-  uint32_t qa[HD / 8][4], ga[HD / 8][4];
-  load_a_frags<HD>(Q, ld, q0, Rb, lane, scale * kLog2e, qa);      // logits in log2 units
-  load_a_frags<HD>(G, d, q0, Rb, lane, 1.f, ga);
-  // D_i = dO_i . O_i in full fp32 (each lane owns columns t, t+4 of every k-step; the quad completes the row)
-  float D0 = 0.f, D1 = 0.f;
-#pragma unroll
-  for (int ks = 0; ks < HD / 8; ++ks) {
-    if (qi0 < Rb) D0 += G[(size_t)qi0 * d + ks * 8 + t] * O[(size_t)qi0 * d + ks * 8 + t] + G[(size_t)qi0 * d + ks * 8 + t + 4] * O[(size_t)qi0 * d + ks * 8 + t + 4];
-    if (qi1 < Rb) D1 += G[(size_t)qi1 * d + ks * 8 + t] * O[(size_t)qi1 * d + ks * 8 + t] + G[(size_t)qi1 * d + ks * 8 + t + 4] * O[(size_t)qi1 * d + ks * 8 + t + 4];
-  }
-  D0 = quad_sum(D0); D1 = quad_sum(D1);
-  const float L0 = qi0 < Rb ? lse[(size_t)head * Rtot + r0 + qi0] * kLog2e : 0.f, L1 = qi1 < Rb ? lse[(size_t)head * Rtot + r0 + qi1] * kLog2e : 0.f;
-  if (t == 0) {
-    if (qi0 < Rb) Dq[(size_t)head * Rtot + r0 + qi0] = D0;
-    if (qi1 < Rb) Dq[(size_t)head * Rtot + r0 + qi1] = D1;
-  }
-  float dq[HD / 8][4];
-#pragma unroll
-  for (int no = 0; no < HD / 8; ++no) dq[no][0] = dq[no][1] = dq[no][2] = dq[no][3] = 0.f;
-  const float ik = ad.drop.inv_keep;
-  int buf = 0;
-  for (int k0 = 0; k0 < Rb; k0 += TCB_T, buf ^= 1) {
-    const int nk = min(TCB_T, Rb - k0);
-    if (k0 + TCB_T < Rb) {
-      const int nn = min(TCB_T, Rb - k0 - TCB_T);
-      tile_copy_async<HD, TCB_T>(Q + (size_t)(k0 + TCB_T) * ld + d, ld, nn, Ks[buf ^ 1]);
-      tile_copy_async<HD, TCB_T>(Q + (size_t)(k0 + TCB_T) * ld + 2 * d, ld, nn, Vs[buf ^ 1]);
-      cp_async_commit();
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncthreads();
-    float s[NT][4], dp[NT][4];
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) { s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f; dp[nt][0] = dp[nt][1] = dp[nt][2] = dp[nt][3] = 0.f; }
-    mma_rows_x_items<HD, NT>(s, qa, Ks[buf], lane);
-    mma_rows_x_items<HD, NT>(dp, ga, Vs[buf], lane);
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      const int kl = nt * 8 + 2 * t, kc = k0 + kl;
-      bool k00 = true, k01 = true, k10 = true, k11 = true;
-      if (ad.drop.active) {
-        if (ad.mask) {
-          k00 = ad.keep(b, head, min(qi0, Rb - 1), min(kc, Rb - 1), Rb, 0); k01 = ad.keep(b, head, min(qi0, Rb - 1), min(kc + 1, Rb - 1), Rb, 0);
-          k10 = ad.keep(b, head, min(qi1, Rb - 1), min(kc, Rb - 1), Rb, 0); k11 = ad.keep(b, head, min(qi1, Rb - 1), min(kc + 1, Rb - 1), Rb, 0);
-        } else {
-          ad.drop.keep2((uint32_t)(r0 + qi0) * (uint32_t)ad.heads + (uint32_t)head, (uint32_t)kc, k00, k01);
-          ad.drop.keep2((uint32_t)(r0 + qi1) * (uint32_t)ad.heads + (uint32_t)head, (uint32_t)kc, k10, k11);
-        }
-      }
-      const float p0 = kl < nk ? ex2f(s[nt][0] - L0) : 0.f, p1 = kl + 1 < nk ? ex2f(s[nt][1] - L0) : 0.f;
-      const float p2 = kl < nk ? ex2f(s[nt][2] - L1) : 0.f, p3 = kl + 1 < nk ? ex2f(s[nt][3] - L1) : 0.f;
-      s[nt][0] = p0 * ((k00 ? dp[nt][0] * ik : 0.f) - D0); s[nt][1] = p1 * ((k01 ? dp[nt][1] * ik : 0.f) - D0);
-      s[nt][2] = p2 * ((k10 ? dp[nt][2] * ik : 0.f) - D1); s[nt][3] = p3 * ((k11 ? dp[nt][3] * ik : 0.f) - D1);
-    }
-    mma_probs_x_values<HD, NT>(dq, s, Ks[buf], lane);
-    __syncthreads();
-  }
-#pragma unroll
-  for (int no = 0; no < HD / 8; ++no) {
-    if (qi0 < Rb) *reinterpret_cast<float2*>(d_qkv + (size_t)(r0 + qi0) * ld + head * HD + no * 8 + 2 * t) = make_float2(dq[no][0] * scale, dq[no][1] * scale);
-    if (qi1 < Rb) *reinterpret_cast<float2*>(d_qkv + (size_t)(r0 + qi1) * ld + head * HD + no * 8 + 2 * t) = make_float2(dq[no][2] * scale, dq[no][3] * scale);
-  }
-}
-
-// dK, dV: the warp's rows are keys, the streamed columns are queries (transposed tiles S^T = K Q^T, dP^T = V dO^T)
-template <int HD>
-__global__ void __launch_bounds__(32 * TCA_WARPS, 3) mha_bwd_kv_tc_kernel(const float* __restrict__ qkv, const float* __restrict__ d_ctx,
-                                                                      const float* __restrict__ lse, const float* __restrict__ Dq,
-                                                                      const int32_t* __restrict__ ro, int d, float scale, AttDrop ad,
-                                                                      float* __restrict__ d_qkv, int Rtot) {
-  pdl_prologue();
-  __shared__ __align__(16) uint32_t Qs[2][TCB_T][HD + 4];
-  __shared__ __align__(16) uint32_t Gs[2][TCB_T][HD + 4];
-  __shared__ float Ls[2][TCB_T], Ds[2][TCB_T];
-  constexpr int NT = TCB_T / 8;
-  const int b = blockIdx.y, head = blockIdx.z, r0 = ro[b], Rb = ro[b + 1] - r0;
-  if ((int)blockIdx.x * TCA_ROWS >= Rb) return;
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, g = lane >> 2, t = lane & 3;
-  const int kb0 = blockIdx.x * TCA_ROWS + wid * 16;
-  const size_t ld = 3 * (size_t)d;
-  const float* Q = qkv + (size_t)r0 * ld + head * HD;
-  const float* G = d_ctx + (size_t)r0 * d + head * HD;
-  const int kj0 = kb0 + g, kj1 = kb0 + g + 8;
-  tile_copy_async<HD, TCB_T>(Q, ld, min(TCB_T, Rb), Qs[0]);
-  tile_copy_async<HD, TCB_T>(G, d, min(TCB_T, Rb), Gs[0]);
-  cp_async_commit();
-  uint32_t ka[HD / 8][4], va[HD / 8][4];
-  load_a_frags<HD>(Q + d, ld, kb0, Rb, lane, 1.f, ka);
-  load_a_frags<HD>(Q + 2 * d, ld, kb0, Rb, lane, 1.f, va);
-  float dk[HD / 8][4], dv[HD / 8][4];
-#pragma unroll
-  for (int no = 0; no < HD / 8; ++no) { dk[no][0] = dk[no][1] = dk[no][2] = dk[no][3] = 0.f; dv[no][0] = dv[no][1] = dv[no][2] = dv[no][3] = 0.f; }
-  const float ik = ad.drop.inv_keep, sl2 = scale * kLog2e;
-  int buf = 0;
-  for (int q0 = 0; q0 < Rb; q0 += TCB_T, buf ^= 1) {
-    const int nq = min(TCB_T, Rb - q0);
-    if (threadIdx.x < TCB_T) {         // (this buffer's previous readers passed the barrier that ended the iteration before last)
-      Ls[buf][threadIdx.x] = (int)threadIdx.x < nq ? lse[(size_t)head * Rtot + r0 + q0 + threadIdx.x] * kLog2e : 0.f;   // log2 units
-      Ds[buf][threadIdx.x] = (int)threadIdx.x < nq ? Dq[(size_t)head * Rtot + r0 + q0 + threadIdx.x] : 0.f;
-    }
-    if (q0 + TCB_T < Rb) {
-      const int nn = min(TCB_T, Rb - q0 - TCB_T);
-      tile_copy_async<HD, TCB_T>(Q + (size_t)(q0 + TCB_T) * ld, ld, nn, Qs[buf ^ 1]);
-      tile_copy_async<HD, TCB_T>(G + (size_t)(q0 + TCB_T) * d, d, nn, Gs[buf ^ 1]);
-      cp_async_commit();
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncthreads();
-    float s[NT][4], dp[NT][4];
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) { s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f; dp[nt][0] = dp[nt][1] = dp[nt][2] = dp[nt][3] = 0.f; }
-    mma_rows_x_items<HD, NT>(s, ka, Qs[buf], lane);       // S^T[key][query] without the 1/sqrt(hd) factor
-    mma_rows_x_items<HD, NT>(dp, va, Gs[buf], lane);      // dP^T[key][query]
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      const int ql = nt * 8 + 2 * t, qc = q0 + ql;    // this lane's two queries: qc, qc + 1 (columns); keys kj0 / kj1 (rows)
-      bool k00 = true, k01 = true, k10 = true, k11 = true;   // kXY: key row X (0: kj0, 1: kj1), query column Y
-      if (ad.drop.active) {
-        const int qa_ = min(qc, Rb - 1), qb_ = min(qc + 1, Rb - 1), ka_ = min(kj0, Rb - 1), kb_ = min(kj1, Rb - 1);
-        k00 = ad.keep(b, head, qa_, ka_, Rb, r0 + qa_); k01 = ad.keep(b, head, qb_, ka_, Rb, r0 + qb_);
-        k10 = ad.keep(b, head, qa_, kb_, Rb, r0 + qa_); k11 = ad.keep(b, head, qb_, kb_, Rb, r0 + qb_);
-      }
-      const float La = Ls[buf][ql], Lb = Ls[buf][ql + 1], Da = Ds[buf][ql], Db = Ds[buf][ql + 1];
-      const float p0 = ql < nq ? ex2f(fmaf(s[nt][0], sl2, -La)) : 0.f, p1 = ql + 1 < nq ? ex2f(fmaf(s[nt][1], sl2, -Lb)) : 0.f;
-      const float p2 = ql < nq ? ex2f(fmaf(s[nt][2], sl2, -La)) : 0.f, p3 = ql + 1 < nq ? ex2f(fmaf(s[nt][3], sl2, -Lb)) : 0.f;
-      s[nt][0] = p0 * ((k00 ? dp[nt][0] * ik : 0.f) - Da); s[nt][1] = p1 * ((k01 ? dp[nt][1] * ik : 0.f) - Db);
-      s[nt][2] = p2 * ((k10 ? dp[nt][2] * ik : 0.f) - Da); s[nt][3] = p3 * ((k11 ? dp[nt][3] * ik : 0.f) - Db);
-      dp[nt][0] = k00 ? p0 * ik : 0.f; dp[nt][1] = k01 ? p1 * ik : 0.f; dp[nt][2] = k10 ? p2 * ik : 0.f; dp[nt][3] = k11 ? p3 * ik : 0.f;
-    }
-    mma_probs_x_values<HD, NT>(dv, dp, Gs[buf], lane);    // dV += Pd^T dO
-    mma_probs_x_values<HD, NT>(dk, s, Qs[buf], lane);     // dK += dS^T Q (the 1/sqrt(hd) factor is applied at the store)
-    __syncthreads();
-  }
-#pragma unroll
-  for (int no = 0; no < HD / 8; ++no) {
-    if (kj0 < Rb) {
-      *reinterpret_cast<float2*>(d_qkv + (size_t)(r0 + kj0) * ld + d + head * HD + no * 8 + 2 * t) = make_float2(dk[no][0] * scale, dk[no][1] * scale);
-      *reinterpret_cast<float2*>(d_qkv + (size_t)(r0 + kj0) * ld + 2 * d + head * HD + no * 8 + 2 * t) = make_float2(dv[no][0], dv[no][1]);
-    }
-    if (kj1 < Rb) {
-      *reinterpret_cast<float2*>(d_qkv + (size_t)(r0 + kj1) * ld + d + head * HD + no * 8 + 2 * t) = make_float2(dk[no][2] * scale, dk[no][3] * scale);
-      *reinterpret_cast<float2*>(d_qkv + (size_t)(r0 + kj1) * ld + 2 * d + head * HD + no * 8 + 2 * t) = make_float2(dv[no][2], dv[no][3]);
-    }
-  }
-}
-
 // ---- host launchers ---------------------------------------------------------------------------
 #define ESAT_NPL_SWITCH(d, CALL)                                                                        \
   switch ((d) / 32) {                                                                                   \
@@ -965,17 +596,9 @@ static AttDrop make_att_drop(const Drop& drop, const uint8_t* mask, const int64_
   return ad;
 }
 
-#define ESAT_HD8_SWITCH(hd, CALL)                                                                       \
-  switch (hd) {                                                                                         \
-    case 8: { constexpr int HD = 8; CALL; break; }                                                      \
-    case 16: { constexpr int HD = 16; CALL; break; }                                                    \
-    case 32: { constexpr int HD = 32; CALL; break; }                                                    \
-    case 48: { constexpr int HD = 48; CALL; break; }                                                    \
-    case 64: { constexpr int HD = 64; CALL; break; }                                                    \
-    default: ADVMIL_REQUIRE(false, "esat: head width %d unsupported on the tensor-core attention", (int)(hd)); \
-  }
-// the tf32 / bf16 modes run attention on the tensor cores when the head width allows it
-static bool mha_use_tc(int precision, int hd) { return precision != ADVMIL_FP32 && (hd == 8 || hd == 16 || hd == 32 || hd == 48 || hd == 64); }
+// the tf32 / bf16 modes run attention on the tcgen05 kernels when the head width allows it; the exact-fp32 mode and the
+// other head widths run the FFMA kernels
+static bool mha_use_tc(int precision, int hd, int d) { return precision != ADVMIL_FP32 && mha_tcgen05_supported(hd, d); }
 
 int mha_fwd(const float* qkv, const int32_t* ro, const int32_t* ro_host, int bags, int Rtot, int d, int heads, const Drop& drop,
             const uint8_t* mask, const int64_t* mask_off, float* ctx, float* lse, int precision, cudaStream_t st) {
@@ -986,25 +609,11 @@ int mha_fwd(const float* qkv, const int32_t* ro, const int32_t* ro_host, int bag
   for (int b = 0; b < bags; ++b) mx = max(mx, ro_host[b + 1] - ro_host[b]);
   const AttDrop ad = make_att_drop(drop, mask, mask_off, heads);
   const float scale = 1.0f / sqrtf((float)hd);
-  if (mha_use_tc(precision, hd) && mha_tcgen05_supported(hd, d))     // tcgen05 / TMEM / TMA kernel (esat_attn_tc.cu)
+  if (mha_use_tc(precision, hd, d))     // tcgen05 / TMEM / TMA kernel (esat_attn_tc.cu)
     return mha_fwd_tcgen05(qkv, ro, bags, Rtot, d, heads, mx, scale, ad, ctx, lse, st);
-  if (mha_use_tc(precision, hd)) {
-    ESAT_HD8_SWITCH(hd, {
-      static bool attr_set = false;    // > 48 KB of dynamic shared memory needs the opt-in once per instantiation
-      if (!attr_set) { ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(mha_fwd_tc_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mha_fwd_tc_smem<HD>())); attr_set = true; }
-      launch_k(mha_fwd_tc_kernel<HD>, dim3(cdiv(mx, TCA_ROWS), bags, heads), dim3(32 * TCA_WARPS), mha_fwd_tc_smem<HD>(), st, qkv, ro, d, scale, ad, ctx, lse, Rtot);
-    });
-  } else {
-    ESAT_HD_SWITCH(hd, (launch_k(mha_fwd_kernel<HD>, dim3(cdiv(mx, ATT_BQ), bags, heads), dim3(ATT_BQ), 0, st, qkv, ro, d, scale, ad, ctx, lse, Rtot)));
-  }
+  ESAT_HD_SWITCH(hd, (launch_k(mha_fwd_kernel<HD>, dim3(cdiv(mx, ATT_BQ), bags, heads), dim3(ATT_BQ), 0, st, qkv, ro, d, scale, ad, ctx, lse, Rtot)));
   ADVMIL_CHECK_LAUNCH();
   return ADVMIL_OK;
-}
-
-static bool mha_bwd_tcgen05_enabled() {
-  static int enabled = -1;
-  if (enabled < 0) { const char* e = getenv("ADVMIL_ATTN_BWD_TCGEN05"); enabled = (e && atoi(e) == 0) ? 0 : 1; }
-  return enabled != 0;
 }
 
 // Dq: [heads, Rtot] scratch
@@ -1018,16 +627,8 @@ int mha_bwd(const float* qkv, const float* ctx, const float* d_ctx, const float*
   for (int b = 0; b < bags; ++b) mx = max(mx, ro_host[b + 1] - ro_host[b]);
   const AttDrop ad = make_att_drop(drop, mask, mask_off, heads);
   const float scale = 1.0f / sqrtf((float)hd);
-  if (mha_use_tc(precision, hd) && mha_tcgen05_supported(hd, d) && mha_bwd_tcgen05_enabled())     // esat_attn_bwd_tc.cu
+  if (mha_use_tc(precision, hd, d))     // esat_attn_bwd_tc.cu
     return mha_bwd_tcgen05(qkv, ctx, d_ctx, lse, ro, bags, Rtot, d, heads, mx, scale, ad, d_qkv, Dq, st);
-  if (mha_use_tc(precision, hd)) {
-    const dim3 grid(cdiv(mx, TCA_ROWS), bags, heads);
-    ESAT_HD8_SWITCH(hd, (launch_k(mha_bwd_q_tc_kernel<HD>, grid, dim3(32 * TCA_WARPS), 0, st, qkv, ctx, d_ctx, lse, ro, d, scale, ad, d_qkv, Dq, Rtot)));
-    ADVMIL_CHECK_LAUNCH();
-    ESAT_HD8_SWITCH(hd, (launch_k(mha_bwd_kv_tc_kernel<HD>, grid, dim3(32 * TCA_WARPS), 0, st, qkv, d_ctx, lse, Dq, ro, d, scale, ad, d_qkv, Rtot)));
-    ADVMIL_CHECK_LAUNCH();
-    return ADVMIL_OK;
-  }
   const dim3 grid(cdiv(mx, ATT_BQ), bags, heads);
   ESAT_HD_SWITCH(hd, (launch_k(mha_bwd_q_kernel<HD>, grid, dim3(ATT_BQ), 0, st, qkv, ctx, d_ctx, lse, ro, d, scale, ad, d_qkv, Dq, Rtot)));
   ADVMIL_CHECK_LAUNCH();

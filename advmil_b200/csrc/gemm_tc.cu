@@ -13,7 +13,6 @@
 //
 // Warp roles (256 threads): warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-7 epilogue
 // (TMEM lane quarter = warp % 4).
-#include <stdlib.h>
 #include <mutex>
 #include "gemm_tc.cuh"
 #include "tc_ptx.cuh"
@@ -48,7 +47,6 @@ template <> struct TcElem<float> {
   static constexpr int MN_SBO = 512;            // 4 k-rows x 128 B per swizzle group
   __host__ __device__ static constexpr uint32_t idesc(int M, int N, int am, int bm) { return idesc_tf32(M, N, am, bm); }
   __device__ __forceinline__ static void mma(uint32_t d, uint64_t a, uint64_t b, uint32_t i, uint32_t acc) { mma_tf32(d, a, b, i, acc); }
-  __device__ __forceinline__ static void mma_pair(uint32_t d, uint64_t a, uint64_t b, uint32_t i, uint32_t acc) { mma_tf32_pair(d, a, b, i, acc); }
 };
 template <> struct TcElem<bf16> {
   static constexpr int KBLK = 64;
@@ -58,7 +56,6 @@ template <> struct TcElem<bf16> {
   static constexpr int MN_SBO = 1024;           // 8 k-rows x 128 B per swizzle atom
   __host__ __device__ static constexpr uint32_t idesc(int M, int N, int am, int bm) { return idesc_bf16(M, N, am, bm); }
   __device__ __forceinline__ static void mma(uint32_t d, uint64_t a, uint64_t b, uint32_t i, uint32_t acc) { mma_f16(d, a, b, i, acc); }
-  __device__ __forceinline__ static void mma_pair(uint32_t d, uint64_t a, uint64_t b, uint32_t i, uint32_t acc) { mma_f16_pair(d, a, b, i, acc); }
 };
 
 // row-major matrix [rows, cols] of T; box = box_rows x (128 B of elements), 128-byte swizzle, OOB reads return zeros
@@ -118,8 +115,8 @@ constexpr int STG_LD_LN = 132;                         // staging row stride for
 // buffer with `lo`; fence.proxy.async hands both to the tensor core); the weight's two parts are prepared in global
 // memory by a small kernel and arrive by TMA.  A stage therefore holds 2 x (A + B): 2 stages at 256 / 192 columns, with
 // 4 epilogue warps, which is enough because every stage now carries 12 MMAs.
-template <int ES, int BLOCK_N, int EPI, int CL = 1, bool X3 = false> struct RowCfg {
-  static_assert(!X3 || (ES == 4 && CL == 1), "split-tf32 runs on fp32 elements, single CTA");
+template <int ES, int BLOCK_N, int EPI, bool X3 = false> struct RowCfg {
+  static_assert(!X3 || ES == 4, "split-tf32 runs on fp32 elements");
   // Epilogue warps per TMEM lane quarter (NSUB).  The bf16 epilogues are chains of dependent ALU / shared / global
   // instructions: with 2 warps per scheduler the epilogue issued ~1 instruction per 8 cycles per warp and the tensor pipe
   // idled behind it (ncu r02: dh 35 % tensor-active at 0.26 IPC per scheduler).  4 warps per quarter (3 at 192 columns, where
@@ -128,7 +125,7 @@ template <int ES, int BLOCK_N, int EPI, int CL = 1, bool X3 = false> struct RowC
   static constexpr int NSUB = (EPI == EPI_LN || X3) ? 1 : (!WIDE_EPI ? 2 : (EPI != EPI_GATE && BLOCK_N == 192 ? 3 : (BLOCK_N >= 128 ? 4 : 2)));
   static constexpr int EPI_WARPS = 4 * NSUB;
   static constexpr int THREADS = 128 + 32 * EPI_WARPS;
-  static constexpr int B_STAGE_BYTES = BLOCK_N * 128 / CL;        // CTA pair: each CTA holds half of the B tile
+  static constexpr int B_STAGE_BYTES = BLOCK_N * 128;
   static constexpr int STAGE_BYTES = (X3 ? 2 : 1) * (A_STAGE_BYTES + B_STAGE_BYTES);
   static constexpr int TMA_BYTES = A_STAGE_BYTES + (X3 ? 2 : 1) * B_STAGE_BYTES;     // what TMA delivers per stage
   // bf16 staging: 32 rows x 64 bytes, XOR-swizzled (2 KB per warp); fp32 staging: 32 x 36 floats; LN: full 128-column rows
@@ -260,13 +257,6 @@ __device__ __forceinline__ float gate_chunk(float (&va)[32], float (&vb)[32], co
   return partial;
 }
 
-// CL = cluster size (1 or 2).  CL == 2 = CTA pair: the two CTAs of a cluster own two consecutive 128-row blocks of the
-// SAME N-tile; each loads its own A tile and HALF of the weight tile, and the leader (rank 0) issues
-// tcgen05.mma.cta_group::2 with M = 256, which reads both halves of B from the two SMs' shared memories and writes each
-// CTA's 128 accumulator rows into that CTA's TMEM.  Per SM the operand bytes per MMA drop from A + B to A + B/2 -- the
-// L2 -> SM ingress is what bounds the single-CTA kernels (profiles/exp_tile_width.py).
-// Barriers: full (leader: the TMA loads of BOTH CTAs complete their bytes on it), empty and tfull (the leader's
-// tcgen05.commit, multicast to both CTAs), tempty (leader: both CTAs' epilogues drained the accumulator buffer).
 // tf32-exact high part and tf32-rounded low part of an fp32 value (cvt.rna.tf32.f32: low 13 mantissa bits zero)
 __device__ __forceinline__ uint32_t tf32_rna(float x) { uint32_t r; asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x)); return r; }
 __device__ __forceinline__ void split_tf32(uint32_t raw, uint32_t& hi, uint32_t& lo) {
@@ -278,12 +268,15 @@ __device__ __forceinline__ void split_tf32(const uint4& v, uint4& hi, uint4& lo)
   split_tf32(v.x, hi.x, lo.x); split_tf32(v.y, hi.y, lo.y); split_tf32(v.z, hi.z, lo.z); split_tf32(v.w, hi.w, lo.w);
 }
 
-template <typename T, int BLOCK_N, int EPI, bool FAST, int CL, bool X3 = false>
-__global__ void __launch_bounds__(RowCfg<(int)sizeof(T), BLOCK_N, EPI, 1, X3>::THREADS, 1)
+// One CTA per SM, persistent over its 128 x BLOCK_N tiles.  Barriers: full (the stage's TMA bytes landed), empty (the
+// MMAs that read the stage retired), conv (X3: the converter warps split the stage's A tile), tfull (an accumulator
+// buffer is complete), tempty (every epilogue thread drained it).
+template <typename T, int BLOCK_N, int EPI, bool FAST, bool X3 = false>
+__global__ void __launch_bounds__(RowCfg<(int)sizeof(T), BLOCK_N, EPI, X3>::THREADS, 1)
 tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmBlo, int M, int N, int K, RowEpi ea) {
   pdl_prologue();
-  using Cfg = RowCfg<(int)sizeof(T), BLOCK_N, EPI, CL, X3>;
+  using Cfg = RowCfg<(int)sizeof(T), BLOCK_N, EPI, X3>;
   constexpr int STAGES = Cfg::STAGES;
   constexpr int KBLK = TcElem<T>::KBLK;
   constexpr int VEC = VecN<T>::N;
@@ -302,63 +295,50 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   uint64_t* bars = (uint64_t*)(gpart + Cfg::GPART_FLOATS);
   uint64_t* full = bars;                 // [STAGES]
   uint64_t* empty = bars + STAGES;       // [STAGES]
-  uint64_t* pfull = bars + 2 * STAGES;   // [STAGES] (CTA pair, leader only)
+  uint64_t* conv = bars + 2 * STAGES;    // [STAGES] X3: the activation tile has been split
   uint64_t* tfull = bars + 3 * STAGES;   // [2]
   uint64_t* tempty = tfull + 2;          // [2]
   uint32_t* tmem_ptr = (uint32_t*)(tempty + 2);
-  uint64_t* conv = pfull;                // [STAGES] X3: the activation tile has been split (pfull is only used by CTA pairs)
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int num_m = (M + TILE_M - 1) / TILE_M, num_n = N / BLOCK_N;
-  const int num_mg = (num_m + CL - 1) / CL;              // groups of CL consecutive row blocks
-  const int total = num_mg * num_n, kblocks = K / KBLK;   // work items per cluster (= per CTA when CL == 1)
-  const int crank = (CL > 1) ? (int)cluster_ctarank() : 0;
-  const int work0 = blockIdx.x / CL, work_stride = gridDim.x / CL;
-  constexpr uint16_t CMASK = (uint16_t)((1u << CL) - 1);
+  const int total = num_m * num_n, kblocks = K / KBLK;
+  const int work0 = blockIdx.x, work_stride = gridDim.x;
 
   if (threadIdx.x == 0) {
     prefetch_tmap(&tmA);
     prefetch_tmap(&tmB);
-    for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); mbar_init(&pfull[i], X3 ? 64 : 1); }
+    for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); mbar_init(&conv[i], X3 ? 64 : 1); }
     if (X3) prefetch_tmap(&tmBlo);
-    // accumulator release: every epilogue thread arrives (single CTA) / lane 0 of every epilogue warp of BOTH CTAs (pair)
-    for (int i = 0; i < 2; ++i) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], CL == 1 ? 32 * Cfg::EPI_WARPS : 2 * Cfg::EPI_WARPS); }
+    // accumulator release: every epilogue thread arrives
+    for (int i = 0; i < 2; ++i) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], 32 * Cfg::EPI_WARPS); }
     fence_barrier_init();
   }
-  if (warp == 2) { if (CL == 1) tmem_alloc(tmem_ptr, Cfg::TMEM_COLS); else tmem_alloc_pair(tmem_ptr, Cfg::TMEM_COLS); }
+  if (warp == 2) tmem_alloc(tmem_ptr, Cfg::TMEM_COLS);
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();      // peer barriers must be initialised before any multicast / remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
 
   if (warp == 0) {
-    // ===================== TMA producer (every CTA: its own A rows, its own share of the B rows) =====================
+    // ===================== TMA producer =====================
     if (lane == 0) {
       int stage = 0; uint32_t phase = 0;
       for (int tile = work0; tile < total; tile += work_stride) {
-        const int m0 = ((tile / num_n) * CL + crank) * TILE_M, n0 = (tile % num_n) * BLOCK_N;
+        const int m0 = (tile / num_n) * TILE_M, n0 = (tile % num_n) * BLOCK_N;
         for (int kb = 0; kb < kblocks; ++kb) {
-          mbar_wait(&empty[stage], phase ^ 1);          // the MMAs that read this slot (in BOTH shared memories) retired
-          if (CL == 1) {
-            mbar_arrive_expect_tx(&full[stage], Cfg::TMA_BYTES);
-            tma_load_2d(A_s + stage * A_STAGE_BYTES, &tmA, &full[stage], kb * KBLK, m0);
-            tma_load_2d(B_s + stage * Cfg::B_STAGE_BYTES, &tmB, &full[stage], kb * KBLK, n0);
-            if (X3) tma_load_2d(BL_s + stage * Cfg::B_STAGE_BYTES, &tmBlo, &full[stage], kb * KBLK, n0);
-          } else {       // both CTAs' loads complete on the LEADER's barrier, which expects the bytes of the whole pair
-            if (crank == 0) mbar_arrive_expect_tx(&full[stage], 2 * Cfg::TMA_BYTES);
-            tma_load_2d_pair(A_s + stage * A_STAGE_BYTES, &tmA, &full[stage], kb * KBLK, m0);
-            tma_load_2d_pair(B_s + stage * Cfg::B_STAGE_BYTES, &tmB, &full[stage], kb * KBLK, n0 + crank * (BLOCK_N / CL));
-          }
+          mbar_wait(&empty[stage], phase ^ 1);          // the MMAs that read this slot retired
+          mbar_arrive_expect_tx(&full[stage], Cfg::TMA_BYTES);
+          tma_load_2d(A_s + stage * A_STAGE_BYTES, &tmA, &full[stage], kb * KBLK, m0);
+          tma_load_2d(B_s + stage * Cfg::B_STAGE_BYTES, &tmB, &full[stage], kb * KBLK, n0);
+          if (X3) tma_load_2d(BL_s + stage * Cfg::B_STAGE_BYTES, &tmBlo, &full[stage], kb * KBLK, n0);
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
       }
     }
-  } else if (warp == 1 && CL > 1 && crank != 0) {
-    // peer CTA: its MMA warp has nothing to do (the leader issues the pair MMAs for both)
   } else if (warp == 1) {
-    // ===================== MMA issuer (the leader CTA of a pair) =====================
-    constexpr uint32_t IDESC = TcElem<T>::idesc(TILE_M * CL, BLOCK_N, 0, 0);
+    // ===================== MMA issuer =====================
+    constexpr uint32_t IDESC = TcElem<T>::idesc(TILE_M, BLOCK_N, 0, 0);
     int stage = 0; uint32_t phase = 0; int it = 0;
     for (int tile = work0; tile < total; tile += work_stride, ++it) {
       // split tf32: ONE accumulator pair per CTA -- columns [0, BLOCK_N) take the hi.hi chain, [BLOCK_N, 2 BLOCK_N) the two
@@ -366,12 +346,12 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       // accumulator costs up to one ulp of it, one-sided, so the small terms must not be chained into the main sum (the
       // epilogue adds the two accumulators once, in round-to-nearest fp32).
       const int acc = X3 ? 0 : (it & 1); const uint32_t aphase = X3 ? (it & 1) : ((it >> 1) & 1);
-      if (CL == 1) mbar_wait(&tempty[acc], aphase ^ 1); else mbar_wait_cluster(&tempty[acc], aphase ^ 1);
+      mbar_wait(&tempty[acc], aphase ^ 1);
       tc_fence_after();
       const uint32_t d_tmem = tmem_base + acc * BLOCK_N;
       for (int kb = 0; kb < kblocks; ++kb) {
         if (X3) mbar_wait(&conv[stage], phase);         // split-tf32: TMA landed AND the converter warps split the A tile
-        else mbar_wait(&full[stage], phase);            // CTA pair: covers the operands of BOTH CTAs
+        else mbar_wait(&full[stage], phase);
         tc_fence_after();
         if (lane == 0) {
           const uint32_t a_addr = smem_u32(A_s + stage * A_STAGE_BYTES), b_addr = smem_u32(B_s + stage * Cfg::B_STAGE_BYTES);
@@ -379,8 +359,7 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           for (int kk = 0; kk < 4; ++kk) {   // one MMA = 32 bytes of K (8 tf32 / 16 bf16) inside the 128-byte swizzle row
             uint64_t ad = smem_desc_sw128(a_addr + kk * 32, 16, 1024);
             uint64_t bd = smem_desc_sw128(b_addr + kk * 32, 16, 1024);
-            if (CL == 1) TcElem<T>::mma(d_tmem, ad, bd, IDESC, (kb | kk) != 0 ? 1u : 0u);
-            else TcElem<T>::mma_pair(d_tmem, ad, bd, IDESC, (kb | kk) != 0 ? 1u : 0u);
+            TcElem<T>::mma(d_tmem, ad, bd, IDESC, (kb | kk) != 0 ? 1u : 0u);
             if constexpr (X3) {              // + lo.hi + hi.lo
               const uint64_t ald = smem_desc_sw128(smem_u32(AL_s + stage * A_STAGE_BYTES) + kk * 32, 16, 1024);
               const uint64_t bld = smem_desc_sw128(smem_u32(BL_s + stage * Cfg::B_STAGE_BYTES) + kk * 32, 16, 1024);
@@ -388,13 +367,8 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               TcElem<T>::mma(d_tmem + BLOCK_N, ad, bld, IDESC, 1u);
             }
           }
-          if (CL == 1) {
-            mma_commit(&empty[stage]);               // smem slot is free once these MMAs retire
-            if (kb == kblocks - 1) mma_commit(&tfull[acc]);
-          } else {                                   // ... in BOTH CTAs; the accumulators of both are complete
-            mma_commit_pair(&empty[stage], CMASK);
-            if (kb == kblocks - 1) mma_commit_pair(&tfull[acc], CMASK);
-          }
+          mma_commit(&empty[stage]);                 // smem slot is free once these MMAs retire
+          if (kb == kblocks - 1) mma_commit(&tfull[acc]);
         }
         __syncwarp();
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
@@ -429,12 +403,10 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int wq = warp & 3;               // TMEM lane quarter this warp may read
     const int sub = ew >> 2;               // which share of the tile's column chunks this warp drains (0..NSUB-1)
     const int half = sub;                  // the 2-warps-per-quarter epilogues: which half of the tile's columns
-    // this warp no longer needs the TMEM accumulator buffer: tell the (leader's) MMA issuer
+    // this warp no longer needs the TMEM accumulator buffer: tell the MMA issuer
     auto release_acc = [&](uint64_t* bar) {
       tc_fence_before();
-      if (CL == 1) { mbar_arrive(bar); return; }
-      __syncwarp();
-      if (lane == 0) { if (crank == 0) mbar_arrive(bar); else mbar_arrive_remote(bar, 0); }
+      mbar_arrive(bar);
     };
     float* stg = stg_all + ew * Cfg::STG_FLOATS_PER_WARP;
     float* coef = coef_all + ew * Cfg::COEF_FLOATS_PER_WARP;
@@ -452,7 +424,7 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     int it = 0;
     for (int tile = work0; tile < total; tile += work_stride, ++it) {
       const int acc = X3 ? 0 : (it & 1); const uint32_t aphase = X3 ? (it & 1) : ((it >> 1) & 1);
-      const int mt = (tile / num_n) * CL + crank, nt = tile % num_n;
+      const int mt = tile / num_n, nt = tile % num_n;
       const int m_base = mt * TILE_M + wq * 32, n0 = nt * BLOCK_N;
       const int m_row = m_base + lane;                     // the row this thread owns in TMEM
       if constexpr (EPI == EPI_BWD) {                      // per-row pooling operands (independent of the accumulator)
@@ -1022,62 +994,27 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();      // nobody exits while a peer may still multicast into / arrive on its shared memory
-  if (warp == 2) { tc_fence_after(); if (CL == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS); else tmem_dealloc_pair(tmem_base, Cfg::TMEM_COLS); }
+  if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem_base, Cfg::TMEM_COLS); }
 }
 
-// ADVMIL_TC_CLUSTER=2 selects the CTA-pair (cta_group::2) variant of the rows kernel, 1 (default) the single-CTA one.
-// Measured on B200 (profiles/exp_tile_width.py, bf16, 262144 rows): with the epilogue removed BOTH variants run the
-// mainloop at 1.40 PFLOP/s on 256-wide tiles (= the measured sustained cuBLAS peak of this pool, 1.13 at 192-wide), and
-// with the epilogue they are within 3 % of each other (pair 1008 / 1184 / 1219 vs single 1052 / 1197 / 1237 TFLOP/s at
-// N = 384 / 512 / 768, K = 1024): operand ingress is not what separates these kernels from the peak, the epilogue's
-// HBM writes and latency are.  The single-CTA variant stays the default; the pair variant is kept tested.
-static int cluster_size() {            // read per launch: tests switch the variant inside one process
-  const char* e = getenv("ADVMIL_TC_CLUSTER");
-  return (e && atoi(e) == 2) ? 2 : 1;
-}
-
+// CTA pairs (tcgen05.mma.cta_group::2, M = 256, each CTA loading half of the weight tile) were measured, no gain: within
+// 3 % of this kernel and mostly slower on B200 (the epilogue's HBM writes and latency bound it, not operand ingress).
 template <typename T, int BLOCK_N, int EPI, bool FAST, bool X3 = false>
 static int launch_rows(const T* A, const T* W, int rows, int K, int N, const RowEpi& ea, cudaStream_t st, const T* Wlo = nullptr) {
-  using Cfg1 = RowCfg<(int)sizeof(T), BLOCK_N, EPI, 1, X3>;
+  using Cfg = RowCfg<(int)sizeof(T), BLOCK_N, EPI, X3>;
   const int num_m = cdiv(rows, TILE_M), num_n = N / BLOCK_N;
-  const int CL = (!X3 && cluster_size() == 2 && num_m >= 2) ? 2 : 1;
   CUtensorMap tmA, tmB, tmBlo;
   ADVMIL_TRY(make_tmap<T>(&tmA, A, rows, K, TILE_M));
-  ADVMIL_TRY(make_tmap<T>(&tmB, W, N, K, BLOCK_N / CL));
-  ADVMIL_TRY(make_tmap<T>(&tmBlo, X3 ? Wlo : W, N, K, BLOCK_N / CL));
+  ADVMIL_TRY(make_tmap<T>(&tmB, W, N, K, BLOCK_N));
+  ADVMIL_TRY(make_tmap<T>(&tmBlo, X3 ? Wlo : W, N, K, BLOCK_N));
   static bool attr_set = false;
   if (!attr_set) {
-    ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(tc_rows_kernel<T, BLOCK_N, EPI, FAST, 1, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg1::SMEM));
-    if constexpr (!X3) {
-      using Cfg2 = RowCfg<(int)sizeof(T), BLOCK_N, EPI, 2>;
-      ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(tc_rows_kernel<T, BLOCK_N, EPI, FAST, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg2::SMEM));
-    }
+    ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(tc_rows_kernel<T, BLOCK_N, EPI, FAST, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
     attr_set = true;
   }
-  if (CL == 1) {
-    const int grid = min(num_m * num_n, sm_count());
-    launch_k(tc_rows_kernel<T, BLOCK_N, EPI, FAST, 1, X3>, dim3(grid), dim3(Cfg1::THREADS), Cfg1::SMEM, st, tmA, tmB, tmBlo, rows, N, K, ea);
-    ADVMIL_CHECK_LAUNCH();
-    return ADVMIL_OK;
-  }
-  if constexpr (!X3) {
-    using Cfg2 = RowCfg<(int)sizeof(T), BLOCK_N, EPI, 2>;
-    const int work = cdiv(num_m, 2) * num_n;
-    const int clusters = min(work, sm_count() / 2);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(clusters * 2);
-    cfg.blockDim = dim3(Cfg2::THREADS);
-    cfg.dynamicSmemBytes = Cfg2::SMEM;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    int M_ = rows, N_ = N, K_ = K;
-    ADVMIL_CHECK_CUDA(cudaLaunchKernelEx(&cfg, tc_rows_kernel<T, BLOCK_N, EPI, FAST, 2>, tmA, tmB, tmBlo, M_, N_, K_, ea));
-    ADVMIL_CHECK_LAUNCH();
-  }
+  const int grid = min(num_m * num_n, sm_count());
+  launch_k(tc_rows_kernel<T, BLOCK_N, EPI, FAST, X3>, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM, st, tmA, tmB, tmBlo, rows, N, K, ea);
+  ADVMIL_CHECK_LAUNCH();
   return ADVMIL_OK;
 }
 

@@ -8,222 +8,15 @@
 // its FLOPs).  One CTA owns 32 or 64 regions and walks the three contractions with the intermediates in shared memory; the
 // weights (192 KB, L2-resident) stream through a double-buffered stage.  The chain is fp32-grade in EVERY precision mode (no
 // tf32 truncation in the discriminator outputs, whose real/fake cancellation amplifies forward errors in the gradients).
-// Two kernels: the default runs on the tensor cores with split tf32 operands (rlip_chain_mma_kernel, below: 84 + 46 us per
-// step for the 32768- and the 16384-region launch); the exact-FFMA kernel it replaced (118 + 58 us) stays as the A/B
-// reference (ADVMIL_RLIP_CHAIN_MMA=0).
-// FFMA kernel: intermediates transposed in shared memory (emb^T / fi^T 34 KB, f1^T 17 KB), a 16-deep weight staging tile.
-// Thread layout as in gemm_simt.cuh: 256 threads, tx = t % 16 owns columns tx*4+j and 64+tx*4+j, ty = t / 16 owns RT rows.
-#include <stdlib.h>
-#include "stages.cuh"
-
-namespace advmil {
-
-namespace {
-
-constexpr int CH_D = 128, CH_DH = 64, CH_BK = 16, CH_THREADS = 256, CH_LDB = 132;
-
-template <int RT>
-struct ChainSmem {
-  static constexpr int TM = 16 * RT, LDT = TM + 4;
-  static constexpr size_t floats = (size_t)CH_D * LDT + (size_t)CH_DH * LDT + 2 * CH_BK * CH_LDB;
-};
-
-// this thread's part of a [NH*64 (n) x 16 (k)] weight tile: W row-major [N, K]; rows n < 64 from W0, n >= 64 from W1
-template <int NH>
-__device__ __forceinline__ void load_b(const float* __restrict__ W0, const float* __restrict__ W1, int K, int k0, int t, float4 (&v)[2]) {
-  const int n = t >> 2, k = k0 + (t & 3) * 4;
-  v[0] = *reinterpret_cast<const float4*>(W0 + (size_t)n * K + k);
-  if (NH == 2) v[1] = *reinterpret_cast<const float4*>(W1 + (size_t)n * K + k);
-}
-template <int NH>
-__device__ __forceinline__ void store_b(float (*S)[CH_LDB], int t, const float4 (&v)[2]) {
-  const int n = t >> 2, k = (t & 3) * 4;
-#pragma unroll
-  for (int i = 0; i < NH; ++i) {
-    S[k + 0][n + 64 * i] = v[i].x; S[k + 1][n + 64 * i] = v[i].y; S[k + 2][n + 64 * i] = v[i].z; S[k + 3][n + 64 * i] = v[i].w;
-  }
-}
-
-// acc[RT][4*NH] = A^T-resident activations (As[k][m], leading dimension LDT) times the streamed weights
-template <int RT, int NH>
-__device__ __forceinline__ void contract(float (&acc)[RT][8], const float* __restrict__ As, int LDT, int K,
-                                         const float* __restrict__ W0, const float* __restrict__ W1,
-                                         float (*Bs)[CH_BK][CH_LDB], int t) {
-  const int tx = t & 15, ty = t >> 4;
-#pragma unroll
-  for (int i = 0; i < RT; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-  float4 rb[2];
-  load_b<NH>(W0, W1, K, 0, t, rb);
-  __syncthreads();                      // the staging tiles (and the activations written by the previous phase) are free / visible
-  store_b<NH>(Bs[0], t, rb);
-  __syncthreads();
-  int buf = 0;
-  for (int k0 = 0; k0 < K; k0 += CH_BK) {
-    const bool more = (k0 + CH_BK) < K;
-    if (more) load_b<NH>(W0, W1, K, k0 + CH_BK, t, rb);
-#pragma unroll
-    for (int kk = 0; kk < CH_BK; ++kk) {
-      float a[RT];
-#pragma unroll
-      for (int i4 = 0; i4 < RT / 4; ++i4) {
-        const float4 av = *reinterpret_cast<const float4*>(As + (size_t)(k0 + kk) * LDT + ty * RT + 4 * i4);
-        a[4 * i4] = av.x; a[4 * i4 + 1] = av.y; a[4 * i4 + 2] = av.z; a[4 * i4 + 3] = av.w;
-      }
-      const float4 b0 = *reinterpret_cast<const float4*>(&Bs[buf][kk][tx * 4]);
-      float b[8] = {b0.x, b0.y, b0.z, b0.w, 0.f, 0.f, 0.f, 0.f};
-      if (NH == 2) {
-        const float4 b1 = *reinterpret_cast<const float4*>(&Bs[buf][kk][64 + tx * 4]);
-        b[4] = b1.x; b[5] = b1.y; b[6] = b1.z; b[7] = b1.w;
-      }
-#pragma unroll
-      for (int i = 0; i < RT; ++i)
-#pragma unroll
-        for (int j = 0; j < 4 * NH; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
-    }
-    if (more) store_b<NH>(Bs[buf ^ 1], t, rb);
-    __syncthreads();
-    buf ^= 1;
-  }
-}
-
-template <int RT, int OCC>
-__global__ void __launch_bounds__(CH_THREADS, OCC)
-rlip_chain_fwd_kernel(const float* __restrict__ emb, const float* __restrict__ F1a_w, const float* __restrict__ F1a_b,
-                      const float* __restrict__ F1b_w, const float* __restrict__ F1b_b, const float* __restrict__ Pg_w,
-                      const float* __restrict__ Pg_b, const float* __restrict__ Ps_w, const float* __restrict__ Ps_b,
-                      const float* __restrict__ Pc_w, int R, Drop dfc1, Drop dga, Drop dgs, float* __restrict__ f1,
-                      float* __restrict__ fi, float* __restrict__ ab, float* __restrict__ part) {
-  pdl_prologue();
-  constexpr int TM = ChainSmem<RT>::TM, LDT = ChainSmem<RT>::LDT, D = CH_D, DH = CH_DH, ABW = 2 * CH_D;
-  extern __shared__ __align__(16) float smem[];
-  float* actT = smem;                                   // [D][LDT]: emb^T, later fi^T
-  float* f1T = actT + (size_t)D * LDT;                  // [DH][LDT]
-  float (*Bs)[CH_BK][CH_LDB] = reinterpret_cast<float (*)[CH_BK][CH_LDB]>(f1T + (size_t)DH * LDT);
-  const int t = threadIdx.x, tx = t & 15, ty = t >> 4, lane = t & 31, warp = t >> 5;
-  const int m0 = blockIdx.x * TM;
-
-  // ---- emb tile -> actT (transposed).  A warp covers 8 rows x 4 float4 (64 B per row): full sectors, 2-way bank conflicts
-  {
-    constexpr int RB = TM / 8, NT = RB * (D / 16);      // (8 rows x 16 columns) sub-tiles
-    const int r_lo = lane & 7, c_lo = lane >> 3;
-    for (int T = warp; T < NT; T += CH_THREADS / 32) {
-      const int row = (T % RB) * 8 + r_lo, c4 = (T / RB) * 4 + c_lo;
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (m0 + row < R) v = *reinterpret_cast<const float4*>(emb + (size_t)(m0 + row) * D + c4 * 4);
-      actT[(size_t)(c4 * 4 + 0) * LDT + row] = v.x; actT[(size_t)(c4 * 4 + 1) * LDT + row] = v.y;
-      actT[(size_t)(c4 * 4 + 2) * LDT + row] = v.z; actT[(size_t)(c4 * 4 + 3) * LDT + row] = v.w;
-    }
-  }
-  float acc[RT][8];
-
-  // ---- phase 1: f1 = dropout(relu(emb F1a^T + b)), 64 columns ----
-  contract<RT, 1>(acc, actT, LDT, D, F1a_w, nullptr, Bs, t);
-  {
-    const int n = tx * 4;
-    const float4 bv = *reinterpret_cast<const float4*>(F1a_b + n);
-    const float bias[4] = {bv.x, bv.y, bv.z, bv.w};
-    float o[RT][4];
-#pragma unroll
-    for (int i = 0; i < RT; ++i) {
-      const int m = m0 + ty * RT + i;
-      bool k[4] = {true, true, true, true};
-      if (dfc1.active && m < R) { dfc1.keep2(m, n, k[0], k[1]); dfc1.keep2(m, n + 2, k[2], k[3]); }
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        float v = fmaxf(acc[i][j] + bias[j], 0.f);
-        if (dfc1.active) v = k[j] ? v * dfc1.inv_keep : 0.f;
-        o[i][j] = v;
-      }
-      if (m < R) *reinterpret_cast<float4*>(f1 + (size_t)m * DH + n) = make_float4(o[i][0], o[i][1], o[i][2], o[i][3]);
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-#pragma unroll
-      for (int i4 = 0; i4 < RT / 4; ++i4)
-        *reinterpret_cast<float4*>(f1T + (size_t)(n + j) * LDT + ty * RT + 4 * i4) =
-            make_float4(o[4 * i4][j], o[4 * i4 + 1][j], o[4 * i4 + 2][j], o[4 * i4 + 3][j]);
-    }
-  }
-
-  // ---- phase 2: fi = f1 F1b^T + b, 128 columns; fi^T replaces emb^T ----
-  contract<RT, 2>(acc, f1T, LDT, DH, F1b_w, F1b_w + (size_t)64 * DH, Bs, t);
-  {
-#pragma unroll
-    for (int jh = 0; jh < 2; ++jh) {
-      const int n = jh * 64 + tx * 4;
-      const float4 bv = *reinterpret_cast<const float4*>(F1b_b + n);
-      const float bias[4] = {bv.x, bv.y, bv.z, bv.w};
-#pragma unroll
-      for (int i = 0; i < RT; ++i) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][jh * 4 + j] += bias[j];
-        const int m = m0 + ty * RT + i;
-        if (m < R)
-          *reinterpret_cast<float4*>(fi + (size_t)m * D + n) = make_float4(acc[i][jh * 4], acc[i][jh * 4 + 1], acc[i][jh * 4 + 2], acc[i][jh * 4 + 3]);
-      }
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-#pragma unroll
-        for (int i4 = 0; i4 < RT / 4; ++i4)
-          *reinterpret_cast<float4*>(actT + (size_t)(n + j) * LDT + ty * RT + 4 * i4) =
-              make_float4(acc[4 * i4][jh * 4 + j], acc[4 * i4 + 1][jh * 4 + j], acc[4 * i4 + 2][jh * 4 + j], acc[4 * i4 + 3][jh * 4 + j]);
-      }
-    }
-  }
-
-  // ---- phase 3: the gate, 64 (tanh_j, sigmoid_j) pairs per pass; same conventions as EpiGate (gemm_simt.cuh) ----
-  const bool hashed = dga.active && !dga.mask && !dgs.mask;
-#pragma unroll 1
-  for (int c = 0; c < D / 64; ++c) {
-    contract<RT, 2>(acc, actT, LDT, D, Pg_w + (size_t)c * 64 * D, Ps_w + (size_t)c * 64 * D, Bs, t);
-    const int j0 = c * 64 + tx * 4;
-    const float4 ba4 = *reinterpret_cast<const float4*>(Pg_b + j0), bb4 = *reinterpret_cast<const float4*>(Ps_b + j0);
-    const float4 wc4 = *reinterpret_cast<const float4*>(Pc_w + j0);
-    const float ba[4] = {ba4.x, ba4.y, ba4.z, ba4.w}, bb[4] = {bb4.x, bb4.y, bb4.z, bb4.w}, wc[4] = {wc4.x, wc4.y, wc4.z, wc4.w};
-#pragma unroll
-    for (int i = 0; i < RT; ++i) {
-      const int m = m0 + ty * RT + i;
-      float partial = 0.f, av[4], bv[4];
-      uint32_t h = 0;
-      if (hashed) h = dga.bits(m, j0);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float a = tanhf(acc[i][j] + ba[j]);
-        const float b = sigmoidf_(acc[i][4 + j] + bb[j]);
-        av[j] = a; bv[j] = b;
-        float ad = a, bd = b;
-        if (dga.active && m < R) {
-          bool ka, kb;
-          if (hashed) { ka = ((h >> (8 * j)) & 0xFFu) >= dga.thresh8j; kb = true; }
-          else gate_keep(dga, dgs, m, j0 + j, ka, kb);
-          ad = ka ? a * dga.inv_keep : 0.f;
-          bd = kb ? b * dgs.inv_keep : 0.f;
-          if (!(ka && kb)) bv[j] = -b;          // joint keep bit in the sign of the stored sigmoid
-        }
-        partial = fmaf(ad * bd, wc[j], partial);
-      }
-      partial = half_warp_sum(partial);
-      if (m < R) {
-        if (ab) {
-          *reinterpret_cast<float4*>(ab + (size_t)m * ABW + c * 128 + tx * 4) = make_float4(av[0], av[1], av[2], av[3]);
-          *reinterpret_cast<float4*>(ab + (size_t)m * ABW + c * 128 + 64 + tx * 4) = make_float4(bv[0], bv[1], bv[2], bv[3]);
-        }
-        if (tx == 0) part[(size_t)c * R + m] = partial;
-      }
-    }
-  }
-}
-
-// =============================================================================================
-// Tensor-core variant of the same chain: warp-level mma.sync m16n8k8 tf32 with SPLIT operands ("3xTF32").  Every fp32
+//
+// The contractions run on the tensor cores as warp-level mma.sync m16n8k8 tf32 with SPLIT operands ("3xTF32").  Every fp32
 // operand is split in registers into hi = rna_tf32(x) and lo = x - hi (exact in fp32; the tensor core reads its top 19
 // bits), each K step issues lo.hi + hi.lo into a small-term accumulator and hi.hi into the main one (the tensor core's
 // fp32 accumulation truncates, so the small terms are never chained into the large sum), and the epilogue adds the two
 // once in round-to-nearest fp32: products are exact to ~2^-21 relative, i.e. fp32-grade, in every precision mode.
-// The FFMA kernel above tops out at the FFMA rate (128 MAC / clk / SM at ~50 % pipe utilisation); the warp-level tf32 MMA
+// An exact-FFMA kernel tops out at the FFMA rate (128 MAC / clk / SM at ~50 % pipe utilisation); the warp-level tf32 MMA
 // does 512 MAC / clk / SM, i.e. 1.33x the FFMA peak after the three-fold split, with a tenth of the issue slots.
+// FFMA chain (118 + 58 us against 84 + 46 us on B200): measured, slower, removed.
 //
 // One CTA = 32 x WM regions with WM x 4 warps as WM (rows) x 4 (columns): a warp owns 32 rows (two 16-row MMA tiles) and a
 // quarter of the output columns of the phase.  Activations stay row-major in shared memory (stride K + 4 floats: the
@@ -233,7 +26,14 @@ rlip_chain_fwd_kernel(const float* __restrict__ emb, const float* __restrict__ F
 // of the SAME columns, so that a thread holds both halves of each (tanh_j, sigmoid_j) pair in matching fragment slots.
 // Measured (ncu, B200): 84 us for 32768 regions with <WM, KC> = <1, 16> (4 CTAs per SM), 46 us for 16384 regions with <2, 32>
 // (2 CTAs per SM); legacy tensor pipe 43-47 % busy, HMMA.1688.F32.TF32 at ~10.6 cycles per instruction and sub-core.
-// =============================================================================================
+#include "stages.cuh"
+
+namespace advmil {
+
+namespace {
+
+constexpr int CH_D = 128, CH_DH = 64;
+
 namespace mm {
 constexpr int LDA = CH_D + 4, LDF = CH_DH + 4, WROWS = 128;
 // WM = warp rows per CTA (a warp owns 32 regions): 64 regions / 256 threads or 32 regions / 128 threads; KC = K extent of a
@@ -244,7 +44,7 @@ struct Cfg {
   static constexpr int TM = 32 * WM, THREADS = 128 * WM, LDW = KC + 4;
   static constexpr int NC1 = CH_D / KC, NC2 = CH_DH / KC, NCHUNK = 3 * NC1 + NC2;
   static constexpr size_t SMEM_FLOATS = (size_t)TM * LDA + (size_t)TM * LDF + 2 * (size_t)WROWS * LDW + 2 * 4 * TM;
-  static constexpr int MIN_CTAS = WM == 2 ? 2 : (KC == 32 ? 3 : 4);
+  static constexpr int MIN_CTAS = WM == 2 ? 2 : 4;
 };
 
 __device__ __forceinline__ void split3(float x, uint32_t& hi, uint32_t& lo) {
@@ -430,7 +230,7 @@ rlip_chain_mma_kernel(const float* __restrict__ emb, const float* __restrict__ F
   }
 
   // ---- phase 3: the gate, 64 (tanh_j, sigmoid_j) pairs per block; n-tiles 0,1 = tanh columns, 2,3 = the sigmoid columns of
-  //      the same pairs.  Conventions as in the FFMA kernel / EpiGate (gemm_simt.cuh) ----
+  //      the same pairs.  Conventions as in EpiGate (gemm_simt.cuh) ----
   const bool hashed = dga.active && !dga.mask && !dgs.mask;
 #pragma unroll 1
   for (int c = 0; c < D / 64; ++c) {
@@ -517,54 +317,18 @@ static int launch_chain_mma(const float* emb, const AdvmilDiscParams& p, int R, 
 
 }  // namespace
 
-bool rlip_chain_supported(int d) {
-  static int enabled = -1;
-  if (enabled < 0) { const char* e = getenv("ADVMIL_RLIP_CHAIN"); enabled = (e && atoi(e) == 0) ? 0 : 1; }
-  return enabled && d == CH_D;
-}
-
-template <int RT, int OCC>
-static int launch_chain(const float* emb, const AdvmilDiscParams& p, int R, const Drop& dfc1, const Drop& dga, const Drop& dgs,
-                        float* f1, float* fi, float* ab, float* part, cudaStream_t st) {
-  const size_t smem = ChainSmem<RT>::floats * sizeof(float);
-  static bool attr_set[64] = {};
-  int dev = 0;
-  ADVMIL_CHECK_CUDA(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(rlip_chain_fwd_kernel<RT, OCC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (dev >= 0 && dev < 64) attr_set[dev] = true;
-  }
-  launch_k(rlip_chain_fwd_kernel<RT, OCC>, dim3(cdiv(R, ChainSmem<RT>::TM)), dim3(CH_THREADS), smem, st, emb, p.F1a_w, p.F1a_b, p.F1b_w,
-           p.F1b_b, p.Pg_w, p.Pg_b, p.Ps_w, p.Ps_b, p.Pc_w, R, dfc1, dga, dgs, f1, fi, ab, part);
-  ADVMIL_CHECK_LAUNCH();
-  return ADVMIL_OK;
-}
+bool rlip_chain_supported(int d) { return d == CH_D; }
 
 int rlip_chain_fwd(const float* emb, const AdvmilDiscParams& p, int R, const Drop& dfc1, const Drop& dga, const Drop& dgs,
                    float* f1, float* fi, float* ab, float* part, cudaStream_t st) {
   ADVMIL_REQUIRE(p.d == CH_D, "rlip_chain_fwd: d=%d unsupported", p.d);
   if (R == 0) return ADVMIL_OK;
-  // ADVMIL_RLIP_CHAIN_MMA: 0 = the FFMA kernel; 1 / 2 / 3 = one tensor-core variant for every launch (A/B tests); default:
   // 64-region CTAs while they fit one wave of 2 CTAs per SM (R = 16384: 46 us against 49 us), 32-region CTAs with 16-deep
   // weight stages (4 CTAs per SM) beyond that (the batched real + fake launch, 2R = 32768: 86 us against 91 us)
-  static int use_mma = -1, sms = 0;
-  if (use_mma < 0) { const char* e = getenv("ADVMIL_RLIP_CHAIN_MMA"); use_mma = e ? atoi(e) : 4; }
+  static int sms = 0;
   if (!sms) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); if (sms <= 0) sms = 148; }
-  if (use_mma == 4) {
-    if (cdiv(R, 64) <= 2 * sms) return mm::launch_chain_mma<2, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-    return mm::launch_chain_mma<1, 16>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-  }
-  if (use_mma == 1) return mm::launch_chain_mma<2, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-  if (use_mma == 2) return mm::launch_chain_mma<1, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-  if (use_mma == 3) return mm::launch_chain_mma<1, 16>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-  static int rt = 0, occ = 0;
-  if (rt == 0) {       // A/B knobs: ADVMIL_RLIP_CHAIN_RT=8 -> 128 regions per CTA; ADVMIL_RLIP_CHAIN_OCC=3 -> 3 CTAs per SM (80 registers; measured 4 % slower)
-    const char* e = getenv("ADVMIL_RLIP_CHAIN_RT"); rt = (e && atoi(e) == 8) ? 8 : 4;
-    const char* o = getenv("ADVMIL_RLIP_CHAIN_OCC"); occ = (o && atoi(o) == 3) ? 3 : 2;
-  }
-  if (rt == 8) return launch_chain<8, 1>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-  if (occ == 2) return launch_chain<4, 2>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-  return launch_chain<4, 3>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
+  if (cdiv(R, 64) <= 2 * sms) return mm::launch_chain_mma<2, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
+  return mm::launch_chain_mma<1, 16>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
 }
 
 }  // namespace advmil

@@ -16,7 +16,8 @@ static inline int region_precision(int precision, bool exact) {
   if (precision == ADVMIL_TF32X3) return ADVMIL_TF32X3;
   return exact ? ADVMIL_TF32X3 : ADVMIL_TF32;      // bf16 mode
 }
-// ESAT self-attention: FFMA kernels in the exact modes (fp32, split tf32), warp-level tf32 tensor-core kernels otherwise
+// ESAT self-attention: FFMA kernels in the exact modes (fp32, split tf32), tcgen05 tf32 kernels otherwise (esat_kernels.cu:
+// head widths other than 16 / 32 / 48 / 64 also run the FFMA kernels)
 static inline int attention_precision(int precision) {
   return (precision == ADVMIL_FP32 || precision == ADVMIL_TF32X3) ? ADVMIL_FP32 : ADVMIL_TF32;
 }

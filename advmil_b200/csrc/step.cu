@@ -6,7 +6,6 @@
 //  * the D-step generator forward (eval) and the G-step generator forward (train) share relu(x W1^T + b1): the projection
 //    kernel of the D phase writes both the eval activations and the G step's dropped copy (its seed is known up front);
 //  * the G step asks D only for dL/dt and never touches D-parameter gradients.
-#include <stdlib.h>
 #include <mutex>
 #include <vector>
 #include "stages.cuh"
@@ -58,7 +57,7 @@ static size_t gen_bufs_bytes(const AdvmilGenParams& g, size_t rows, size_t nb) {
 // After the eval projection exists, the train-mode generator forward of the G step (dropout on the cached projection, gate
 // GEMM, pooling, head) depends on nothing the D phase still has to do, while the D phase's head forward/backward is a
 // chain of small region-level kernels that leaves most SMs idle.  The disc call therefore issues that forward on a side
-// stream; the gen call joins it.  ADVMIL_STEP_OVERLAP=0 disables the fork (the gen call then runs the forward itself).
+// stream; the gen call joins it.
 struct SideState {
   static constexpr int SLOTS = 4;       // engines (workspaces) with a forked forward in flight at the same time
   cudaStream_t stream = nullptr;
@@ -72,18 +71,13 @@ struct SideState {
 static constexpr int MAX_DEVICES = 64;
 static SideState g_side[MAX_DEVICES];
 static std::mutex g_side_mu;
-static int g_side_enabled = -1;
 static int side_get(SideState** out) {
   *out = nullptr;
-  if (g_side_enabled < 0) {
-    const char* e = getenv("ADVMIL_STEP_OVERLAP");
-    g_side_enabled = (e && atoi(e) == 0) ? 0 : 1;
-  }
   int dev = 0;
   ADVMIL_CHECK_CUDA(cudaGetDevice(&dev));
   if (dev < 0 || dev >= MAX_DEVICES) return ADVMIL_OK;     // no overlap on an out-of-range ordinal: the gen call runs the forward
   SideState& s = g_side[dev];
-  if (g_side_enabled && !s.stream) {
+  if (!s.stream) {
     ADVMIL_CHECK_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
     ADVMIL_CHECK_CUDA(cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming));
     for (int i = 0; i < SideState::SLOTS; ++i) ADVMIL_CHECK_CUDA(cudaEventCreateWithFlags(&s.done[i], cudaEventDisableTiming));
@@ -169,7 +163,7 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   std::lock_guard<std::mutex> side_lock(g_side_mu);
   SideState* side = nullptr;
   ADVMIL_TRY(side_get(&side));
-  if (side && side->stream) {
+  if (side) {
     // a gen call never came for this workspace (exception between the phases): the forked forward may still be reading
     // and writing the persistent region -- the new step must not overwrite it before that forward has drained
     const int old = side->find(a->workspace);
@@ -190,9 +184,7 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   STEP_TAKE(y_pre, char, (size_t)rows * d * es);
   AdvmilEmbedActs ea{};
   ea.emb = emb2; ea.y_pre = y_pre; ea.precision = a->precision;
-  const char* fuse_env = getenv("ADVMIL_FUSE_PROJ_EMBED");          // "0" = separate K1 and K5 launches (debugging / A-B tests)
-  const int fuse_pe = (fuse_env && atoi(fuse_env) == 0) ? 0 : 1;
-  const bool fused = fuse_pe && gp.C == dp.C && proj_embed_supported(rows, gp.C, gp.h, d, a->precision);
+  const bool fused = gp.C == dp.C && proj_embed_supported(rows, gp.C, gp.h, d, a->precision);
   if (fused) {     // K1 and K5+K6 read the same x: one pass over stacked weights, then the generator forward skips K1
     for (int i = 0; i < nb; ++i)
       ADVMIL_REQUIRE((bags->offsets_host[i + 1] - bags->offsets_host[i]) % 16 == 0,
@@ -206,8 +198,8 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   ADVMIL_TRY(advmil_generator_fwd(&gp, bags, &ga, stream));
   if (!fused) ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, stream));
   // ---- fork: the G step's train-mode generator forward runs on the side stream from here on ----
-  const int slot = (side && side->stream) ? side->find(nullptr) : -1;      // no free slot: the gen call runs the forward itself
-  if (g_side_enabled && slot >= 0 && a->gen_grads && a->pred_g && a->noise_g) {
+  const int slot = side ? side->find(nullptr) : -1;      // no free slot: the gen call runs the forward itself
+  if (slot >= 0 && a->gen_grads && a->pred_g && a->noise_g) {
     ADVMIL_CHECK_CUDA(cudaEventRecord(side->fork, st));
     ADVMIL_CHECK_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
     AdvmilGenActs gt;
@@ -269,7 +261,7 @@ extern "C" int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream) {
   std::unique_lock<std::mutex> side_lock(g_side_mu);
   SideState* side = nullptr;
   ADVMIL_TRY(side_get(&side));
-  const int slot = (side && side->stream) ? side->find(a->workspace) : -1;
+  const int slot = side ? side->find(a->workspace) : -1;
   if (slot >= 0) {
     ADVMIL_CHECK_CUDA(cudaStreamWaitEvent(st, side->done[slot], 0));
     side->pending_ws[slot] = nullptr;

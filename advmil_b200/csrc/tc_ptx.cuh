@@ -40,29 +40,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   __trap();
 }
 
-// wait on a barrier that peer CTAs arrive on (cluster-scope acquire)
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t addr = smem_u32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; spin < (1u << 26); ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (done) return;
-  }
-  __trap();
-}
-// arrive on the barrier at the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint64_t* local_bar, uint32_t rank) {
-  uint32_t ra;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(local_bar)), "r"(rank));
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(ra) : "memory");
-}
-
 // ---- TMA ----------------------------------------------------------------------------------------
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)m) : "memory");
@@ -74,35 +51,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
           smem_u32(smem_dst)),
       "l"((uint64_t)m), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
-}
-
-// CTA-pair load: lands in THIS CTA's shared memory, completes its bytes on the mbarrier at the same offset in the pair's
-// leader CTA (rank 0), which is the one that issues the pair MMA
-__device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorMap* m, uint64_t* local_bar, int c0, int c1) {
-  uint32_t lead_bar;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(lead_bar) : "r"(smem_u32(local_bar)), "r"(0));
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-          smem_u32(smem_dst)),
-      "l"((uint64_t)m), "r"(lead_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-
-// same, multicast to every CTA of the cluster named in cta_mask (same CTA-relative smem offset and mbarrier offset)
-__device__ __forceinline__ void tma_load_2d_mcast(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1,
-                                                  uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], "
-      "[%2], %5;" ::"r"(smem_u32(smem_dst)),
-      "l"((uint64_t)m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
-      : "memory");
-}
-
-// ---- clusters -------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 
 // ---- tcgen05 --------------------------------------------------------------------------------------
@@ -138,48 +86,6 @@ __device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint64_t adesc, uint64_
 // arrives on the mbarrier once all previously issued MMAs of this thread have completed
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// same, arriving on the barrier at this offset in every CTA of cta_mask
-__device__ __forceinline__ void mma_commit_mcast(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(cta_mask)
-               : "memory");
-}
-
-// ---- CTA-pair (cta_group::2) variants: one MMA spans the two SMs of a cluster (M = 256), each CTA supplies its 128 rows
-// of A and HALF of the B tile from its own shared memory, and holds its 128 accumulator rows in its own TMEM ------------
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result, uint32_t ncols) {   // one warp in EACH CTA of the pair
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)), "r"(ncols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void mma_tf32_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mma_f16_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrives (once all previously issued pair MMAs retired) on the barrier at this offset in every CTA of cta_mask
-__device__ __forceinline__ void mma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(cta_mask)
-               : "memory");
 }
 
 // TMEM -> registers: this warp's 32 lanes x 32 consecutive fp32 columns (thread i gets lane i's row)

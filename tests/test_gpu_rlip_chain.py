@@ -1,61 +1,18 @@
 """Region-level chain of the RLIP head (csrc/rlip_chain.cu; reference model/model_utils.py:202-210 and
-model/backbone_utils.py:47-56): every kernel variant -- the exact-FFMA kernel (ADVMIL_RLIP_CHAIN_MMA=0) and the three
-tensor-core tilings (1: 64-region CTAs, 2: 32-region CTAs with 32-deep weight stages, 3: 32-region CTAs with 16-deep
-stages) -- against the CPU oracle on region counts that leave ragged tiles (1, 37, 100 and 165 regions), eval and train
-(injected masks).  The variant is read once per process, so each runs in its own interpreter."""
-import os
-import subprocess
-import sys
-import tempfile
-
+model/backbone_utils.py:47-56).  rlip_chain_fwd runs one of two tilings chosen by the region count of the launch: 64-region
+CTAs while the launch fits two of them per SM, 32-region CTAs beyond.  Both are checked against the CPU oracle (eval and
+train with injected masks; outputs, dt and every D gradient): the 64-region tiling on region counts that leave ragged tiles
+(1, 37, 100 and 165 regions), the 32-region tiling on a count above the threshold.  The two tilings are also compared with
+each other on the same bag, once alone and once packed with a bag that pushes the launch over the threshold."""
 import numpy as np
 import pytest
+import torch
 
-pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-CHILD = r"""
-import sys, numpy as np, torch
-sys.path.insert(0, %(root)r)
+from advmil_b200 import ops
 from oracle import advmil_oracle as O
 from tests.util import build_D, d_masks, to_dev_masks
-out = {}
-for N, train, seed in ((16, True, 3), (592, False, 4), (1600, True, 5), (2640, True, 6)):
-    sd = O.synth_state_dict(O.D_SHAPES(1024, 128, (64, 128)), seed + 50)
-    D = build_D(1024, 128, "instance", "x")
-    D.load_state_dict({k: v.clone() for k, v in sd.items()})
-    x = O.synth_bag(N, seed, 1024)
-    masks = d_masks(N // 16, 128, seed * 10 + 5) if train else None
-    D.train(train)
-    if train:
-        D._inject_masks = to_dev_masks(masks)
-    t = torch.tensor([[0.41]], device="cuda", requires_grad=True)
-    o = D(x.cuda().unsqueeze(0), t)
-    o.sum().backward()
-    out["out.%%d" %% N] = o.detach().cpu().numpy()
-    out["dt.%%d" %% N] = t.grad.cpu().numpy()
-    for k, p in D.named_parameters():
-        out["g.%%d.%%s" %% (N, k)] = p.grad.detach().cpu().numpy()
-    if %(with_oracle)d:
-        sdr = {k: v.clone().requires_grad_(True) for k, v in sd.items()}
-        t2 = torch.tensor([[0.41]], requires_grad=True)
-        od = O.prjdisc_forward(sdr, x, t2, masks, "instance", "x")
-        od["out"].sum().backward()
-        out["ref.out.%%d" %% N] = od["out"].detach().numpy()
-        out["ref.dt.%%d" %% N] = t2.grad.numpy()
-        for k, v in sdr.items():
-            if v.grad is not None:
-                out["ref.g.%%d.%%s" %% (N, k)] = v.grad.numpy()
-np.savez(%(path)r, **out)
-"""
 
-
-def _run(variant, path, with_oracle):
-    env = dict(os.environ, ADVMIL_RLIP_CHAIN_MMA=str(variant))
-    code = CHILD % {"root": ROOT, "path": path, "with_oracle": int(with_oracle)}
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-2000:]
-    return dict(np.load(path))
+pytestmark = pytest.mark.gpu
 
 
 def _close(a, e, rtol, name, atol=0.0):
@@ -65,33 +22,54 @@ def _close(a, e, rtol, name, atol=0.0):
     assert not (err > tol).any(), f"{name}: max err {err.max():.3e} (scale {scale:.3e})"
 
 
+def _vs_oracle(N, train, seed, C=1024):
+    sd = O.synth_state_dict(O.D_SHAPES(C, 128, (64, 128)), seed + 50)
+    D = build_D(C, 128, "instance", "x")
+    D.load_state_dict({k: v.clone() for k, v in sd.items()})
+    x = O.synth_bag(N, seed, C)
+    masks = d_masks(N // 16, 128, seed * 10 + 5) if train else None
+    D.train(train)
+    if train:
+        D._inject_masks = to_dev_masks(masks)
+    t = torch.tensor([[0.41]], device="cuda", requires_grad=True)
+    o = D(x.cuda().unsqueeze(0), t)
+    o.sum().backward()
+    got = {"out": o.detach().cpu().numpy(), "dt": t.grad.cpu().numpy()}
+    got.update({"g." + k: p.grad.detach().cpu().numpy() for k, p in D.named_parameters()})
+
+    sdr = {k: v.clone().requires_grad_(True) for k, v in sd.items()}
+    t2 = torch.tensor([[0.41]], requires_grad=True)
+    od = O.prjdisc_forward(sdr, x, t2, masks, "instance", "x")
+    od["out"].sum().backward()
+    ref = {"out": od["out"].detach().numpy(), "dt": t2.grad.numpy()}
+    ref.update({"g." + k: v.grad.numpy() for k, v in sdr.items() if v.grad is not None})
+
+    # fp32 mode: 1e-5, norm-wise per tensor; gradients that cancel to ~0 are skipped as in
+    # test_gpu_parity_modules._cmp_grads; the same rule: |a - e| <= 1e-5 (|e| + max|e|) + one fp32 ulp of the network's
+    # largest gradient entry (tests/util.py)
+    floor = max(2.0 ** -23 * float(np.abs(v).max()) for k, v in ref.items() if k.startswith("g."))
+    for k, e in ref.items():
+        if float(np.abs(e).max()) < 1e-7:
+            continue
+        _close(got[k], e, 1e-5, f"N={N} train={train}: {k}", atol=floor if k.startswith("g.") else 0.0)
+
+
 def test_chain_variants_agree_with_the_oracle_and_with_each_other():
-    with tempfile.TemporaryDirectory() as td:
-        res = {v: _run(v, os.path.join(td, f"v{v}.npz"), with_oracle=(v == 0)) for v in (0, 1, 2, 3)}
-    ref = res[0]
-    names = [k for k in ref if not k.startswith("ref.")]
-    # every variant against the oracle (fp32 mode: 1e-5, norm-wise per tensor; gradients that cancel to ~0 are skipped as in
-    # test_gpu_parity_modules._cmp_grads;
-    # the same rule: |a - e| <= 1e-5 (|e| + max|e|) + one fp32 ulp of the network's largest gradient entry, tests/util.py)
-    floors = {}
-    for k in ref:
-        if k.startswith("ref.g."):
-            n = k.split(".")[2]
-            floors[n] = max(floors.get(n, 0.0), 2.0 ** -23 * float(np.abs(ref[k]).max()))
-    for v, r in res.items():
-        for k in names:
-            e = ref.get("ref." + k)
-            if e is None or float(np.abs(e).max()) < 1e-7:
-                continue
-            _close(r[k], e, 1e-5, f"variant {v} vs oracle: {k}", atol=floors[k.split(".")[1]] if k.startswith("g.") else 0.0)
-    # the tensor-core variants against the exact-FFMA kernel: forward outputs to fp32 rounding of their O(0.1 - 1) terms (the
-    # instance inner product and the projection nearly cancel in out; same absolute floor as test_discriminator_vs_oracle)
-    for v in (1, 2, 3):
-        for k in names:
-            if k.startswith("out"):
-                _close(res[v][k], ref[k], 1e-5, f"variant {v} vs FFMA: {k}", atol=1e-5 * 1e-2)
-    # the three tilings run the same arithmetic on different CTA shapes
-    for v in (2, 3):
-        for k in names:
-            if k.startswith("out"):
-                _close(res[v][k], res[1][k], 1e-5, f"variant {v} vs variant 1: {k}", atol=1e-5 * 1e-2)
+    for N, train, seed in ((16, True, 3), (592, False, 4), (1600, True, 5), (2640, True, 6)):
+        _vs_oracle(N, train, seed)
+    # above the threshold (cdiv(R, 64) > 2 * SMs): the 32-region tiling; 64 input features keep the oracle cheap
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    R_big = 2 * sms * 64 + 37
+    _vs_oracle(16 * R_big, True, 7, C=64)
+
+    # the same 165-region bag through both tilings: alone (64-region CTAs), then first in a launch that also holds R_big
+    # regions (32-region CTAs); forward outputs to fp32 rounding (same absolute floor as test_discriminator_vs_oracle)
+    C = 64
+    D = build_D(C, 128, "instance", "x").eval()
+    D.load_state_dict(O.synth_state_dict(O.D_SHAPES(C, 128, (64, 128)), 58))
+    x = O.synth_bag(2640, 8, C).cuda()
+    filler = O.synth_bag(16 * R_big, 9, C).cuda()
+    with torch.no_grad():
+        alone = D.forward_packed(ops.PackedBags.from_single(x), torch.tensor([[0.41]], device="cuda")).reshape(-1)
+        packed = D.forward_packed(ops.PackedBags.from_list([x, filler]), torch.tensor([[0.41], [0.7]], device="cuda")).reshape(-1)
+    _close(packed[:1].cpu().numpy(), alone.cpu().numpy(), 1e-5, "64-region vs 32-region tiling", atol=1e-5 * 1e-2)

@@ -114,30 +114,3 @@ def test_tf32_mode_generator_and_discriminator_vs_oracle(N, train):
                 assert_close(p.grad.cpu(), ref[k].grad, 2e-2, "grad " + k, atol=2e-5 * gmax)
     finally:
         advmil_b200.set_precision("fp32")
-
-
-@pytest.mark.parametrize("precision", ["tf32", "bf16"])
-def test_cta_pair_variant_equals_single_cta(monkeypatch, precision):
-    """ADVMIL_TC_CLUSTER=2 runs the rows kernel as CTA pairs (tcgen05.mma.cta_group::2, M = 256, each CTA holding half of
-    the weight tile): same contraction order per output element, so every epilogue must reproduce the single-CTA results."""
-    prec = ops.PRECISIONS[precision]
-    g = torch.Generator(device="cuda").manual_seed(11)
-    rows = 1000                       # 8 row blocks: 4 pairs, the last block ragged
-    x = torch.randn(rows, 1024, device="cuda", generator=g)
-    W = torch.randn(384, 1024, device="cuda", generator=g) / 32
-    b = torch.randn(384, device="cuda", generator=g)
-    v = torch.randn(rows, 384, device="cuda", generator=g)
-    Wa, Wb = [torch.randn(384, 384, device="cuda", generator=g) / 20 for _ in range(2)]
-    ba, bb, wc = [torch.randn(384, device="cuda", generator=g) * 0.1 for _ in range(3)]
-    bc = torch.randn(1, device="cuda", generator=g)
-    dY = torch.randn(rows, 384, device="cuda", generator=g)
-    res = {}
-    for cl in ("1", "2"):
-        monkeypatch.setenv("ADVMIL_TC_CLUSTER", cl)
-        y = ops.linear_forward(x, W, b, act=1, p_drop=0.25, seed=3, train=True, precision=prec)
-        s, ab = ops.gated_score_forward(v, Wa, ba, Wb, bb, wc, bc, p_drop=0.25, seed=5, train=True, precision=prec)
-        dX, _, _ = ops.linear_backward(dY, None, W, need_dw=False, need_db=False, precision=prec)
-        torch.cuda.synchronize()
-        res[cl] = (y.float(), s, ab.float(), dX.float())
-    for a_, b_ in zip(res["1"], res["2"]):
-        assert torch.equal(a_, b_)
