@@ -49,7 +49,7 @@ DISC_TENSORS = ["Wc", "bc", "ln_g", "ln_b", "F1a_w", "F1a_b", "F1b_w", "F1b_b", 
 class DiscParams(C.Structure):
     _fields_ = [(n, c_fp) for n in DISC_TENSORS] + [
         ("C", C.c_int32), ("d", C.c_int32), ("t1", C.c_int32), ("t2", C.c_int32),
-        ("inner_instance", C.c_int32), ("prj_path", C.c_int32), ("p", C.c_float), ("ln_eps", C.c_float)]
+        ("inner_instance", C.c_int32), ("prj_path", C.c_int32), ("p", C.c_float), ("ln_eps", C.c_float), ("ksize", C.c_int32)]
 
 
 class DiscGrads(C.Structure):

@@ -248,15 +248,23 @@ extern "C" int advmil_generator_sample(const AdvmilGenParams* p, const float* H,
 // =============================================================================================
 // discriminator
 // =============================================================================================
+// the patch embedding's kernel size: 1 (ksize 0 = the ABI's zero default) or 3
+static int disc_ksize(const AdvmilDiscParams* p) { return p->ksize == 0 ? 1 : p->ksize; }
+static int check_ksize(const AdvmilDiscParams* p) {
+  ADVMIL_REQUIRE(p->ksize == 0 || p->ksize == 1 || p->ksize == 3, "disc: patch-embedding ksize %d unsupported (0, 1 or 3)", p->ksize);
+  return ADVMIL_OK;
+}
+
 extern "C" size_t advmil_disc_workspace_bytes(const AdvmilDiscParams* p, int32_t rows, int32_t bags, int32_t backward) {
-  const size_t d = p->d, dh = p->d / 2, C = p->C, R = rows / 16;
+  const size_t d = p->d, dh = p->d / 2, R = rows / 16;
+  const size_t Kc = (size_t)p->C * disc_ksize(p) * disc_ksize(p);     // columns of the embedding's weight operand
   const size_t abw = gate_width(p->d);
   size_t f = 0;
   // head forward
   f += abw * d + abw + 512 + (abw / 128) * R + 256 + seg_pool_ws_floats((int)R, bags, (int)d) + 256 + (bags + 1) + 64;
   if (backward) {
     // embed backward
-    size_t e = (size_t)rows * d + (size_t)row_chunks(rows) * 3 * d + bwd_weight_ws_floats(rows, (int)d, (int)C) + 1024;
+    size_t e = (size_t)rows * d + (size_t)row_chunks(rows) * 3 * d + bwd_weight_ws_floats(rows, (int)d, (int)Kc) + 1024;
     // head backward
     size_t hb = (size_t)bags * (3 * d + dh + p->t2 + p->t1 + 2) + 2048;
     hb += R * abw + R * d + R * dh + abw * d + abw + 1024;
@@ -271,9 +279,10 @@ extern "C" size_t advmil_disc_workspace_bytes(const AdvmilDiscParams* p, int32_t
 extern "C" int advmil_disc_embed_fwd(const AdvmilDiscParams* p, const AdvmilBags* bags, AdvmilEmbedActs* a, void* stream) {
   ADVMIL_REQUIRE(p && a && a->emb, "disc_embed_fwd: null argument");
   ADVMIL_TRY(check_bags(bags, p->C, true, a->precision));
+  ADVMIL_TRY(check_ksize(p));
   ProfScope ps(PROF_EMBED, (cudaStream_t)stream);
   return region_embed_fwd(bags->x, p->Wc, p->bc, p->ln_g, p->ln_b, bags->rows, p->C, p->d, p->ln_eps, a->y_pre, a->emb,
-                          a->precision, (cudaStream_t)stream);
+                          a->precision, (cudaStream_t)stream, disc_ksize(p));
 }
 
 namespace advmil {
@@ -282,15 +291,18 @@ int disc_embed_bwd_impl(const AdvmilDiscParams* p, const AdvmilBags* bags, const
   ADVMIL_REQUIRE(p && a && d_emb && g, "disc_embed_bwd: null argument");
   ADVMIL_REQUIRE(a->y_pre, "disc_embed_bwd: forward was run without saving y_pre");
   ADVMIL_TRY(check_bags(bags, p->C, true, a->precision));
-  const int rows = bags->rows, d = p->d, C = p->C;
+  ADVMIL_TRY(check_ksize(p));
+  const int rows = bags->rows, d = p->d, C = p->C, ks = disc_ksize(p);
   Workspace ws(a->workspace, a->workspace_bytes);
   WS_TAKE(d_y, float, (size_t)rows * d);
   WS_TAKE(lnws, float, (size_t)row_chunks(rows) * 3 * d);
-  WS_TAKE(bwws, float, bwd_weight_ws_floats(rows, d, C));
+  WS_TAKE(bwws, float, bwd_weight_ws_floats(rows, d, ks * ks * C));
   { ProfScope ps(PROF_LN_BWD, st);
     ADVMIL_TRY(ln_pool_bwd(a->y_pre, d_emb, d_emb2, p->ln_g, p->ln_b, rows, d, p->ln_eps, d_y, g->ln_g, g->ln_b, g->bc, accumulate, lnws,
                            elem_of_precision(a->precision), st)); }
-  { ProfScope ps(PROF_BWD_W_EMBED, st); ADVMIL_TRY(bwd_weight(d_y, bags->x, rows, d, C, g->Wc, accumulate, bwws, a->precision, st)); }
+  { ProfScope ps(PROF_BWD_W_EMBED, st);
+    if (ks == 3) ADVMIL_TRY(bwd_weight_conv3(d_y, bags->x, rows, d, C, g->Wc, accumulate, bwws, a->precision, st));
+    else ADVMIL_TRY(bwd_weight(d_y, bags->x, rows, d, C, g->Wc, accumulate, bwws, a->precision, st)); }
   return ADVMIL_OK;
 }
 }  // namespace advmil

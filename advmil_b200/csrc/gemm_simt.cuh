@@ -71,7 +71,40 @@ struct TileLoader {
   }
 };
 
-template <bool A_KC, bool B_KC, class Epi>
+// Implicit-GEMM loaders of the 3x3 convolution inside every 4x4 region of 16 rows (row 16r + 4i + j = grid cell (i, j) of
+// region r), for x [rows, C] with ld == C and a tap-major K or N index tap * C + c (tap = 3 kh + kw).  The row read for
+// row m and tap is m's neighbour at (i + kh - 1, j + kw - 1), or zero outside the grid: no im2col copy of x.  C % 16 == 0,
+// so a BK = 16 block or a float4 never spans two taps.
+__device__ __forceinline__ int conv3_src_row(int m, int tap) {
+  const int di = tap / 3 - 1, dj = tap % 3 - 1, i = ((m >> 2) & 3) + di, j = (m & 3) + dj;
+  return ((unsigned)i < 4u && (unsigned)j < 4u) ? m + 4 * di + dj : -1;
+}
+// A(m, k) = x[nbr(m, tap)][c], k = tap * C + c   (the forward's activation operand, K-contiguous like TileLoader<true>)
+struct Conv3LoaderA : TileLoader<true> {
+  __device__ __forceinline__ static void load(const float* __restrict__ P, int ld, int mn0, int MN, int k0, int kend,
+                                              int t, float4 (&v)[2]) {
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      const int mn = mn0 + (t >> 2) + 64 * i, k = k0 + (t & 3) * 4;
+      const int tap = k / ld, src = (mn < MN && k < kend) ? conv3_src_row(mn, tap) : -1;
+      v[i] = src >= 0 ? *reinterpret_cast<const float4*>(P + (size_t)src * ld + (k - tap * ld)) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+  }
+};
+// B(k, n) = x[nbr(k, tap)][c], n = tap * C + c   (the weight gradient's X operand, N-contiguous like TileLoader<false>)
+struct Conv3LoaderB : TileLoader<false> {
+  __device__ __forceinline__ static void load(const float* __restrict__ P, int ld, int mn0, int MN, int k0, int kend,
+                                              int t, float4 (&v)[2]) {
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      const int k = k0 + (t >> 5) + 8 * i, mn = mn0 + (t & 31) * 4;
+      const int tap = mn / ld, src = (k < kend && mn < MN) ? conv3_src_row(k, tap) : -1;
+      v[i] = src >= 0 ? *reinterpret_cast<const float4*>(P + (size_t)src * ld + (mn - tap * ld)) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+  }
+};
+
+template <bool A_KC, bool B_KC, class Epi, class LA = TileLoader<A_KC>, class LB = TileLoader<B_KC>>
 __global__ void __launch_bounds__(GEMM_THREADS) gemm_simt_kernel(GemmArgs g, Epi epi) {
   pdl_prologue();
   __shared__ __align__(16) float As[2][BK][BM + 4];
@@ -89,18 +122,18 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_simt_kernel(GemmArgs g, Epi
     for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
 
   float4 ra[2], rb[2];
-  TileLoader<A_KC>::load(g.A, g.lda, m0, g.M, kbeg, kend, t, ra);
-  TileLoader<B_KC>::load(g.B, g.ldb, n0, g.N, kbeg, kend, t, rb);
-  TileLoader<A_KC>::store(As[0], t, ra);
-  TileLoader<B_KC>::store(Bs[0], t, rb);
+  LA::load(g.A, g.lda, m0, g.M, kbeg, kend, t, ra);
+  LB::load(g.B, g.ldb, n0, g.N, kbeg, kend, t, rb);
+  LA::store(As[0], t, ra);
+  LB::store(Bs[0], t, rb);
   __syncthreads();
 
   int buf = 0;
   for (int k0 = kbeg; k0 < kend; k0 += BK) {
     const bool more = (k0 + BK) < kend;
     if (more) {
-      TileLoader<A_KC>::load(g.A, g.lda, m0, g.M, k0 + BK, kend, t, ra);
-      TileLoader<B_KC>::load(g.B, g.ldb, n0, g.N, k0 + BK, kend, t, rb);
+      LA::load(g.A, g.lda, m0, g.M, k0 + BK, kend, t, ra);
+      LB::load(g.B, g.ldb, n0, g.N, k0 + BK, kend, t, rb);
     }
 #pragma unroll
     for (int kk = 0; kk < BK; ++kk) {
@@ -116,8 +149,8 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_simt_kernel(GemmArgs g, Epi
         for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
     }
     if (more) {
-      TileLoader<A_KC>::store(As[buf ^ 1], t, ra);
-      TileLoader<B_KC>::store(Bs[buf ^ 1], t, rb);
+      LA::store(As[buf ^ 1], t, ra);
+      LB::store(Bs[buf ^ 1], t, rb);
     }
     __syncthreads();
     buf ^= 1;
@@ -328,10 +361,10 @@ struct EpiPartial {
   }
 };
 
-template <bool A_KC, bool B_KC, class Epi>
+template <bool A_KC, bool B_KC, class Epi, class LA = TileLoader<A_KC>, class LB = TileLoader<B_KC>>
 inline int launch_gemm(const GemmArgs& g, const Epi& epi, int splits, cudaStream_t st) {
   dim3 grid(cdiv(g.M, BM), cdiv(g.N, BN), splits);
-  launch_k(gemm_simt_kernel<A_KC, B_KC, Epi>, dim3(grid), dim3(GEMM_THREADS), 0, st, g, epi);
+  launch_k(gemm_simt_kernel<A_KC, B_KC, Epi, LA, LB>, dim3(grid), dim3(GEMM_THREADS), 0, st, g, epi);
   ADVMIL_CHECK_LAUNCH();
   return ADVMIL_OK;
 }

@@ -54,15 +54,27 @@ int gated_score_fwd(const void* v, const float* Wp, const float* bp, const float
 }
 
 int region_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta, int rows,
-                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st) {
+                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st, int ksize) {
   ADVMIL_REQUIRE(rows % 16 == 0, "region_embed: rows %d not a multiple of 16 (backbone_utils.py:65)", rows);
   ADVMIL_REQUIRE(d <= 128 && d % 4 == 0 && C % 4 == 0, "region_embed: d=%d (<=128, %%4) C=%d (%%4) unsupported", d, C);
+  ADVMIL_REQUIRE(ksize == 1 || C % 16 == 0, "region_embed: the 3x3 embedding needs C %% 16 == 0 (C=%d)", C);
+  // rejected here rather than in the backward: bf16 runs only on tcgen05, and the 3x3 weight gradient tiles its 9 C columns
+  // by 128 or 256 without straddling a tap
+  ADVMIL_REQUIRE(ksize == 1 || precision != ADVMIL_BF16 || C % 128 == 0,
+                 "region_embed: the bf16 3x3 embedding needs C %% 128 == 0 (C=%d)", C);
   if (rows == 0) return ADVMIL_OK;
   if (precision != ADVMIL_FP32 && tc_embed_supported(rows, C, d, elem_of_precision(precision)))
-    return tc_region_embed_fwd(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, precision, st);
+    return ksize == 3 ? tc_conv3_embed_fwd(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, precision, st)
+                      : tc_region_embed_fwd(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, precision, st);
   ADVMIL_REQUIRE(precision != ADVMIL_BF16, kBf16Shape, "region_embed_fwd", rows, C, d);
-  GemmArgs g{(const float*)x, Wc, rows, d, C, C, C, C};
   EpiLNPool epi{(float*)y_pre, emb, bc, gamma, beta, d, eps};
+  if (ksize == 3) {
+    const float* Wk;
+    ADVMIL_TRY(conv3_weight_f32(Wc, d, C, st, &Wk));
+    GemmArgs g{(const float*)x, Wk, rows, d, 9 * C, C, 9 * C, 9 * C};
+    return launch_gemm<true, true, EpiLNPool, Conv3LoaderA>(g, epi, 1, st);
+  }
+  GemmArgs g{(const float*)x, Wc, rows, d, C, C, C, C};
   return launch_gemm<true, true>(g, epi, 1, st);
 }
 
@@ -108,6 +120,24 @@ int bwd_weight(const void* dY, const void* X, int rows, int N1, int N2, float* d
   EpiPartial epi{ws};
   ADVMIL_TRY((launch_gemm<false, false>(g, epi, splits, st)));
   return splitk_reduce(ws, splits, (size_t)N1 * N2, dW, accumulate, st);
+}
+
+int bwd_weight_conv3(const void* dY, const void* X, int rows, int N1, int C, float* dW, int accumulate, float* ws,
+                     int precision, cudaStream_t st) {
+  ADVMIL_REQUIRE(N1 % 4 == 0 && C % 16 == 0 && rows % 16 == 0 && (((uintptr_t)dY | (uintptr_t)X) % 16 == 0),
+                 "bwd_weight_conv3: N1=%d (%%4) C=%d (%%16) rows=%d (%%16) unsupported", N1, C, rows);
+  if (rows == 0) { if (!accumulate) return fill_zero(dW, (size_t)N1 * C * 9, st); return ADVMIL_OK; }
+  if (precision != ADVMIL_FP32 && tc_conv3_bwd_weight_supported(rows, N1, C, elem_of_precision(precision)))
+    return tc_conv3_bwd_weight(dY, X, rows, N1, C, dW, accumulate, ws, precision, st);
+  ADVMIL_REQUIRE(precision != ADVMIL_BF16, kBf16Shape, "bwd_weight_conv3", rows, N1, 9 * C);
+  const int N2 = 9 * C;
+  int splits = pick_splits(rows, N1, N2);
+  int kchunk = cdiv(cdiv(rows, splits), BK) * BK;
+  splits = cdiv(rows, kchunk);
+  GemmArgs g{(const float*)dY, (const float*)X, N1, N2, rows, N1, C, kchunk};
+  EpiPartial epi{ws};
+  ADVMIL_TRY((launch_gemm<false, false, EpiPartial, TileLoader<false>, Conv3LoaderB>(g, epi, splits, st)));
+  return splitk_reduce_conv3(ws, splits, N1, C, dW, accumulate, st);
 }
 
 }  // namespace advmil

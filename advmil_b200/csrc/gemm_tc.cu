@@ -73,6 +73,25 @@ static int make_tmap(CUtensorMap* m, const T* base, long long rows, long long co
   if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed (%d) rows=%lld cols=%lld", (int)r, rows, cols); return ADVMIL_ERR_CUDA; }
   return ADVMIL_OK;
 }
+// x [16 R, C] viewed as R regions of 4 x 4 patches (row 16r + 4i + j = region r, grid row i, grid column j), innermost first:
+// {C, j, i, r}.  A box {KBLK, 4, 4, box_regions} is box_regions * 16 rows x 128 B: in shared memory the same image as a
+// 2-D box of that many rows.  A box shifted by (di, dj) in the grid lands partly outside it and TMA fills those elements
+// with zeros: that is the 3x3 convolution's zero padding at every region border (and the tail past the last region).
+template <typename T>
+static int make_tmap_regions(CUtensorMap* m, const T* base, long long regions, long long C, int box_regions,
+                             CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B) {
+  EncodeTiledFn enc = get_encode();
+  if (!enc) { set_error("cuTensorMapEncodeTiled unavailable"); return ADVMIL_ERR_CUDA; }
+  const cuuint64_t rb = (cuuint64_t)C * sizeof(T);
+  cuuint64_t gdim[4] = {(cuuint64_t)C, 4, 4, (cuuint64_t)regions};
+  cuuint64_t gstr[3] = {rb, 4 * rb, 16 * rb};
+  cuuint32_t box[4] = {(cuuint32_t)TcElem<T>::KBLK, 4, 4, (cuuint32_t)box_regions};
+  cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
+  CUresult r = enc(m, TcElem<T>::DT, 4, (void*)base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed (%d) regions=%lld C=%lld", (int)r, regions, C); return ADVMIL_ERR_CUDA; }
+  return ADVMIL_OK;
+}
 
 static int sm_count() {
   static int n = 0;
@@ -271,7 +290,10 @@ __device__ __forceinline__ void split_tf32(const uint4& v, uint4& hi, uint4& lo)
 // One CTA per SM, persistent over its 128 x BLOCK_N tiles.  Barriers: full (the stage's TMA bytes landed), empty (the
 // MMAs that read the stage retired), conv (X3: the converter warps split the stage's A tile), tfull (an accumulator
 // buffer is complete), tempty (every epilogue thread drained it).
-template <typename T, int BLOCK_N, int EPI, bool FAST, bool X3 = false>
+// CONV: implicit-GEMM 3x3 convolution inside each 4x4 region, K = 9 C.  tmA is the region view of x (make_tmap_regions),
+// W the tap-major repacked weight [N, 9 C]; k block kb = 9 kc + tap reads channel block kc of x shifted by the tap, so
+// the nine boxes of one channel block cover the same 128 rows back to back and x is read from HBM about once.
+template <typename T, int BLOCK_N, int EPI, bool FAST, bool X3 = false, bool CONV = false>
 __global__ void __launch_bounds__(RowCfg<(int)sizeof(T), BLOCK_N, EPI, X3>::THREADS, 1)
 tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmBlo, int M, int N, int K, RowEpi ea) {
@@ -329,9 +351,16 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         for (int kb = 0; kb < kblocks; ++kb) {
           mbar_wait(&empty[stage], phase ^ 1);          // the MMAs that read this slot retired
           mbar_arrive_expect_tx(&full[stage], Cfg::TMA_BYTES);
-          tma_load_2d(A_s + stage * A_STAGE_BYTES, &tmA, &full[stage], kb * KBLK, m0);
-          tma_load_2d(B_s + stage * Cfg::B_STAGE_BYTES, &tmB, &full[stage], kb * KBLK, n0);
-          if (X3) tma_load_2d(BL_s + stage * Cfg::B_STAGE_BYTES, &tmBlo, &full[stage], kb * KBLK, n0);
+          int kw = kb * KBLK;                             // k coordinate of the weight tile
+          if constexpr (CONV) {
+            const int kc = kb / 9, tap = kb - 9 * kc;
+            tma_load_4d(A_s + stage * A_STAGE_BYTES, &tmA, &full[stage], kc * KBLK, tap % 3 - 1, tap / 3 - 1, m0 >> 4);
+            kw = tap * (K / 9) + kc * KBLK;
+          } else {
+            tma_load_2d(A_s + stage * A_STAGE_BYTES, &tmA, &full[stage], kb * KBLK, m0);
+          }
+          tma_load_2d(B_s + stage * Cfg::B_STAGE_BYTES, &tmB, &full[stage], kw, n0);
+          if (X3) tma_load_2d(BL_s + stage * Cfg::B_STAGE_BYTES, &tmBlo, &full[stage], kw, n0);
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -999,21 +1028,24 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 
 // CTA pairs (tcgen05.mma.cta_group::2, M = 256, each CTA loading half of the weight tile) were measured, no gain: within
 // 3 % of this kernel and mostly slower on B200 (the epilogue's HBM writes and latency bound it, not operand ingress).
-template <typename T, int BLOCK_N, int EPI, bool FAST, bool X3 = false>
+// CONV: A is x [rows, K / 9] (rows % 16 == 0), read through its region view
+template <typename T, int BLOCK_N, int EPI, bool FAST, bool X3 = false, bool CONV = false>
 static int launch_rows(const T* A, const T* W, int rows, int K, int N, const RowEpi& ea, cudaStream_t st, const T* Wlo = nullptr) {
   using Cfg = RowCfg<(int)sizeof(T), BLOCK_N, EPI, X3>;
   const int num_m = cdiv(rows, TILE_M), num_n = N / BLOCK_N;
   CUtensorMap tmA, tmB, tmBlo;
-  ADVMIL_TRY(make_tmap<T>(&tmA, A, rows, K, TILE_M));
+  if constexpr (CONV) ADVMIL_TRY(make_tmap_regions<T>(&tmA, A, rows / 16, K / 9, TILE_M / 16));
+  else ADVMIL_TRY(make_tmap<T>(&tmA, A, rows, K, TILE_M));
   ADVMIL_TRY(make_tmap<T>(&tmB, W, N, K, BLOCK_N));
   ADVMIL_TRY(make_tmap<T>(&tmBlo, X3 ? Wlo : W, N, K, BLOCK_N));
+  auto kern = tc_rows_kernel<T, BLOCK_N, EPI, FAST, X3, CONV>;
   static bool attr_set = false;
   if (!attr_set) {
-    ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(tc_rows_kernel<T, BLOCK_N, EPI, FAST, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
+    ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
     attr_set = true;
   }
   const int grid = min(num_m * num_n, sm_count());
-  launch_k(tc_rows_kernel<T, BLOCK_N, EPI, FAST, X3>, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM, st, tmA, tmB, tmBlo, rows, N, K, ea);
+  launch_k(kern, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM, st, tmA, tmB, tmBlo, rows, N, K, ea);
   ADVMIL_CHECK_LAUNCH();
   return ADVMIL_OK;
 }
@@ -1040,7 +1072,9 @@ template <typename T, int BLOCK_N, bool X3 = false> struct WgCfg {
   static constexpr size_t SMEM = 1024 + (size_t)STAGES * STAGE_BYTES * (X3 ? 2 : 1) + 4 * 32 * STG_LD * 4 + 256;
 };
 
-template <typename T, int BLOCK_N, bool X3 = false>
+// CONV: dWc of the 3x3 region convolution, N2 = 9 C tap-major (column tap * C + c); tmB is the region view of x with
+// KR / 16 regions per box, and a BLOCK_N-column tile (C % BLOCK_N == 0) reads x shifted by its tap
+template <typename T, int BLOCK_N, bool X3 = false, bool CONV = false>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA /*dY*/, const __grid_constant__ CUtensorMap tmB /*X*/,
                 int rows, int N1, int N2, int rows_per_split, float* __restrict__ ws) {
@@ -1092,9 +1126,17 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmA /*dY*/, const __grid_con
 #pragma unroll
         for (int g = 0; g < Cfg::A_GROUPS; ++g)
           tma_load_2d(S_s + stage * SB + g * Cfg::GROUP_BYTES, &tmA, &full[stage], m0 + g * MNG, r0);
+        if constexpr (CONV) {
+          const int C = N2 / 9, tap = n0 / C, c0 = n0 - tap * C;
 #pragma unroll
-        for (int g = 0; g < Cfg::B_GROUPS; ++g)
-          tma_load_2d(S_s + stage * SB + Cfg::A_BYTES + g * Cfg::GROUP_BYTES, &tmB, &full[stage], n0 + g * MNG, r0);
+          for (int g = 0; g < Cfg::B_GROUPS; ++g)
+            tma_load_4d(S_s + stage * SB + Cfg::A_BYTES + g * Cfg::GROUP_BYTES, &tmB, &full[stage], c0 + g * MNG, tap % 3 - 1,
+                        tap / 3 - 1, r0 >> 4);
+        } else {
+#pragma unroll
+          for (int g = 0; g < Cfg::B_GROUPS; ++g)
+            tma_load_2d(S_s + stage * SB + Cfg::A_BYTES + g * Cfg::GROUP_BYTES, &tmB, &full[stage], n0 + g * MNG, r0);
+        }
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       }
     }
@@ -1384,6 +1426,58 @@ int tc_region_embed_fwd(const void* x, const float* Wc, const float* bc, const f
   return tc_embed_t<float>(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, st);
 }
 
+// tap-major K-major operand of a 3x3 weight W [N, C, 3, 3]: out[o, tap * C + c] = W[o, c, kh, kw], tap = 3 kh + kw;
+// out_lo != nullptr (fp32 only): split-tf32 parts, hi to `out`, lo to `out_lo`
+template <typename T>
+__global__ void conv3_pack_kernel(const float* __restrict__ W, int N, int C, T* __restrict__ out, T* __restrict__ out_lo) {
+  pdl_prologue();
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (size_t)N * 9 * C) return;
+  const int o = (int)(i / (9 * (size_t)C)), r = (int)(i - (size_t)o * 9 * C), tap = r / C, c = r - tap * C;
+  const float v = W[((size_t)o * C + c) * 9 + tap];
+  if constexpr (sizeof(T) == 4) {
+    if (out_lo) {
+      uint32_t h, l;
+      split_tf32(__float_as_uint(v), h, l);
+      out[i] = __uint_as_float(h); out_lo[i] = __uint_as_float(l);
+      return;
+    }
+  }
+  st1(out + i, v);
+}
+template <typename T>
+static int conv3_operand(const float* W, int N, int C, bool split, cudaStream_t st, const T** hi, const T** lo) {
+  const size_t n = (size_t)N * 9 * C;
+  void* p = nullptr;
+  ADVMIL_TRY(weight_scratch(WS_EMBED, n * sizeof(T) * (split ? 2 : 1), st, &p));
+  T* h = (T*)p;
+  T* l = split ? h + n : nullptr;
+  launch_k(conv3_pack_kernel<T>, dim3(cdiv(n, 256)), dim3(256), 0, st, W, N, C, h, l);
+  ADVMIL_CHECK_LAUNCH();
+  *hi = h;
+  if (lo) *lo = l;
+  return ADVMIL_OK;
+}
+int conv3_weight_f32(const float* W, int N, int C, cudaStream_t st, const float** out) {
+  return conv3_operand<float>(W, N, C, false, st, out, nullptr);
+}
+
+template <typename T, bool X3 = false>
+static int tc_conv3_embed_t(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta, int rows,
+                            int C, int d, float eps, void* y_pre, float* emb, cudaStream_t st) {
+  const T *Wt, *Wl;
+  ADVMIL_TRY(conv3_operand<T>(Wc, d, C, X3, st, &Wt, &Wl));
+  RowEpi ea{};
+  ea.bias = bc; ea.y_pre = y_pre; ea.emb = emb; ea.gamma = gamma; ea.beta = beta; ea.eps = eps;
+  return launch_rows<T, 128, EPI_LN, true, X3, true>((const T*)x, Wt, rows, 9 * C, d, ea, st, Wl);
+}
+int tc_conv3_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta,
+                       int rows, int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st) {
+  if (precision == ADVMIL_BF16) return tc_conv3_embed_t<bf16>(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, st);
+  if (precision == ADVMIL_TF32X3) return tc_conv3_embed_t<float, true>(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, st);
+  return tc_conv3_embed_t<float>(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, st);
+}
+
 // dX = dY . W with W [Ny, Nx] row-major fp32: the engine needs W^T [Nx, Ny] K-major in the operand type; the transpose
 // of the (small) weight goes to library scratch
 // out_lo != nullptr (fp32 only): split-tf32 parts of the scaled transpose -- hi to `out`, lo to `out_lo`
@@ -1470,14 +1564,16 @@ size_t tc_bwd_weight_ws_floats(int rows, int N1, int N2) {
   return a > b ? a : b;
 }
 
-template <typename T, int BLOCK_N, bool X3 = false>
+// CONV: X is x [rows, N2 / 9], read through its region view
+template <typename T, int BLOCK_N, bool X3 = false, bool CONV = false>
 static int launch_wgrad(const T* dY, const T* X, int rows, int N1, int N2, int rows_per_split, int nsplit, float* ws,
                         cudaStream_t st) {
   using Cfg = WgCfg<T, BLOCK_N, X3>;
   CUtensorMap tmA, tmB;
   ADVMIL_TRY(make_tmap<T>(&tmA, dY, rows, N1, Cfg::KR, TcElem<T>::MN_SWZ));
-  ADVMIL_TRY(make_tmap<T>(&tmB, X, rows, N2, Cfg::KR, TcElem<T>::MN_SWZ));
-  auto kern = tc_wgrad_kernel<T, BLOCK_N, X3>;
+  if constexpr (CONV) ADVMIL_TRY(make_tmap_regions<T>(&tmB, X, rows / 16, N2 / 9, Cfg::KR / 16, TcElem<T>::MN_SWZ));
+  else ADVMIL_TRY(make_tmap<T>(&tmB, X, rows, N2, Cfg::KR, TcElem<T>::MN_SWZ));
+  auto kern = tc_wgrad_kernel<T, BLOCK_N, X3, CONV>;
   static bool attr_set = false;
   if (!attr_set) {
     ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
@@ -1513,6 +1609,30 @@ int tc_bwd_weight(const void* dY, const void* X, int rows, int N1, int N2, float
   if (precision == ADVMIL_BF16) return tc_bwd_weight_t<bf16>(dY, X, rows, N1, N2, dW, accumulate, ws, st);
   if (precision == ADVMIL_TF32X3) return tc_bwd_weight_t<float, true>(dY, X, rows, N1, N2, dW, accumulate, ws, st);
   return tc_bwd_weight_t<float>(dY, X, rows, N1, N2, dW, accumulate, ws, st);
+}
+
+// 9 C columns tap-major: a 256- or 128-column tile never straddles two taps because C is a multiple of the tile width
+bool tc_conv3_bwd_weight_supported(int rows, int N1, int C, int dt) {
+  const int bn = wgrad_block_n(9 * C);
+  return tc_bwd_weight_supported(rows, N1, 9 * C, dt) && bn != 0 && C % bn == 0;
+}
+template <typename T, bool X3 = false>
+static int tc_conv3_bwd_weight_t(const void* dY, const void* X, int rows, int N1, int C, float* dW, int accumulate, float* ws,
+                                 cudaStream_t st) {
+  constexpr int KR = TcElem<T>::KBLK;
+  const int N2 = 9 * C;
+  const int splits = wgrad_splits(rows, N1, N2, X3);
+  const int rows_per_split = cdiv(cdiv(rows, splits), KR) * KR;
+  const int nsplit = cdiv(rows, rows_per_split);
+  if (wgrad_block_n(N2) == 256) ADVMIL_TRY((launch_wgrad<T, 256, X3, true>((const T*)dY, (const T*)X, rows, N1, N2, rows_per_split, nsplit, ws, st)));
+  else ADVMIL_TRY((launch_wgrad<T, 128, X3, true>((const T*)dY, (const T*)X, rows, N1, N2, rows_per_split, nsplit, ws, st)));
+  return splitk_reduce_conv3(ws, nsplit, N1, C, dW, accumulate, st);
+}
+int tc_conv3_bwd_weight(const void* dY, const void* X, int rows, int N1, int C, float* dW, int accumulate, float* ws,
+                        int precision, cudaStream_t st) {
+  if (precision == ADVMIL_BF16) return tc_conv3_bwd_weight_t<bf16>(dY, X, rows, N1, C, dW, accumulate, ws, st);
+  if (precision == ADVMIL_TF32X3) return tc_conv3_bwd_weight_t<float, true>(dY, X, rows, N1, C, dW, accumulate, ws, st);
+  return tc_conv3_bwd_weight_t<float>(dY, X, rows, N1, C, dW, accumulate, ws, st);
 }
 
 }  // namespace advmil

@@ -19,6 +19,11 @@ int tc_gated_score_fwd(const void* v, const float* Wp, const float* bp, const fl
 bool tc_embed_supported(int rows, int C, int d, int dt);
 int tc_region_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta,
                         int rows, int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st);
+// 3x3 region convolution (Wc [d, C, 3, 3]; same support rule as tc_embed_supported, rows % 16 == 0)
+int tc_conv3_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta,
+                       int rows, int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st);
+// fp32 tap-major repack [N, 9 C] of a 3x3 weight in library scratch (the FFMA engine's operand)
+int conv3_weight_f32(const float* W, int N, int C, cudaStream_t st, const float** out);
 bool tc_bwd_data_supported(int rows, int Ny, int Nx, int dt);
 int tc_bwd_data(const void* dY, const float* W, int rows, int Ny, int Nx, void* dX, const BwdDataExtras& ex,
                 int precision, cudaStream_t st);
@@ -26,5 +31,8 @@ bool tc_bwd_weight_supported(int rows, int N1, int N2, int dt);
 size_t tc_bwd_weight_ws_floats(int rows, int N1, int N2);
 int tc_bwd_weight(const void* dY, const void* X, int rows, int N1, int N2, float* dW, int accumulate, float* ws,
                   int precision, cudaStream_t st);
+bool tc_conv3_bwd_weight_supported(int rows, int N1, int C, int dt);
+int tc_conv3_bwd_weight(const void* dY, const void* X, int rows, int N1, int C, float* dW, int accumulate, float* ws,
+                        int precision, cudaStream_t st);
 
 }  // namespace advmil

@@ -188,6 +188,31 @@ int splitk_reduce(const float* ws, int splits, size_t n, float* out, int accumul
   return ADVMIL_OK;
 }
 
+// out[o][c][tap] (+)= sum_z ws[z][o][tap * C + c]: the tap-major partials of a 3x3 weight gradient into the Conv2d layout
+// [N1, C, 3, 3].  One block per (o, 128 channels): coalesced reads per tap, a [128][9] shared tile, coalesced writes.
+__global__ void splitk_reduce_conv3_kernel(const float* __restrict__ ws, int splits, int N1, int C, float* __restrict__ out,
+                                           int accumulate) {
+  pdl_prologue();
+  __shared__ float t[128 * 9];
+  const int o = blockIdx.y, c0 = blockIdx.x * 128, c = c0 + threadIdx.x;
+  const size_t n = (size_t)N1 * 9 * C;
+  for (int tap = 0; tap < 9; ++tap) {
+    float acc = 0.f;
+    if (c < C)
+      for (int z = 0; z < splits; ++z) acc += ws[(size_t)z * n + ((size_t)o * 9 + tap) * C + c];
+    t[threadIdx.x * 9 + tap] = acc;
+  }
+  __syncthreads();
+  const int nc = min(128, C - c0);
+  float* dst = out + ((size_t)o * C + c0) * 9;
+  for (int j = threadIdx.x; j < nc * 9; j += 128) dst[j] = accumulate ? dst[j] + t[j] : t[j];
+}
+int splitk_reduce_conv3(const float* ws, int splits, int N1, int C, float* out, int accumulate, cudaStream_t st) {
+  launch_k(splitk_reduce_conv3_kernel, dim3(dim3(cdiv(C, 128), N1)), dim3(128), 0, st, ws, splits, N1, C, out, accumulate);
+  ADVMIL_CHECK_LAUNCH();
+  return ADVMIL_OK;
+}
+
 template <typename T>
 __global__ void apply_dropout_kernel(const T* __restrict__ src, size_t nvec, int vec_per_row, Drop drop, T* __restrict__ dst) {
   pdl_prologue();

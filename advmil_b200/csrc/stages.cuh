@@ -42,8 +42,10 @@ int proj_embed_fwd(const void* x, const float* W1, const float* b1, const float*
 int gated_score_fwd(const void* v, const float* Wp, const float* bp, const float* wc, const float* bc, int rows, int L,
                     int D, const Drop& da, const Drop& db, void* ab, float* s, float* part_ws, int precision,
                     cudaStream_t st);
+// ksize 1: y = x Wc^T + bc (Wc [d, C]); ksize 3: y = 3x3 convolution, zero padded, inside every 4x4 region of 16 rows
+// (Wc [d, C, 3, 3], the Conv2d layout)
 int region_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta, int rows,
-                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st);
+                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st, int ksize = 1);
 // dX[rows,Nx] = (dY[rows,Ny] . W[Ny,Nx] + pool terms) * relu'  (W row-major [Ny, Nx])
 struct BwdDataExtras {
   const float* w = nullptr; const float* dz = nullptr; const float* dmean = nullptr;
@@ -60,6 +62,10 @@ int bwd_data(const void* dY, const float* W, int rows, int Ny, int Nx, void* dX,
 size_t bwd_weight_ws_floats(int rows, int N1, int N2);
 int bwd_weight(const void* dY, const void* X, int rows, int N1, int N2, float* dW, int accumulate, float* ws,
                int precision, cudaStream_t st);
+// dW[N1, C, 3, 3] (+)= the weight gradient of the 3x3 region convolution of X[rows, C] (rows % 16 == 0) under dY[rows, N1]
+// (ws >= bwd_weight_ws_floats(rows, N1, 9 C) floats)
+int bwd_weight_conv3(const void* dY, const void* X, int rows, int N1, int C, float* dW, int accumulate, float* ws,
+                     int precision, cudaStream_t st);
 
 // ---- rlip_chain.cu ----------------------------------------------------------------------------
 // fc1 MLP + GAPool gate of the RLIP head over R regions in one FFMA kernel (d == 128): writes f1 [R, d/2], fi [R, d],
@@ -108,6 +114,8 @@ int reduce_rows(const float* part, int nparts, int width, float* out, int accumu
 int reduce_rows_strided(const float* part, int nparts, int stride, int ncols, float* out, int accumulate, cudaStream_t st);
 int splitk_reduce(const float* ws, int splits, size_t n, float* out, int accumulate, cudaStream_t st);
 int splitk_reduce_t(const float* ws, int splits, int R, int Cc, float* out, int accumulate, cudaStream_t st);
+// ws slices [N1][9 C] tap-major -> out [N1][C][3][3]
+int splitk_reduce_conv3(const float* ws, int splits, int N1, int C, float* out, int accumulate, cudaStream_t st);
 int apply_dropout(const void* src, int rows, int width, const Drop& drop, void* dst, int dt, cudaStream_t st);
 int fill_zero(float* p, size_t n, cudaStream_t st);
 int cast_f32_to_bf16(const float* in, size_t n, void* out, cudaStream_t st);

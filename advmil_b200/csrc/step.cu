@@ -184,7 +184,7 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   STEP_TAKE(y_pre, char, (size_t)rows * d * es);
   AdvmilEmbedActs ea{};
   ea.emb = emb2; ea.y_pre = y_pre; ea.precision = a->precision;
-  const bool fused = gp.C == dp.C && proj_embed_supported(rows, gp.C, gp.h, d, a->precision);
+  const bool fused = gp.C == dp.C && (dp.ksize == 0 || dp.ksize == 1) && proj_embed_supported(rows, gp.C, gp.h, d, a->precision);
   if (fused) {     // K1 and K5+K6 read the same x: one pass over stacked weights, then the generator forward skips K1
     for (int i = 0; i < nb; ++i)
       ADVMIL_REQUIRE((bags->offsets_host[i + 1] - bags->offsets_host[i]) % 16 == 0,

@@ -52,6 +52,14 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       "l"((uint64_t)m), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
+// 4-D tile load (c0 innermost); coordinates may be negative or run past the extent: those elements arrive as zeros
+__device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2, int c3) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(
+          smem_u32(smem_dst)),
+      "l"((uint64_t)m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+      : "memory");
+}
 
 // ---- tcgen05 --------------------------------------------------------------------------------------
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_result, uint32_t ncols) {  // one full warp, ncols pow2 >= 32

@@ -43,12 +43,13 @@ def gen_cfg_lists(cfg: ops.GenConfig):
 
 
 def _disc_cfg(icfg: Sequence[int], fcfg: Sequence[float]) -> ops.DiscConfig:
-    C, d, t1, t2, inner, prj = [int(v) for v in icfg]
-    return ops.DiscConfig(C=C, d=d, t1=t1, t2=t2, inner_instance=inner, prj_path=prj, p=float(fcfg[0]), ln_eps=float(fcfg[1]))
+    C, d, t1, t2, inner, prj, ksize = [int(v) for v in icfg]
+    return ops.DiscConfig(C=C, d=d, t1=t1, t2=t2, inner_instance=inner, prj_path=prj, p=float(fcfg[0]), ln_eps=float(fcfg[1]),
+                          ksize=ksize)
 
 
 def disc_cfg_lists(cfg: ops.DiscConfig):
-    return ([cfg.C, cfg.d, cfg.t1, cfg.t2, cfg.inner_instance, cfg.prj_path], [cfg.p, cfg.ln_eps])
+    return ([cfg.C, cfg.d, cfg.t1, cfg.t2, cfg.inner_instance, cfg.prj_path, cfg.ksize], [cfg.p, cfg.ln_eps])
 
 
 _MODE = None

@@ -123,7 +123,7 @@ class PrjDiscriminator(nn.Module):
         C, d, t1, t2 = self.dims
         return ops.DiscConfig(C=C, d=d, t1=t1, t2=t2, inner_instance=int(self.inner_product == "instance"),
                               prj_path={"x": 1, "y": 2}.get(self.prj_path, 0), p=self.net_pair_one.p,
-                              ln_eps=self.net_pair_one.embedding.norm.eps)
+                              ln_eps=self.net_pair_one.embedding.norm.eps, ksize=self.net_pair_one.embedding.conv.kernel_size[0])
 
     def disc_params(self):
         y = self.net_pair_two
@@ -181,7 +181,7 @@ class Discriminator(PrjDiscriminator):
     def config(self) -> ops.DiscConfig:
         C, d, t1, t2 = self.dims
         return ops.DiscConfig(C=C, d=d, t1=t1, t2=t2, inner_instance=0, prj_path=3, p=self.net_pair_one.p,
-                              ln_eps=self.net_pair_one.embedding.norm.eps)
+                              ln_eps=self.net_pair_one.embedding.norm.eps, ksize=self.net_pair_one.embedding.conv.kernel_size[0])
 
     def disc_params(self):
         y = self.net_pair_two

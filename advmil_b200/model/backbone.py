@@ -166,6 +166,9 @@ class DualTrans_HS(nn.Module):
             raise NotImplementedError("the fused ESAT path covers one Transformer encoder layer (model/backbone.py:33)")
         self.dims = (dim_in, dim_hid, dim_out)
         self.patch_embedding_layer = make_embedding_layer(emb_backbone, args_emb_backbone)
+        if self.patch_embedding_layer.conv.kernel_size != (1, 1):
+            # advmil_esat_fwd / _bwd take the patch embedding as a per-patch linear [d, C]; load_backbone fixes ksize 1 (:21)
+            raise NotImplementedError("the fused ESAT path covers the ksize-1 patch embedding only")
         self.dim_hid = dim_hid
         self.patch_encoder_layer = make_transformer_layer(tra_backbone, args_tra_backbone)
         self.pool = GAPool(dim_out, dim_out)

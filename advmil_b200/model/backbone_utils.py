@@ -56,16 +56,17 @@ def sequence2square_index(n_rows: int, s: int = 4) -> torch.Tensor:
 
 
 class AVGPoolPatchEmbedding(nn.Module):
-    """Patch embedding container (reference model/backbone_utils.py:129-168): conv (1x1 == per-patch linear), norm,
-    ReLU, 4x4 average pool.  Only the configuration the AdvMIL configs reach is supported by the fused kernel:
-    scale 4, ksize 1, stride 1 (config/cfg_nlst.yaml:41-42)."""
+    """Patch embedding container (reference model/backbone_utils.py:129-168): conv, norm, ReLU, 4x4 average pool.  The
+    fused kernels cover what the AdvMIL configs reach: scale 4, stride 1, no depth-wise conv, and ksize 1 (per-patch linear,
+    config/cfg_nlst.yaml:41-42) or 3 (3x3 convolution over each region's 4x4 grid of patches, zero padded at its border;
+    the reference class's default, disc_netx_ksize: 3)."""
 
     def __init__(self, in_dim, out_dim, scale: int = 4, dw_conv=False, ksize=3, stride=1):
         super().__init__()
         assert scale == 4, "It only supports for scale = 4"
         assert ksize == 1 or ksize == 3, "It only supports for ksize = 1 or 3"
-        if ksize != 1 or stride != 1 or dw_conv:
-            raise NotImplementedError("advmil_b200 fuses the ksize=1/stride=1 (FC) patch embedding only")
+        if stride != 1 or dw_conv:
+            raise NotImplementedError("advmil_b200 fuses the stride-1, non-depth-wise patch embedding only")
         self.scale, self.stride = scale, stride
         self.conv = nn.Conv2d(in_dim, out_dim, ksize, stride, padding=(ksize - 1) // 2)
         self.pool = nn.AdaptiveAvgPool2d(1)
@@ -77,7 +78,7 @@ class AVGPoolPatchEmbedding(nn.Module):
         from .. import ops, get_precision
         bags = ops.PackedBags.from_single(x)
         cfg = ops.DiscConfig(C=self.conv.in_channels, d=self.conv.out_channels, t1=1, t2=self.conv.out_channels,
-                             ln_eps=self.norm.eps)
+                             ln_eps=self.norm.eps, ksize=self.conv.kernel_size[0])
         params = [self.conv.weight, self.conv.bias, self.norm.weight, self.norm.bias] + [None] * 20
         acts = ops.disc_embed_forward(cfg, params, bags, ops.PRECISIONS[get_precision()], save=False)
         return acts["emb"].unsqueeze(0)

@@ -453,13 +453,14 @@ class DiscConfig:
     prj_path: int = 1
     p: float = 0.25
     ln_eps: float = 1e-5
+    ksize: int = 1          # patch-embedding conv kernel: 1 (per-patch linear) or 3 (3x3 inside each 4x4 region)
 
     def c(self, params) -> DiscParams:
         s = DiscParams()
         for name, t in zip(DISC_TENSORS, params):
             setattr(s, name, _ptr(t))
         s.C, s.d, s.t1, s.t2 = self.C, self.d, self.t1, self.t2
-        s.inner_instance, s.prj_path, s.p, s.ln_eps = self.inner_instance, self.prj_path, self.p, self.ln_eps
+        s.inner_instance, s.prj_path, s.p, s.ln_eps, s.ksize = self.inner_instance, self.prj_path, self.p, self.ln_eps, self.ksize
         return s
 
 

@@ -115,7 +115,7 @@ typedef struct AdvmilGenActs {
 /* ---- discriminator: RLIP (model/GANSurv.py:71-105, model/model_utils.py:157-210,
  *      model/backbone_utils.py:31-77,129-168) ----------------------------------------------- */
 typedef struct AdvmilDiscParams {
-  const float *Wc, *bc;        /* net_pair_one.embedding.conv [d,C(,1,1)],[d] */
+  const float *Wc, *bc;        /* net_pair_one.embedding.conv [d,C(,1,1)] (ksize 0 / 1) or [d,C,3,3] (ksize 3),[d] */
   const float *ln_g, *ln_b;    /* net_pair_one.embedding.norm [d],[d] */
   const float *F1a_w, *F1a_b;  /* net_pair_one.fc1.0 [d/2,d] */
   const float *F1b_w, *F1b_b;  /* net_pair_one.fc1.3 [d,d/2] */
@@ -133,6 +133,10 @@ typedef struct AdvmilDiscParams {
                                   out = fc(cat[hx, ht]) with no inner product (inner_instance ignored) */
   float p;                     /* disc_netx_dropout */
   float ln_eps;
+  int32_t ksize;               /* disc_netx_ksize: kernel size of the patch-embedding conv.  0 or 1 = per-patch linear;
+                                  3 = 3x3 convolution (stride 1, padding 1) over each region's 4x4 grid of patches, zero
+                                  padded at the region border (needs C % 16 == 0, and C % 128 == 0 in ADVMIL_BF16);
+                                  anything else = ADVMIL_ERR_INVALID */
 } AdvmilDiscParams;
 
 typedef struct AdvmilDiscGrads {
@@ -209,7 +213,8 @@ ADVMIL_API int advmil_generator_sample(const AdvmilGenParams* p, const float* H,
                             int32_t bags, int32_t samples, float* out, void* stream);
 
 /* ---- discriminator ------------------------------------------------------------------------ */
-/* K5+K6 (AVGPoolPatchEmbedding.forward, model/backbone_utils.py:158-168): emb[r] = mean_{k<16} relu(LN(x[16r+k]Wc^T+bc)).
+/* K5+K6 (AVGPoolPatchEmbedding.forward, model/backbone_utils.py:158-168): emb[r] = mean_{k<16} relu(LN(x[16r+k]Wc^T+bc)),
+ * or with ksize 3 the same over y = conv3x3(region r's 4x4 grid of rows) + bc.
  * Every bag length must be a multiple of 16 (backbone_utils.py:65) else ADVMIL_ERR_INVALID. */
 ADVMIL_API size_t advmil_disc_workspace_bytes(const AdvmilDiscParams* p, int32_t rows, int32_t bags, int32_t backward);
 ADVMIL_API int advmil_disc_embed_fwd(const AdvmilDiscParams* p, const AdvmilBags* bags, AdvmilEmbedActs* acts, void* stream);
