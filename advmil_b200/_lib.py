@@ -120,8 +120,13 @@ class EsatStepArgs(C.Structure):
                 ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
 
 
+class ClusterStepArgs(C.Structure):
+    _fields_ = [("base", StepArgs), ("Wphi", c_fp), ("bphi", c_fp), ("dWphi", c_fp), ("dbphi", c_fp), ("cid", c_ip),
+                ("num_clusters", C.c_int32)]
+
+
 ABI_STRUCTS = [Bags, GenParams, GenGrads, GenActs, DiscParams, DiscGrads, EmbedActs, HeadActs, StepArgs, EsatParams, EsatGrads,
-               EsatActs, EsatStepArgs]
+               EsatActs, EsatStepArgs, ClusterStepArgs]
 
 # every symbol include/advmil_b200.h declares: name -> (restype, argtypes)
 _i32, _i64, _f, _vp, _sz, _u64 = C.c_int32, C.c_int64, C.c_float, C.c_void_p, C.c_size_t, C.c_uint64
@@ -173,6 +178,13 @@ SYMBOLS = {
     "advmil_adv_step_esat_workspace_bytes": (_sz, [_P(EsatParams), _P(GenParams), _P(DiscParams), _i32, _i32, _i32]),
     "advmil_adv_step_esat_disc": (C.c_int, [_P(EsatStepArgs), _vp]),
     "advmil_adv_step_esat_gen": (C.c_int, [_P(EsatStepArgs), _vp]),
+    "advmil_adv_step_cluster_workspace_bytes": (_sz, [_P(GenParams), _P(DiscParams), _i32, _i32, _i32, _i32]),
+    "advmil_adv_step_cluster_disc": (C.c_int, [_P(ClusterStepArgs), _vp]),
+    "advmil_adv_step_cluster_gen": (C.c_int, [_P(ClusterStepArgs), _vp]),
+    "advmil_cluster_pool_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
+    "advmil_cluster_pool_fwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _P(C.c_int32), _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp,
+                                          _vp, _sz, _vp]),
+    "advmil_cluster_pool_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "advmil_mha_fwd": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _f, _u64, _i32, _vp, _vp, _i32, _vp, _vp, _vp]),
     "advmil_mha_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _f, _u64, _i32, _vp, _vp, _i32, _vp, _vp, _vp]),
     "advmil_bf16p12_decode": (C.c_int, [_vp, _vp, C.c_char_p, _vp, _vp, _i64, _i32, _vp, _vp]),
@@ -185,7 +197,7 @@ SYMBOLS = {
 
 PROF_TAGS = ["proj_fwd", "gate_fwd", "pool_fwd", "embed_fwd", "pool_gate_bwd", "bwd_data", "bwd_w_gate", "bwd_w_proj",
              "ln_bwd", "bwd_w_embed", "colsum", "dropout", "head_fwd", "head_bwd", "gen_tail", "loss_opt", "proj_embed_fwd",
-             "attn_fwd", "attn_bwd"]
+             "attn_fwd", "attn_bwd", "proj_segmean_fwd"]
 
 _lib = None
 

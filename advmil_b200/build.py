@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "csrc", "_obj")
 LIB = os.path.join(HERE, "libadvmil_b200.so")
-SOURCES = ["api.cu", "gemm_stages.cu", "gemm_tc.cu", "seg_kernels.cu", "tail_kernels.cu", "step.cu", "esat_kernels.cu", "esat.cu", "codec.cu", "rlip_chain.cu", "esat_attn_tc.cu", "esat_attn_bwd_tc.cu"]
+SOURCES = ["api.cu", "gemm_stages.cu", "gemm_tc.cu", "seg_kernels.cu", "tail_kernels.cu", "step.cu", "esat_kernels.cu", "esat.cu", "codec.cu", "rlip_chain.cu", "esat_attn_tc.cu", "esat_attn_bwd_tc.cu", "cluster_pool.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math=false",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-Xcompiler", "-O2"]

@@ -87,6 +87,7 @@ extern "C" size_t advmil_abi_sizeof(int which) {
     case 10: return sizeof(AdvmilEsatGrads);
     case 11: return sizeof(AdvmilEsatActs);
     case 12: return sizeof(AdvmilEsatStepArgs);
+    case 13: return sizeof(AdvmilClusterStepArgs);
     default: return 0;
   }
 }

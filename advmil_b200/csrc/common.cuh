@@ -99,7 +99,8 @@ enum ProfTag : int {
   PROF_PROJ_EMBED = 16, // K1 + K5/K6 fused over stacked weights (bf16 fused step)
   PROF_ATTN_FWD = 17,   // ESAT self-attention forward
   PROF_ATTN_BWD = 18,   // ESAT self-attention backward (dQ pass + dK/dV pass)
-  PROF_NTAGS = 19
+  PROF_PROJ_SEGMEAN = 19, // K9: DeepAttMISL projection + ReLU + per-(bag, cluster) mean in one pass (+ finalize)
+  PROF_NTAGS = 20
 };
 struct ProfScope {
   int tag; cudaStream_t st; void* rec;

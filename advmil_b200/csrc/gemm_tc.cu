@@ -102,7 +102,8 @@ static int sm_count() {
 // ------------------------------------------------------------------------------------------------
 // epilogue parameter block
 // ------------------------------------------------------------------------------------------------
-enum RowEpiKind : int { EPI_LINEAR = 0, EPI_GATE = 1, EPI_LN = 2, EPI_BWD = 3, EPI_PE = 4 /* K1 + K5/K6 on stacked weights */ };
+enum RowEpiKind : int { EPI_LINEAR = 0, EPI_GATE = 1, EPI_LN = 2, EPI_BWD = 3, EPI_PE = 4 /* K1 + K5/K6 on stacked weights */,
+                        EPI_POOL = 5 /* K9: relu(x W^T + b) -> per-(tile, bag, cluster) column sums */ };
 
 // out / ab / y_pre / relu_src are [rows, *] activation tensors of the kernel's element type T (fp32 or bf16)
 struct RowEpi {
@@ -116,6 +117,10 @@ struct RowEpi {
   const float* dmean; int accumulate;
   float* colpart;                                                                // EPI_BWD: [4 * num_m][N] column sums of dX per 32 rows
   const void* relu_src; int ld_src; float inv_keep;
+  // EPI_POOL reuses fields of the block above (its layout, and so every other instantiation, stays as it is):
+  //   out = optional ReLU keep bits uint32 [rows][N / 32] (bit i of word c = column 32 c + i), ldo = N / 32, bias,
+  //   part = column sums [(m-tile + bag) * D + cluster][N] (fp32), D = number of clusters, relu_src = cluster ids int32
+  //   [rows], offsets / bags = the packed bags (every bag length a multiple of 16)
 };
 
 constexpr int TILE_M = 128;
@@ -141,17 +146,17 @@ template <int ES, int BLOCK_N, int EPI, bool X3 = false> struct RowCfg {
   // idled behind it (ncu r02: dh 35 % tensor-active at 0.26 IPC per scheduler).  4 warps per quarter (3 at 192 columns, where
   // 6 chunks divide evenly) give the schedulers the warps to hide those latencies; registers: 65536 / 640 threads = 102.
   static constexpr bool WIDE_EPI = ES == 2 && (EPI == EPI_GATE || EPI == EPI_BWD || EPI == EPI_LINEAR);
-  static constexpr int NSUB = (EPI == EPI_LN || X3) ? 1 : (!WIDE_EPI ? 2 : (EPI != EPI_GATE && BLOCK_N == 192 ? 3 : (BLOCK_N >= 128 ? 4 : 2)));
+  static constexpr int NSUB = (EPI == EPI_LN || EPI == EPI_POOL || X3) ? 1 : (!WIDE_EPI ? 2 : (EPI != EPI_GATE && BLOCK_N == 192 ? 3 : (BLOCK_N >= 128 ? 4 : 2)));
   static constexpr int EPI_WARPS = 4 * NSUB;
   static constexpr int THREADS = 128 + 32 * EPI_WARPS;
   static constexpr int B_STAGE_BYTES = BLOCK_N * 128;
   static constexpr int STAGE_BYTES = (X3 ? 2 : 1) * (A_STAGE_BYTES + B_STAGE_BYTES);
   static constexpr int TMA_BYTES = A_STAGE_BYTES + (X3 ? 2 : 1) * B_STAGE_BYTES;     // what TMA delivers per stage
   // bf16 staging: 32 rows x 64 bytes, XOR-swizzled (2 KB per warp); fp32 staging: 32 x 36 floats; LN: full 128-column rows
-  static constexpr int STG_FLOATS_PER_WARP = (EPI == EPI_LN) ? 32 * STG_LD_LN : ((ES == 2 && EPI != EPI_PE) ? 32 * 64 / 4 : 32 * STG_LD);
+  static constexpr int STG_FLOATS_PER_WARP = (EPI == EPI_LN) ? 32 * STG_LD_LN : ((ES == 2 && EPI != EPI_PE && EPI != EPI_POOL) ? 32 * 64 / 4 : 32 * STG_LD);
   // gate: per 32-pair chunk 32 tanh biases | 32 sigmoid biases | 32 w_c (4 / NSUB chunks per warp);
-  // proj+embed: conv bias | gamma | beta (128 each)
-  static constexpr int COEF_FLOATS_PER_WARP = (EPI == EPI_GATE) ? 384 / NSUB : (EPI == EPI_PE) ? 384 : 0;
+  // proj+embed: conv bias | gamma | beta (128 each); cluster pool: per-cluster column sums of the warp's two 16-row halves
+  static constexpr int COEF_FLOATS_PER_WARP = (EPI == EPI_GATE) ? 384 / NSUB : (EPI == EPI_PE) ? 384 : (EPI == EPI_POOL) ? 2 * 16 * 32 : 0;
   static constexpr int GPART_FLOATS = (EPI == EPI_GATE && NSUB == 4) ? 2 * 8 * 32 : 0;   // partial-score exchange between warp pairs
   static constexpr int TMEM_COLS = (2 * BLOCK_N <= 64) ? 64 : (2 * BLOCK_N <= 128) ? 128 : (2 * BLOCK_N <= 256) ? 256 : 512;
   static constexpr size_t FIXED = 1024 /*align slack*/ + (size_t)EPI_WARPS * (STG_FLOATS_PER_WARP + COEF_FLOATS_PER_WARP + 96) * 4 +
@@ -465,6 +470,12 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           if (ea.dmean) inv = ik / (float)(ea.offsets[bg + 1] - ea.offsets[bg]);
         }
         mybag[lane] = bg; myw[lane] = wv; myinv[lane] = inv;
+      }
+      int pool_cid = -1;
+      if constexpr (EPI == EPI_POOL) {                     // cluster id and bag of this thread's row (-1: past the last row)
+        int bg = -1;
+        if (m_row < M) { pool_cid = reinterpret_cast<const int32_t*>(ea.relu_src)[m_row]; bg = bag_of_row(ea.offsets, ea.bags, m_row); }
+        mybag[lane] = bg;
       }
       if constexpr (EPI == EPI_GATE) {                     // this warp's 32-pair chunks: biases and w_c into shared memory
         constexpr int PCW = 4 / NSUB;                      // pair chunks per warp (a 256-column tile holds 4)
@@ -906,6 +917,69 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (m < M) *reinterpret_cast<float2*>(ea.emb + (size_t)(m >> 4) * 128 + k * 32 + c2) = make_float2(a0 * 0.0625f, a1 * 0.0625f);
             __syncwarp();
           }
+        }
+      } else if constexpr (EPI == EPI_POOL) {
+        // K9 (DeepAttMISL, model/backbone.py:105-117): v = relu(x W^T + b) is summed per (bag, cluster id) here and never
+        // written.  Bag lengths are multiples of 16 and a warp owns 32 aligned rows, so each 16-row half of a warp lies in
+        // one bag; a tile is 8 such segments.  Per 32-column chunk: lane c adds column c of its two halves, row by row, into
+        // per-cluster sums in shared memory; then (named barrier over the 4 epilogue warps) the 4 warps, a quarter of the
+        // clusters each, add each bag's segments in row order and write one partial per (tile, bag, cluster).
+        // No atomics: the result does not depend on scheduling.  cluster_pool_finalize adds the partials in a fixed order.
+        constexpr int NCH = BLOCK_N / 32;
+        const int ncl = ea.D;
+        float* sacc = coef;                                 // [2 halves][16 clusters][32 columns] of this warp
+        uint32_t* keep = reinterpret_cast<uint32_t*>(ea.out);
+        auto seg_bag = [&](int sg) { return rowbag[(sg >> 1) * 32 + (sg & 1) * 16]; };
+#pragma unroll 1
+        for (int ch = 0; ch < NCH; ++ch) {
+          const int col0 = n0 + ch * 32;
+          float v[32];
+          ld_acc(ch * 32, v);
+          if (ch == NCH - 1) { release_acc(&tempty[acc]); }
+#pragma unroll
+          for (int q = 0; q < 8; ++q) {
+            const float4 b4 = __ldg(reinterpret_cast<const float4*>(ea.bias + col0) + q);
+            v[4 * q] += b4.x; v[4 * q + 1] += b4.y; v[4 * q + 2] += b4.z; v[4 * q + 3] += b4.w;
+          }
+          if (keep && m_row < M) {
+            uint32_t kw = 0;
+#pragma unroll
+            for (int i = 0; i < 32; ++i) kw |= (v[i] > 0.f ? 1u : 0u) << i;
+            keep[(size_t)m_row * ea.ldo + (col0 >> 5)] = kw;
+          }
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i], 0.f);
+          stage_chunk(stg, STG_LD, 0, v, lane);
+          for (int k = 0; k < ncl; ++k) { sacc[k * 32 + lane] = 0.f; sacc[(16 + k) * 32 + lane] = 0.f; }
+          __syncwarp();
+#pragma unroll 4
+          for (int r = 0; r < 32; ++r) {
+            const int k = __shfl_sync(0xffffffffu, pool_cid, r);
+            const float xv = stg[r * STG_LD + lane];
+            if ((unsigned)k < (unsigned)ncl) sacc[((r >> 4) * 16 + k) * 32 + lane] += xv;
+          }
+          asm volatile("bar.sync 1, 128;" ::: "memory");      // the tile's 8 segments of this chunk are summed
+          // every warp writes the clusters k = wq, wq + 4, ... of each bag in the tile: the bag's segments (adjacent) are
+          // added in row order; the 8 loads are issued before the adds
+#pragma unroll 1
+          for (int sg = 0; sg < 8; ++sg) {
+            const int b = seg_bag(sg);
+            if (b < 0 || (sg > 0 && seg_bag(sg - 1) == b)) continue;     // not the first segment of its bag in this tile
+            int se = sg;
+            while (se < 7 && seg_bag(se + 1) == b) ++se;
+            float* dst = ea.part + (size_t)(mt + b) * ncl * N + col0 + lane;
+#pragma unroll 1
+            for (int k = wq; k < ncl; k += 4) {
+              float xs[8];
+#pragma unroll
+              for (int s2 = 0; s2 < 8; ++s2) xs[s2] = coef_all[(s2 >> 1) * Cfg::COEF_FLOATS_PER_WARP + ((s2 & 1) * 16 + k) * 32 + lane];
+              float t = 0.f;
+#pragma unroll
+              for (int s2 = 0; s2 < 8; ++s2) if (s2 >= sg && s2 <= se) t += xs[s2];
+              dst[(size_t)k * N] = t;
+            }
+          }
+          asm volatile("bar.sync 1, 128;" ::: "memory");      // before the next chunk overwrites the sums and the staging
         }
       } else if constexpr (EPI == EPI_GATE) {
         // BLOCK_N = 256 = two packed gate blocks (64 tanh | 64 sigmoid columns) = four 32-pair chunks; this warp owns
@@ -1371,6 +1445,39 @@ int tc_proj_embed_fwd(const void* x, const float* W1, const float* b1, const flo
   if (hdrop && drop2) { ea.out2 = hdrop; ea.drop2 = *drop2; }
   ea.h_cols = h; ea.bias2 = bc; ea.gamma = gamma; ea.beta = beta; ea.eps = eps; ea.y_pre = y_pre; ea.emb = emb;
   return launch_rows<bf16, 256, EPI_PE, true>((const bf16*)x, Wt, rows, C, h + d, ea, st);
+}
+
+// K9: relu(x W^T + b) reduced per (bag, cluster id) in the epilogue; part = [(rows / 128 + bags + 1) * ncl][N] column sums
+bool tc_proj_pool_supported(int rows, int C, int N, int dt) { return rows_ok(rows, dt) && C % kblk_of(dt) == 0 && pick_block_n(N) != 0; }
+template <typename T, bool X3>
+static int tc_proj_pool_t(const void* x, const T* W, const T* Wlo, const float* b, const int32_t* cid, const int32_t* offsets,
+                          int bags, int rows, int C, int N, int ncl, uint32_t* keep, float* part, cudaStream_t st) {
+  RowEpi ea{};
+  ea.out = keep; ea.ldo = N / 32; ea.bias = b; ea.part = part; ea.D = ncl; ea.relu_src = cid; ea.offsets = offsets; ea.bags = bags;
+  int bn = pick_block_n(N);
+  if (X3 && bn == 256) bn = 128;      // split tf32 doubles a stage: 256 columns leave room for one stage only
+  switch (bn) {
+    case 64: return launch_rows<T, 64, EPI_POOL, true, X3>((const T*)x, W, rows, C, N, ea, st, Wlo);
+    case 128: return launch_rows<T, 128, EPI_POOL, true, X3>((const T*)x, W, rows, C, N, ea, st, Wlo);
+    case 192: return launch_rows<T, 192, EPI_POOL, true, X3>((const T*)x, W, rows, C, N, ea, st, Wlo);
+    case 256: if constexpr (!X3) return launch_rows<T, 256, EPI_POOL, true, X3>((const T*)x, W, rows, C, N, ea, st, Wlo);
+  }
+  set_error("tc: unsupported N=%d", N);
+  return ADVMIL_ERR_INVALID;
+}
+int tc_proj_pool_fwd(const void* x, const float* W, const float* b, const int32_t* cid, const int32_t* offsets, int bags, int rows,
+                     int C, int N, int ncl, uint32_t* keep, float* part, int precision, cudaStream_t st) {
+  if (precision == ADVMIL_BF16) {
+    const bf16* Wt;
+    ADVMIL_TRY(weight_operand<bf16>(W, (size_t)N * C, WS_LINEAR, st, &Wt));
+    return tc_proj_pool_t<bf16, false>(x, Wt, nullptr, b, cid, offsets, bags, rows, C, N, ncl, keep, part, st);
+  }
+  if (precision == ADVMIL_TF32X3) {
+    const float *Wh, *Wl;
+    ADVMIL_TRY(weight_split(W, (size_t)N * C, WS_LINEAR, st, &Wh, &Wl));
+    return tc_proj_pool_t<float, true>(x, Wh, Wl, b, cid, offsets, bags, rows, C, N, ncl, keep, part, st);
+  }
+  return tc_proj_pool_t<float, false>(x, W, nullptr, b, cid, offsets, bags, rows, C, N, ncl, keep, part, st);
 }
 
 bool tc_gate_supported(int rows, int L, int D, int dt) { return rows_ok(rows, dt) && L % kblk_of(dt) == 0 && D % 128 == 0; }

@@ -12,6 +12,11 @@ bool tc_proj_embed_supported(int rows, int C, int h, int d, int dt);
 int tc_proj_embed_fwd(const void* x, const float* W1, const float* b1, const float* Wc, const float* bc, const float* gamma,
                       const float* beta, int rows, int C, int h, int d, float eps, void* hout, void* hdrop, const Drop* drop2,
                       void* y_pre, float* emb, cudaStream_t st);
+// K9: part[(m-tile + bag) * ncl + cluster][N] = column sums of relu(x W^T + b) over the tile's rows of that bag and cluster;
+// keep (optional) = the ReLU keep bits [rows][N / 32].  Every bag length a multiple of 16; ncl <= 16.
+bool tc_proj_pool_supported(int rows, int C, int N, int dt);
+int tc_proj_pool_fwd(const void* x, const float* W, const float* b, const int32_t* cid, const int32_t* offsets, int bags, int rows,
+                     int C, int N, int ncl, uint32_t* keep, float* part, int precision, cudaStream_t st);
 bool tc_gate_supported(int rows, int L, int D, int dt);
 int tc_gated_score_fwd(const void* v, const float* Wp, const float* bp, const float* wc, const float* bc, int rows,
                        int L, int D, const Drop& da, const Drop& db, void* ab, float* s, float* part, int precision,

@@ -67,6 +67,21 @@ int bwd_weight(const void* dY, const void* X, int rows, int N1, int N2, float* d
 int bwd_weight_conv3(const void* dY, const void* X, int rows, int N1, int C, float* dW, int accumulate, float* ws,
                      int precision, cudaStream_t st);
 
+// ---- cluster_pool.cu: K9 of the DeepAttMISL generator ------------------------------------------------------------------
+constexpr int CLUSTER_POOL_MAX = 16;     // clusters per bag the tcgen05 epilogue keeps sums for
+// true when cluster_pool_fwd runs for this shape and mode (tcgen05 engine; the fp32 mode composes linear_fwd and the
+// segment mean instead)
+bool cluster_pool_fused(int rows, int C, int h, int precision);
+size_t cluster_pool_ws_floats(int rows, int bags, int h, int ncl);
+// hc [bags * ncl, h] = per-(bag, cluster) mean of relu(x W^T + b), counts [bags * ncl]; keep (optional) [rows, h / 32] ReLU
+// keep bits; ws >= cluster_pool_ws_floats.  Every bag length a multiple of 16, 1 <= ncl <= CLUSTER_POOL_MAX.
+int cluster_pool_fwd(const void* x, const float* W, const float* b, const int32_t* cid, const int32_t* offsets,
+                     const int32_t* offsets_host, int rows, int bags, int C, int h, int ncl, int precision, float* hc,
+                     int32_t* counts, uint32_t* keep, float* ws, cudaStream_t st);
+// d_hx [rows, h] (T of precision) = keep * d_hc[bag, cid] / count
+int cluster_pool_bwd(const float* d_hc, const uint32_t* keep, const int32_t* cid, const int32_t* offsets, const int32_t* counts,
+                     int rows, int bags, int h, int ncl, int precision, void* d_hx, cudaStream_t st);
+
 // ---- rlip_chain.cu ----------------------------------------------------------------------------
 // fc1 MLP + GAPool gate of the RLIP head over R regions in one FFMA kernel (d == 128): writes f1 [R, d/2], fi [R, d],
 // ab [R, 2d] packed (optional) and the per-64-pair partial logits part [d/64][R] (finished by seg_softmax_pool_fwd)

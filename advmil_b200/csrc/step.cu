@@ -458,3 +458,263 @@ extern "C" int advmil_adv_step_esat_gen(const AdvmilEsatStepArgs* a, void* strea
   esat_request_overlap(0);
   return rc;
 }
+
+
+// =====================================================================================================================
+// The same two-phase step for the DeepAttMISL generator (bcb_mode `cluster`, model/backbone.py:89-123) with the RLIP
+// discriminator.  The disc phase runs K9 once -- projection, ReLU and the per-(bag, cluster) mean in one tcgen05 pass that
+// never writes the [rows, h] activation (cluster_pool.cu) -- and keeps hc, the counts and the ReLU keep bits in the
+// persistent region; the eval pass (disc phase) and the train pass (gen phase) of the attention stage both start from that
+// hc: phis has no dropout and G's parameters do not change between the phases.  The attention stage sees num_clusters rows
+// per bag and always runs in fp32 (like Generator.forward).  The fp32 mode (and any shape without the tcgen05 pass) composes
+// linear_fwd and the segment mean instead and keeps relu(x Wphi^T + b) itself for the backward.  The D part of both
+// phases is that of the ABMIL step: one shared region embedding, one batched head pass over [fake | real] pairs.
+// =====================================================================================================================
+namespace advmil {
+
+__global__ void iota_scaled_kernel(int n, int step, int32_t* __restrict__ out) {
+  pdl_prologue();
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i <= n) out[i] = i * step;
+}
+
+struct ClusterBufs { float* hc; int32_t* counts; uint32_t* keep; char* hx; int32_t* hoffs; };
+static size_t cluster_persist_bytes(int rows, int nb, int C, int h, int ncl, int precision) {
+  const size_t nbc = (size_t)nb * ncl;
+  const size_t act = cluster_pool_fused(rows, C, h, precision) ? (size_t)rows * (h / 32) * sizeof(uint32_t)
+                                                                : (size_t)rows * h * elem_bytes(elem_of_precision(precision));
+  return align_up(nbc * h * sizeof(float), 256) + align_up(nbc * sizeof(int32_t), 256) + align_up(act, 256) +
+         align_up((nb + 1) * sizeof(int32_t), 256) + 4 * 256;
+}
+static int take_cluster(Workspace& ws, int rows, int nb, int C, int h, int ncl, int precision, ClusterBufs& B) {
+  const size_t nbc = (size_t)nb * ncl;
+  B = ClusterBufs{};
+  B.hc = ws.take<float>(nbc * h);
+  B.counts = ws.take<int32_t>(nbc);
+  if (cluster_pool_fused(rows, C, h, precision)) B.keep = ws.take<uint32_t>((size_t)rows * (h / 32));
+  else B.hx = ws.take<char>((size_t)rows * h * elem_bytes(elem_of_precision(precision)));
+  B.hoffs = ws.take<int32_t>(nb + 1);
+  if (!B.hc || !B.counts || !(B.keep || B.hx) || !B.hoffs) { set_error("adv_step_cluster: workspace too small (have %zu bytes)", ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  return ADVMIL_OK;
+}
+// packed view of hc: num_clusters fp32 rows of width h per bag
+static AdvmilBags cluster_bags(const ClusterBufs& B, int nb, int ncl, int h, std::vector<int32_t>& offs_host) {
+  offs_host.resize(nb + 1);
+  for (int i = 0; i <= nb; ++i) offs_host[i] = i * ncl;
+  AdvmilBags cb{};
+  cb.x = B.hc; cb.offsets = B.hoffs; cb.offsets_host = offs_host.data();
+  cb.rows = nb * ncl; cb.bags = nb; cb.C = h; cb.max_bag_rows = ncl; cb.elem = ELEM_F32;
+  return cb;
+}
+static int cluster_step_check(const AdvmilClusterStepArgs* ca) {
+  ADVMIL_REQUIRE(ca, "adv_step_cluster: null argument");
+  const AdvmilStepArgs* a = &ca->base;
+  ADVMIL_REQUIRE(a->gen && a->disc && a->bags && a->t && a->e && a->visible && a->losses && a->workspace && ca->Wphi && ca->bphi && ca->cid,
+                 "adv_step_cluster: null argument");
+  ADVMIL_REQUIRE(a->gen->W0 && !a->gen->Wrho, "adv_step_cluster: the attention stage has no rho layer and needs the noise head");
+  ADVMIL_REQUIRE(a->gen->noise0 == 0, "adv_step_cluster: noise on the first head layer (gen_noi_noise '1-*') is not covered by the fused step");
+  ADVMIL_REQUIRE(a->gen->C == a->gen->h, "adv_step_cluster: the attention stage reads the h-wide cluster means (C %d != h %d)", a->gen->C, a->gen->h);
+  ADVMIL_REQUIRE(a->disc->ksize == 0 || a->disc->ksize == 1, "adv_step_cluster: the fused step covers the ksize-1 discriminator");
+  ADVMIL_REQUIRE(ca->num_clusters >= 1 && ca->num_clusters <= CLUSTER_POOL_MAX, "adv_step_cluster: num_clusters %d outside 1..%d",
+                 ca->num_clusters, CLUSTER_POOL_MAX);
+  const AdvmilBags* b = a->bags;
+  ADVMIL_REQUIRE(b->offsets_host && b->bags > 0 && b->offsets_host[0] == 0 && b->offsets_host[b->bags] == b->rows, "bags: bad offsets");
+  for (int i = 0; i < b->bags; ++i)
+    ADVMIL_REQUIRE((b->offsets_host[i + 1] - b->offsets_host[i]) % 16 == 0,
+                   "bags: bag %d has a length that is not a multiple of 16 (model/backbone_utils.py:65)", i);
+  return ADVMIL_OK;
+}
+static size_t disc_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb, int precision) {
+  const size_t es = elem_bytes(elem_of_precision(precision)), R = rows / 16;
+  return align_up(2 * R * d->d * sizeof(float), 256) + align_up(rows * d->d * es, 256) + head_bytes(*d, 2 * R, 2 * nb) +
+         align_up(2 * R * d->d * sizeof(float), 256) + 8 * 256 + 6 * nb * sizeof(float) + align_up((2 * nb + 2) * sizeof(int32_t), 256) +
+         advmil_disc_workspace_bytes(d, 2 * rows, 2 * nb, 1) + 256;
+}
+static size_t gen_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb) {
+  const size_t R = rows / 16;
+  return align_up(R * d->d * sizeof(float), 256) + head_bytes(*d, R, nb) + 8 * 256 + 4 * nb * sizeof(float) +
+         advmil_disc_workspace_bytes(d, rows, nb, 1) + 256;
+}
+// D phase after pred_d exists: shared region embedding, batched head over [fake | real] pairs, D loss, D backward
+static int disc_rlip(const AdvmilStepArgs* a, Workspace& ws, cudaStream_t st) {
+  const AdvmilDiscParams& dp = *a->disc;
+  const AdvmilBags* bags = a->bags;
+  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  const size_t es = elem_bytes(elem_of_precision(a->precision));
+  const bool batched = a->n_real > 0.f;                 // no real pair anywhere: only the fake half runs
+  STEP_TAKE(emb2, float, (size_t)2 * R * d);
+  STEP_TAKE(y_pre, char, (size_t)rows * d * es);
+  AdvmilEmbedActs ea{};
+  ea.emb = emb2; ea.y_pre = y_pre; ea.precision = a->precision;
+  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
+  AdvmilHeadActs ha{};
+  if (!take_head(ws, dp, 2 * (size_t)R, 2 * (size_t)nb, ha)) { set_error("adv_step_cluster_disc: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
+  STEP_TAKE(d_emb2, float, (size_t)2 * R * d);
+  STEP_TAKE(t2, float, 2 * nb);
+  STEP_TAKE(d_out2, float, 2 * nb);
+  STEP_TAKE(offs2, int32_t, 2 * nb + 2);
+  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, 2 * rows, 2 * nb, 1);
+  STEP_TAKE(dws, char, dws_bytes);
+  std::vector<int32_t> offs2_host(2 * nb + 1);
+  for (int i = 0; i <= nb; ++i) { offs2_host[i] = bags->offsets_host[i]; offs2_host[nb + i] = bags->offsets_host[i] + rows; }
+  launch_k(dup_offsets_kernel, dim3(cdiv(nb + 1, 128)), dim3(128), 0, st, bags->offsets, nb, rows, offs2);
+  ADVMIL_CHECK_LAUNCH();
+  launch_k(real_mask_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, a->e, a->visible, nb, a->real_mask);
+  ADVMIL_CHECK_LAUNCH();
+  ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2, a->pred_d, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  if (batched) {
+    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2 + nb, a->t, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(emb2 + (size_t)R * d, emb2, (size_t)R * d * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
+  AdvmilBags vb = *bags;
+  vb.offsets = offs2; vb.offsets_host = offs2_host.data(); vb.rows = batched ? 2 * rows : rows; vb.bags = batched ? 2 * nb : nb;
+  ha.emb = emb2; ha.t = t2; ha.out = a->f_fake_d;
+  ha.mask_fc1 = a->d_mask_fc1; ha.mask_ga = a->d_mask_ga; ha.mask_gs = a->d_mask_gs; ha.mask_fc2 = a->d_mask_fc2;
+  ha.seed = a->seed_d; ha.train = 1; ha.precision = a->precision; ha.workspace = dws; ha.workspace_bytes = dws_bytes;
+  ADVMIL_TRY(advmil_disc_head_fwd(&dp, &vb, &ha, (void*)st));
+  ADVMIL_TRY(advmil_disc_loss(a->f_fake_d + nb, a->f_fake_d, a->real_mask, nb, a->loss_d, a->n_real, a->n_fake, a->losses,
+                              d_out2 + nb, d_out2, (void*)st));
+  ADVMIL_TRY(advmil_disc_head_bwd(&dp, &vb, &ha, d_out2, d_emb2, nullptr, a->disc_grads, 0, (void*)st));
+  ea.workspace = dws; ea.workspace_bytes = dws_bytes;
+  return disc_embed_bwd_impl(&dp, bags, &ea, d_emb2, batched ? d_emb2 + (size_t)R * d : nullptr, a->disc_grads, 0, st);
+}
+// G phase after pred_g exists: D(x, pred_g) in eval mode, G loss, and dL/dpred_g (recon + the adversarial term through D)
+static int gen_rlip(const AdvmilStepArgs* a, Workspace& ws, float* d_pred, cudaStream_t st) {
+  const AdvmilDiscParams& dp = *a->disc;
+  const AdvmilBags* bags = a->bags;
+  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  STEP_TAKE(emb, float, (size_t)R * d);
+  AdvmilEmbedActs ea{};
+  ea.emb = emb; ea.y_pre = nullptr; ea.precision = a->precision;
+  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
+  AdvmilHeadActs ha{};
+  if (!take_head(ws, dp, R, nb, ha)) { set_error("adv_step_cluster_gen: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
+  STEP_TAKE(d_fake, float, nb);
+  STEP_TAKE(d_t, float, nb);
+  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, rows, nb, 1);
+  STEP_TAKE(dws, char, dws_bytes);
+  ha.ab = nullptr;
+  ha.emb = emb; ha.t = a->pred_g; ha.out = a->f_fake_g; ha.seed = 0; ha.train = 0; ha.precision = a->precision;
+  ha.workspace = dws; ha.workspace_bytes = dws_bytes;
+  ADVMIL_TRY(advmil_disc_head_fwd(&dp, bags, &ha, (void*)st));
+  ADVMIL_TRY(advmil_gen_loss(a->pred_g, a->t, a->e, a->visible, a->f_fake_g, nb, a->n_visible, a->n_fake, a->coef_gan,
+                             a->recon_alpha, a->recon_gamma, a->recon_norm, a->losses + 1, d_pred, d_fake, (void*)st));
+  ADVMIL_TRY(advmil_disc_head_bwd(&dp, bags, &ha, d_fake, nullptr, d_t, nullptr, 0, (void*)st));
+  launch_k(add_inplace_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, d_pred, d_t, nb);
+  ADVMIL_CHECK_LAUNCH();
+  return ADVMIL_OK;
+}
+}  // namespace advmil
+
+extern "C" size_t advmil_adv_step_cluster_workspace_bytes(const AdvmilGenParams* g, const AdvmilDiscParams* d, int32_t rows,
+                                                          int32_t bags, int32_t num_clusters, int32_t precision) {
+  const int C = d->C, h = g->h, ncl = num_clusters;
+  const size_t nb = bags, nbc = nb * ncl, abw = gate_width(h);
+  const size_t es = elem_bytes(elem_of_precision(precision));
+  const bool fused = cluster_pool_fused(rows, C, h, precision);
+  const size_t persistent = cluster_persist_bytes(rows, bags, C, h, ncl, precision);
+  const size_t k9 = fused ? align_up(cluster_pool_ws_floats(rows, bags, h, ncl) * sizeof(float), 256)
+                          : advmil_segment_mean_workspace_bytes(rows, bags, h, ncl) + 256;
+  const size_t disc = k9 + gen_bufs_bytes(*g, nbc, nb) + align_up(nbc * h * sizeof(float), 256) +
+                      advmil_generator_workspace_bytes(g, (int)nbc, bags, 0) + 256 + disc_part_bytes(d, rows, nb, precision);
+  const size_t gen = gen_bufs_bytes(*g, nbc, nb) + align_up(nbc * h * sizeof(float), 256) + align_up(nbc * abw * sizeof(float), 256) +
+                     advmil_generator_workspace_bytes(g, (int)nbc, bags, 1) + 256 + align_up(nb * sizeof(float), 256) +
+                     align_up(nbc * h * sizeof(float), 256) + align_up((size_t)rows * h * es, 256) +
+                     align_up(bwd_weight_ws_floats(rows, h, C) * sizeof(float), 256) + align_up((size_t)row_chunks(rows) * h * sizeof(float), 256) +
+                     gen_part_bytes(d, rows, nb);
+  return persistent + (disc > gen ? disc : gen) + 4096;
+}
+
+extern "C" int advmil_adv_step_cluster_disc(const AdvmilClusterStepArgs* ca, void* stream) {
+  ADVMIL_TRY(cluster_step_check(ca));
+  const AdvmilStepArgs* a = &ca->base;
+  ADVMIL_REQUIRE(a->disc_grads && a->pred_d && a->f_fake_d && a->real_mask && a->noise_d, "adv_step_cluster_disc: missing buffers");
+  cudaStream_t st = (cudaStream_t)stream;
+  const AdvmilGenParams& gp = *a->gen;
+  const AdvmilBags* bags = a->bags;
+  const int rows = bags->rows, nb = bags->bags, C = bags->C, h = gp.h, ncl = ca->num_clusters, nbc = nb * ncl;
+  const int prec = a->precision;
+  ADVMIL_REQUIRE(C == a->disc->C && bags->elem == elem_of_precision(prec), "adv_step_cluster_disc: x width %d / element type do not match", C);
+  Workspace ws(a->workspace, a->workspace_bytes);
+  ClusterBufs B;
+  ADVMIL_TRY(take_cluster(ws, rows, nb, C, h, ncl, prec, B));
+  // ---- K9 once per step: hc, counts and the backward's ReLU mask stay in the persistent region ----
+  if (cluster_pool_fused(rows, C, h, prec)) {
+    STEP_TAKE(part, float, cluster_pool_ws_floats(rows, nb, h, ncl));
+    ProfScope ps(PROF_PROJ_SEGMEAN, st);
+    ADVMIL_TRY(cluster_pool_fwd(bags->x, ca->Wphi, ca->bphi, ca->cid, bags->offsets, bags->offsets_host, rows, nb, C, h, ncl, prec,
+                                B.hc, B.counts, B.keep, part, st));
+  } else {
+    const size_t sm_bytes = advmil_segment_mean_workspace_bytes(rows, nb, h, ncl);
+    STEP_TAKE(smws, char, sm_bytes);
+    Drop none = Drop::make(nullptr, 0, 0, 0.f, 0, 0);
+    { ProfScope ps(PROF_PROJ, st); ADVMIL_TRY(linear_fwd(bags->x, ca->Wphi, ca->bphi, rows, C, h, 1, none, B.hx, prec, st)); }
+    ADVMIL_TRY(advmil_segment_mean_by_id_fwd(B.hx, elem_of_precision(prec), ca->cid, bags->offsets, bags->offsets_host, rows, nb, h, ncl,
+                                             B.hc, B.counts, smws, sm_bytes, stream));
+  }
+  launch_k(iota_scaled_kernel, dim3(cdiv(nb + 1, 128)), dim3(128), 0, st, nb, ncl, B.hoffs);
+  ADVMIL_CHECK_LAUNCH();
+  // ---- attention stage, eval mode, detached (model_handler.py:383-387) ----
+  std::vector<int32_t> hoffs_host;
+  const AdvmilBags cb = cluster_bags(B, nb, ncl, h, hoffs_host);
+  GenBufs gb;
+  if (!take_gen(ws, gp, nbc, nb, gb)) { set_error("adv_step_cluster_disc: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
+  STEP_TAKE(hh, float, (size_t)nbc * h);
+  const size_t gws_bytes = advmil_generator_workspace_bytes(&gp, nbc, nb, 0);
+  STEP_TAKE(gws, char, gws_bytes);
+  AdvmilGenActs ga{};
+  ga.h = hh; ga.ab = nullptr; ga.s = gb.s; ga.w = gb.w; ga.z = gb.z; ga.H = gb.H; ga.H1 = gb.H1; ga.pre = gb.pre;
+  ga.pred = a->pred_d; ga.noise0 = nullptr; ga.noise1 = a->noise_d;
+  ga.seed = 0; ga.train = 0; ga.precision = ADVMIL_FP32; ga.workspace = gws; ga.workspace_bytes = gws_bytes;
+  ADVMIL_TRY(advmil_generator_fwd(&gp, &cb, &ga, stream));
+  return disc_rlip(a, ws, st);
+}
+
+extern "C" int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* ca, void* stream) {
+  ADVMIL_TRY(cluster_step_check(ca));
+  const AdvmilStepArgs* a = &ca->base;
+  ADVMIL_REQUIRE(a->gen_grads && a->pred_g && a->f_fake_g && a->noise_g && ca->dWphi && ca->dbphi, "adv_step_cluster_gen: missing buffers");
+  cudaStream_t st = (cudaStream_t)stream;
+  const AdvmilGenParams& gp = *a->gen;
+  const AdvmilBags* bags = a->bags;
+  const int rows = bags->rows, nb = bags->bags, C = bags->C, h = gp.h, ncl = ca->num_clusters, nbc = nb * ncl;
+  const int prec = a->precision, dt = elem_of_precision(prec);
+  Workspace ws(a->workspace, a->workspace_bytes);
+  ClusterBufs B;                                    // hc / counts / keep bits were written by advmil_adv_step_cluster_disc
+  ADVMIL_TRY(take_cluster(ws, rows, nb, C, h, ncl, prec, B));
+  // ---- attention stage, train mode, on the same hc ----
+  std::vector<int32_t> hoffs_host;
+  const AdvmilBags cb = cluster_bags(B, nb, ncl, h, hoffs_host);
+  GenBufs gb;
+  if (!take_gen(ws, gp, nbc, nb, gb)) { set_error("adv_step_cluster_gen: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
+  STEP_TAKE(hh, float, (size_t)nbc * h);
+  STEP_TAKE(ab, float, (size_t)nbc * gate_width(h));
+  const size_t gws_bytes = advmil_generator_workspace_bytes(&gp, nbc, nb, 1);
+  STEP_TAKE(gws, char, gws_bytes);
+  AdvmilGenActs ga{};
+  ga.h = hh; ga.ab = ab; ga.s = gb.s; ga.w = gb.w; ga.z = gb.z; ga.H = gb.H; ga.H1 = gb.H1; ga.pre = gb.pre;
+  ga.pred = a->pred_g; ga.noise0 = nullptr; ga.noise1 = a->noise_g;
+  ga.mask_h = a->g_mask_h; ga.mask_a = a->g_mask_a; ga.mask_b = a->g_mask_b; ga.mask_rho = nullptr; ga.mask_mlp0 = a->g_mask_mlp0;
+  ga.seed = a->seed_g; ga.train = 1; ga.precision = ADVMIL_FP32; ga.workspace = gws; ga.workspace_bytes = gws_bytes;
+  ADVMIL_TRY(advmil_generator_fwd(&gp, &cb, &ga, stream));
+  // ---- D(x, pred_g), G loss, dL/dpred_g ----
+  STEP_TAKE(d_pred, float, nb);
+  ADVMIL_TRY(gen_rlip(a, ws, d_pred, st));
+  // ---- attention stage backward down to d_hc, then K9's backward and dWphi / dbphi ----
+  STEP_TAKE(d_hc, float, (size_t)nbc * h);
+  AdvmilGenGrads gg = *a->gen_grads;
+  gg.dx = d_hc;
+  ADVMIL_TRY(advmil_generator_bwd(&gp, &cb, &ga, d_pred, &gg, stream));
+  STEP_TAKE(d_hx, char, (size_t)rows * h * elem_bytes(dt));
+  if (B.keep) {
+    ProfScope ps(PROF_BWD_DATA, st);
+    ADVMIL_TRY(cluster_pool_bwd(d_hc, B.keep, ca->cid, bags->offsets, B.counts, rows, nb, h, ncl, prec, d_hx, st));
+  } else {
+    ADVMIL_TRY(advmil_segment_mean_by_id_bwd(d_hc, B.hx, dt, ca->cid, bags->offsets, B.counts, rows, nb, h, ncl, 1, d_hx, stream));
+  }
+  STEP_TAKE(bwws, float, bwd_weight_ws_floats(rows, h, C));
+  { ProfScope ps(PROF_BWD_W_PROJ, st); ADVMIL_TRY(bwd_weight(d_hx, bags->x, rows, h, C, ca->dWphi, 0, bwws, prec, st)); }
+  STEP_TAKE(csws, float, (size_t)row_chunks(rows) * h);
+  { ProfScope ps(PROF_COLSUM, st); ADVMIL_TRY(colsum(d_hx, dt, rows, h, h, ca->dbphi, 0, csws, st)); }
+  return ADVMIL_OK;
+}

@@ -118,6 +118,11 @@ class DeepAttMISL(_GatedMILBase):
         return ops.GenConfig(C=h, h=h, o=h, hid=hid, noise0=noise[0], noise1=noise[1], out_scale=out_scale,
                              p_backbone=self.p, p_head=p_head, has_rho=False)
 
+    def phi_params(self):
+        """The parameters of phis.0: the 1x1 conv weight [h, C, 1, 1] (contiguous: the memory of the [h, C] projection
+        weight) and its bias [h]."""
+        return self.phis[0].weight, self.phis[0].bias
+
     def cluster_rows(self, x_path: torch.Tensor, cluster_id: torch.Tensor, lengths=None, offsets=None) -> torch.Tensor:
         """[rows,C] (+ ids) -> per-(bag, cluster) mean of relu(phis(x)) [bags*num_clusters, h], differentiable.
         offsets: the packed bags' int32 device offsets when the caller already has them (building them here costs a

@@ -120,7 +120,8 @@ class AdvStep(_DataParallelMixin):
                  loss_d="bce", recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32",
                  process_group=None):
         if netG.backbone.kind != "abmil":
-            raise NotImplementedError("AdvStep is the C-fused step of the ABMIL generator; use ModuleAdvStep for bcb_mode "
+            other = {"cluster": "ClusterAdvStep", "patch": "EsatAdvStep"}.get(netG.backbone.kind, "ModuleAdvStep")
+            raise NotImplementedError(f"AdvStep is the C-fused step of the ABMIL generator; use {other} for bcb_mode "
                                       f"'{netG.backbone.kind}'")
         if list(netG.noise) != [0, 1]:
             raise NotImplementedError(f"AdvStep covers gen_noi_noise '0-1' (config/cfg_nlst.yaml:30), got {list(netG.noise)}: noise "
@@ -344,6 +345,117 @@ class EsatAdvStep(AdvStep):
         out["f_fake_d"] = out["f_d"][:nb]
         out["f_real"] = out["f_d"][nb:] if n_real > 0 else None
         out["_keep"] = (t, e, visible, noise_d, noise_g, pe, bags)
+        self._inflight = out
+        return out
+
+
+class ClusterAdvStep(AdvStep):
+    """The C-fused adversarial step for the DeepAttMISL generator (`bcb_mode: cluster`) with the RLIP discriminator:
+    `advmil_adv_step_cluster_disc / _gen` issue the launch sequence of `ModuleAdvStep` from two host calls.  The projection
+    of phis runs once per step: one tcgen05 pass computes relu(x Wphi^T + b), its per-(bag, cluster) means and the ReLU keep
+    bits without writing the activation (the fp32 mode composes the FFMA projection and the segment mean), and the D
+    phase's eval pass and the G phase's train pass of the attention stage both start from those means.  Same step
+    semantics, outputs and `loss_dict` as `AdvStep` (model/model_handler.py:349-498).  `step(..., ext=cluster ids)`;
+    injected generator masks are over the attention stage's [bags * num_clusters, h] rows, as in `ModuleAdvStep`."""
+
+    def __init__(self, netG, netD, lr_g=8e-5, lr_d=8e-5, weight_decay_g=5e-4, coef_gan=0.004, coef_l1=1e-5,
+                 loss_d="bce", recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32", process_group=None):
+        bb = netG.backbone
+        if bb.kind != "cluster":
+            raise NotImplementedError(f"ClusterAdvStep is the C-fused step of the DeepAttMISL generator, got bcb_mode '{bb.kind}': "
+                                      "use AdvStep (abmil), EsatAdvStep (patch) or ModuleAdvStep")
+        if list(netG.noise) != [0, 1]:
+            raise NotImplementedError(f"ClusterAdvStep covers gen_noi_noise '0-1', got {list(netG.noise)}: use ModuleAdvStep")
+        if not 1 <= bb.num_clusters <= 16:
+            raise NotImplementedError(f"ClusterAdvStep covers 1..16 clusters, got {bb.num_clusters}: use ModuleAdvStep")
+        if netD.config().ksize not in (0, 1):
+            raise NotImplementedError("ClusterAdvStep covers the ksize-1 discriminator: use ModuleAdvStep")
+        self.netG, self.netD = netG, netD
+        self.gcfg, self.dcfg = netG.config(), netD.config()
+        self.gparams, self.dparams = netG.gen_params(), netD.disc_params()
+        self.G = FlatParams(netG, list(netG.parameters()), weight_decay_rule=True)
+        self.Wphi, self.bphi = bb.phi_params()            # after FlatParams: views of the flat buffer
+        self.D = FlatParams(netD, self.dparams, weight_decay_rule=False)
+        self.ggrads, self.dgrads = self.G.grads_for(self.gparams), self.D.grads_for(self.dparams)
+        self.dWphi, self.dbphi = self.G.grads_for([self.Wphi, self.bphi])
+        covered = [t for t in self.gparams if t is not None] + [self.Wphi, self.bphi]
+        assert self.G.total == sum((t.numel() + 3) // 4 * 4 for t in covered), "generator parameters outside the cluster step"
+        self.lr_g, self.lr_d, self.wd_g = lr_g, lr_d, weight_decay_g
+        self.coef_gan, self.coef_l1 = coef_gan, coef_l1
+        self.loss_d = {"bce": 0, "hinge": 1, "wasserstein": 2}[loss_d]
+        self.recon = ({"l1": 0, "l2": 1}[recon_norm], recon_alpha, recon_gamma)
+        self.precision = ops.PRECISIONS[precision]
+        self._inflight = None
+        self._init_dp(process_group)
+
+    def step(self, bags: ops.PackedBags, t: torch.Tensor, e: torch.Tensor, visible: torch.Tensor,
+             noise_d: Optional[torch.Tensor] = None, noise_g: Optional[torch.Tensor] = None, ext=None,
+             masks_d_real=None, masks_d_fake=None, masks_g=None, global_counts=None) -> Dict:
+        """ext: the cluster id of every row, [rows] or [1, rows], float (what the handler passes) or int32 (used as is)."""
+        if ext is None:
+            raise ValueError("ClusterAdvStep.step needs the cluster id of every row (ext)")
+        lib = _lib.load()
+        st = torch.cuda.current_stream().cuda_stream
+        bags = bags.for_precision(self.precision)
+        dev, nb = bags.x.device, bags.bags
+        cid = ext.reshape(-1)
+        cid = (cid if cid.dtype == torch.int32 else cid.to(torch.int32)).contiguous()
+        assert cid.numel() == bags.rows and cid.device == dev, "one cluster id per row, on the bags' device"
+        f32 = dict(dtype=torch.float32, device=dev)
+        t = t.reshape(-1).contiguous().float()
+        e = e.reshape(-1).contiguous().float()
+        visible = visible.reshape(-1).to(torch.uint8).contiguous()
+        if global_counts is None:
+            real_mask = ((e == 1) & (visible != 0))
+            cnt = torch.stack([real_mask.sum(), torch.tensor(nb, device=dev), visible.sum()]).float()
+            self._allreduce(cnt)
+            n_real, n_fake, n_vis = [float(v) for v in cnt.tolist()]
+        else:
+            n_real, n_fake, n_vis = [float(v) for v in global_counts]
+        noise_d = (noise_d if noise_d is not None else self._draw(nb, dev)).contiguous().float()
+        noise_g = (noise_g if noise_g is not None else self._draw(nb, dev)).contiguous().float()
+        gp, dp, gg, dg = self._structs()
+        ncl = self.netG.backbone.num_clusters
+        need = lib.advmil_adv_step_cluster_workspace_bytes(C.byref(gp), C.byref(dp), bags.rows, nb, ncl, self.precision)
+        ws = getattr(self, "_ws", None)
+        if ws is None or ws.numel() < need or ws.device != dev:
+            self._ws = ws = torch.empty(int(need * 1.05) + 4096, dtype=torch.uint8, device=dev)      # grow-only
+        out = {"losses": torch.zeros(8, **f32), "pred_d": torch.empty(nb, **f32), "pred_g": torch.empty(nb, **f32),
+               "f_d": torch.empty(2 * nb, **f32), "f_fake_g": torch.empty(nb, **f32),
+               "real_mask": torch.empty(nb, dtype=torch.uint8, device=dev)}
+        md = self._cat_masks(masks_d_fake, masks_d_real, ("fc1", "ga", "gs", "fc2"))
+        mg = {k: v.contiguous() for k, v in (masks_g or {}).items()}
+        b = bags.c()
+        ca = _lib.ClusterStepArgs()
+        a = ca.base
+        a.gen, a.disc, a.gen_grads, a.disc_grads, a.bags = C.pointer(gp), C.pointer(dp), C.pointer(gg), C.pointer(dg), C.pointer(b)
+        a.t, a.e, a.visible = t.data_ptr(), e.data_ptr(), visible.data_ptr()
+        a.noise_d, a.noise_g = noise_d.data_ptr(), noise_g.data_ptr()
+        for k in ("h", "a", "b", "mlp0"):
+            setattr(a, "g_mask_" + k, ops._ptr(mg.get(k)))
+        for k in ("fc1", "ga", "gs", "fc2"):
+            setattr(a, "d_mask_" + k, ops._ptr(md.get(k)))
+        a.seed_d, a.seed_g = self._seed(), self._seed()
+        a.n_real, a.n_fake, a.n_visible, a.loss_d = n_real, n_fake, n_vis, self.loss_d
+        a.recon_norm, a.recon_alpha, a.recon_gamma = self.recon
+        a.coef_gan, a.precision = self.coef_gan, self.precision
+        a.losses, a.pred_d, a.f_fake_d, a.real_mask = (out["losses"].data_ptr(), out["pred_d"].data_ptr(),
+                                                       out["f_d"].data_ptr(), out["real_mask"].data_ptr())
+        a.pred_g, a.f_fake_g = out["pred_g"].data_ptr(), out["f_fake_g"].data_ptr()
+        a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
+        ca.Wphi, ca.bphi, ca.dWphi, ca.dbphi = self.Wphi.data_ptr(), self.bphi.data_ptr(), self.dWphi.data_ptr(), self.dbphi.data_ptr()
+        ca.cid, ca.num_clusters = cid.data_ptr(), ncl
+        check(lib.advmil_adv_step_cluster_disc(C.byref(ca), st), "advmil_adv_step_cluster_disc")
+        self._allreduce(self.D.grad)
+        self.D.adam(self.lr_d)
+        check(lib.advmil_adv_step_cluster_gen(C.byref(ca), st), "advmil_adv_step_cluster_gen")
+        if self.coef_l1 > 1e-8:
+            check(lib.advmil_abs_sum(self.G.flat.data_ptr(), self.G.total, out["losses"][4:].data_ptr(), st), "advmil_abs_sum")
+        self._allreduce(self.G.grad)
+        self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
+        out["f_fake_d"] = out["f_d"][:nb]
+        out["f_real"] = out["f_d"][nb:] if n_real > 0 else None
+        out["_keep"] = (t, e, visible, noise_d, noise_g, md, mg, cid, bags)
         self._inflight = out
         return out
 

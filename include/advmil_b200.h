@@ -178,7 +178,8 @@ typedef struct AdvmilHeadActs {       /* K7+K8: region MLP, GAPool, bag MLP, tim
 ADVMIL_API int advmil_abi_version(void);
 ADVMIL_API const char* advmil_last_error(void);
 /* sizeof() of the ABI structs, for binding self-checks: which = 0 Bags, 1 GenParams, 2 GenGrads, 3 GenActs,
- * 4 DiscParams, 5 DiscGrads, 6 EmbedActs, 7 HeadActs, 8 StepArgs, 9 EsatParams, 10 EsatGrads, 11 EsatActs, 12 EsatStepArgs */
+ * 4 DiscParams, 5 DiscGrads, 6 EmbedActs, 7 HeadActs, 8 StepArgs, 9 EsatParams, 10 EsatGrads, 11 EsatActs, 12 EsatStepArgs,
+ * 13 ClusterStepArgs */
 ADVMIL_API size_t advmil_abi_sizeof(int which);
 /* counts kernel launches issued by this library since the last reset (bench "gpu_launches") */
 ADVMIL_API int64_t advmil_launch_count(int reset);
@@ -241,6 +242,23 @@ ADVMIL_API int advmil_segment_mean_by_id_fwd(const void* v /*elem*/, int32_t ele
 ADVMIL_API int advmil_segment_mean_by_id_bwd(const float* d_out, const void* v /*elem*/, int32_t elem, const int32_t* cid,
                                   const int32_t* offsets, const int32_t* counts, int32_t rows, int32_t bags, int32_t width,
                                   int32_t num_clusters, int32_t relu_mask, void* d_v /*elem*/, void* stream);
+
+/* The same K9 as ONE tcgen05 pass (ADVMIL_TF32 / ADVMIL_TF32X3 / ADVMIL_BF16; the fp32 mode has no such pass): hc[b,c] =
+ * per-(bag, cluster) mean of relu(x W^T + b) (x [rows,C] of the precision's element type, W [h,C], b [h]), counts
+ * [bags*num_clusters] int32; keep (optional, device uint32 [rows, h/32]): the ReLU keep bits (pre-activation > 0), bit i of
+ * word j = column 32 j + i.  The [rows,h] activation is never written.  Rows whose id is outside [0, num_clusters) count
+ * nowhere.  Every bag length must be a multiple of 16 and 1 <= num_clusters <= 16, else ADVMIL_ERR_INVALID.  Deterministic
+ * (no floating-point atomics).  workspace >= advmil_cluster_pool_workspace_bytes. */
+ADVMIL_API size_t advmil_cluster_pool_workspace_bytes(int32_t rows, int32_t bags, int32_t h, int32_t num_clusters);
+ADVMIL_API int advmil_cluster_pool_fwd(const void* x, const float* W, const float* b, const int32_t* cid, const int32_t* offsets,
+                                       const int32_t* offsets_host, int32_t rows, int32_t bags, int32_t C, int32_t h,
+                                       int32_t num_clusters, int32_t precision, float* hc, int32_t* counts, uint32_t* keep,
+                                       void* workspace, size_t workspace_bytes, void* stream);
+/* its backward: d_hx[n,:] = keep(n,:) * d_hc[bag(n), cid[n], :] / count (element type of precision; zeros for ids outside
+ * [0, num_clusters)) */
+ADVMIL_API int advmil_cluster_pool_bwd(const float* d_hc, const uint32_t* keep, const int32_t* cid, const int32_t* offsets,
+                                       const int32_t* counts, int32_t rows, int32_t bags, int32_t h, int32_t num_clusters,
+                                       int32_t precision, void* d_hx, void* stream);
 
 /* ---- stage-level entry points (also used by the DeepAttMISL path and by the kernel unit tests) ---- */
 /* y = act(x W^T + b): act 0 none, 1 relu; optional dropout (p, mask or seed/site) -> y [rows,N].  W: [N,K] fp32.
@@ -351,6 +369,29 @@ ADVMIL_API size_t advmil_adv_step_workspace_bytes(const AdvmilGenParams* gen, co
                                        int32_t bags, int32_t precision);
 ADVMIL_API int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream);
 ADVMIL_API int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream);
+
+/* ---- the same two-phase step for the DeepAttMISL generator (bcb_mode `cluster`, model/backbone.py:89-123) with the RLIP
+ *      discriminator.  The disc phase runs K9 (advmil_cluster_pool_fwd) once and keeps hc, counts and the ReLU keep bits in
+ *      the workspace (the fp32 mode keeps relu(x Wphi^T + b) itself); the eval and the train pass of the attention stage
+ *      (num_clusters rows per bag, always ADVMIL_FP32) both start from that hc: phis has no dropout and G's parameters do
+ *      not change between the phases.  Same semantics, outputs and loss layout as advmil_adv_step_disc / _gen.
+ *      base.gen: the attention stage (C = h) and the noise head, Wrho == NULL; base.gen_grads its gradients (dx is set by
+ *      the step).  g_mask_h / _a / _b: [bags * num_clusters, h], g_mask_mlp0 as in AdvmilStepArgs.  K9 runs as the
+ *      single tcgen05 pass in ADVMIL_TF32 / _TF32X3 / _BF16 wherever that pass covers the shape; elsewhere (ADVMIL_FP32,
+ *      and fp32 features with fewer than 128 rows) the step composes advmil_linear_fwd and advmil_segment_mean_by_id_fwd,
+ *      reported under the ADVMIL_PROF_PROJ tag instead of the K9 tag.  Every bag length a
+ *      multiple of 16, 1 <= num_clusters <= 16, noise0 == 0, ksize-1 discriminator: else ADVMIL_ERR_INVALID. */
+typedef struct AdvmilClusterStepArgs {
+  AdvmilStepArgs base;
+  const float *Wphi, *bphi;            /* backbone.phis.0 [h, C(,1,1)], [h] */
+  float *dWphi, *dbphi;                /* their gradients (written) */
+  const int32_t* cid;                  /* [rows] cluster id of every row */
+  int32_t num_clusters;
+} AdvmilClusterStepArgs;
+ADVMIL_API size_t advmil_adv_step_cluster_workspace_bytes(const AdvmilGenParams* gen, const AdvmilDiscParams* disc, int32_t rows,
+                                                          int32_t bags, int32_t num_clusters, int32_t precision);
+ADVMIL_API int advmil_adv_step_cluster_disc(const AdvmilClusterStepArgs* a, void* stream);
+ADVMIL_API int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* a, void* stream);
 
 /* ---- ESAT backbone: DualTrans_HS (model/backbone.py:171-196) as load_backbone('patch', dims) builds it (:31-35):
  *      AVGPoolPatchEmbedding(C -> d, scale 4, ksize 1; model/backbone_utils.py:129-168) -> optional sincos positional
