@@ -90,25 +90,122 @@ static int side_get(SideState** out) {
   type* var = ws.take<type>(count);                                                                         \
   if (!var) { set_error("%s: workspace too small (have %zu bytes)", __func__, ws.cap); return ADVMIL_ERR_WORKSPACE; }
 
+// ---- the RLIP discriminator's part of the two phases, shared by the ABMIL, ESAT and DeepAttMISL steps ----------------
+// Scratch bytes of the D phase from the region embedding on, and of the G phase's D(x, pred_g) with the caller's d_pred.
+// `who` names the public entry point in error messages.
+static size_t disc_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb, int precision) {
+  const size_t es = elem_bytes(elem_of_precision(precision)), R = rows / 16;
+  return align_up(2 * R * d->d * sizeof(float), 256) + align_up(rows * d->d * es, 256) + head_bytes(*d, 2 * R, 2 * nb) +
+         align_up(2 * R * d->d * sizeof(float), 256) + 8 * 256 + 6 * nb * sizeof(float) + align_up((2 * nb + 2) * sizeof(int32_t), 256) +
+         advmil_disc_workspace_bytes(d, 2 * rows, 2 * nb, 1) + 256;
+}
+static size_t gen_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb) {
+  const size_t R = rows / 16;
+  return align_up(R * d->d * sizeof(float), 256) + head_bytes(*d, R, nb) + 8 * 256 + 4 * nb * sizeof(float) +
+         advmil_disc_workspace_bytes(d, rows, nb, 1) + 256;
+}
+// D phase, region embedding: ea.emb has room for the [2R, d] copy that disc_rlip duplicates for the batched head.  With
+// run == false the caller writes ea.emb / ea.y_pre itself (the ABMIL step: fused with its projection, or after its forward).
+static int disc_embed(const AdvmilStepArgs* a, Workspace& ws, bool run, AdvmilEmbedActs& ea, const char* who, cudaStream_t st) {
+  const size_t rows = a->bags->rows, d = a->disc->d;
+  ea = AdvmilEmbedActs{};
+  ea.emb = ws.take<float>(2 * (rows / 16) * d);
+  ea.y_pre = ws.take<char>(rows * d * elem_bytes(elem_of_precision(a->precision)));
+  ea.precision = a->precision;
+  if (!ea.emb || !ea.y_pre) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  return run ? advmil_disc_embed_fwd(a->disc, a->bags, &ea, (void*)st) : ADVMIL_OK;
+}
+// D phase after pred_d and the region embedding exist: batched head over [fake | real] pairs, D loss, D backward
+static int disc_rlip(const AdvmilStepArgs* a, Workspace& ws, AdvmilEmbedActs& ea, const char* who, cudaStream_t st) {
+  const AdvmilDiscParams& dp = *a->disc;
+  const AdvmilBags* bags = a->bags;
+  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  const bool batched = a->n_real > 0.f;                 // no real pair anywhere: only the fake half runs
+  AdvmilHeadActs ha{};
+  const bool head_ok = take_head(ws, dp, 2 * (size_t)R, 2 * (size_t)nb, ha);
+  float* d_emb2 = ws.take<float>((size_t)2 * R * d);
+  float* t2 = ws.take<float>(2 * nb);
+  float* d_out2 = ws.take<float>(2 * nb);
+  int32_t* offs2 = ws.take<int32_t>(2 * nb + 2);
+  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, 2 * rows, 2 * nb, 1);
+  char* dws = ws.take<char>(dws_bytes);
+  if (!head_ok || !d_emb2 || !t2 || !d_out2 || !offs2 || !dws) {
+    set_error("%s: workspace too small (have %zu bytes)", who, ws.cap);
+    return ADVMIL_ERR_WORKSPACE;
+  }
+  float* emb2 = ea.emb;
+  std::vector<int32_t> offs2_host(2 * nb + 1);
+  for (int i = 0; i <= nb; ++i) { offs2_host[i] = bags->offsets_host[i]; offs2_host[nb + i] = bags->offsets_host[i] + rows; }
+  launch_k(dup_offsets_kernel, dim3(cdiv(nb + 1, 128)), dim3(128), 0, st, bags->offsets, nb, rows, offs2);
+  ADVMIL_CHECK_LAUNCH();
+  launch_k(real_mask_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, a->e, a->visible, nb, a->real_mask);
+  ADVMIL_CHECK_LAUNCH();
+  ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2, a->pred_d, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  if (batched) {
+    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2 + nb, a->t, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(emb2 + (size_t)R * d, emb2, (size_t)R * d * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
+  AdvmilBags vb = *bags;
+  vb.offsets = offs2; vb.offsets_host = offs2_host.data(); vb.rows = batched ? 2 * rows : rows; vb.bags = batched ? 2 * nb : nb;
+  ha.emb = emb2; ha.t = t2; ha.out = a->f_fake_d;
+  ha.mask_fc1 = a->d_mask_fc1; ha.mask_ga = a->d_mask_ga; ha.mask_gs = a->d_mask_gs; ha.mask_fc2 = a->d_mask_fc2;
+  ha.seed = a->seed_d; ha.train = 1; ha.precision = a->precision; ha.workspace = dws; ha.workspace_bytes = dws_bytes;
+  ADVMIL_TRY(advmil_disc_head_fwd(&dp, &vb, &ha, (void*)st));
+  // ---- loss (loss/utils.py:182-203) and backward ----
+  ADVMIL_TRY(advmil_disc_loss(a->f_fake_d + nb, a->f_fake_d, a->real_mask, nb, a->loss_d, a->n_real, a->n_fake, a->losses,
+                              d_out2 + nb, d_out2, (void*)st));
+  ADVMIL_TRY(advmil_disc_head_bwd(&dp, &vb, &ha, d_out2, d_emb2, nullptr, a->disc_grads, 0, (void*)st));
+  ea.workspace = dws; ea.workspace_bytes = dws_bytes;
+  return disc_embed_bwd_impl(&dp, bags, &ea, d_emb2, batched ? d_emb2 + (size_t)R * d : nullptr, a->disc_grads, 0, st);
+}
+// G phase after pred_g exists: D(x, pred_g) with the updated discriminator in eval mode, G loss, and dL/dpred_g (recon +
+// the adversarial term through D) into d_pred [bags]
+static int gen_rlip(const AdvmilStepArgs* a, Workspace& ws, float* d_pred, const char* who, cudaStream_t st) {
+  const AdvmilDiscParams& dp = *a->disc;
+  const AdvmilBags* bags = a->bags;
+  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  float* emb = ws.take<float>((size_t)R * d);
+  AdvmilHeadActs ha{};
+  const bool head_ok = take_head(ws, dp, R, nb, ha);
+  float* d_fake = ws.take<float>(nb);
+  float* d_t = ws.take<float>(nb);
+  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, rows, nb, 1);
+  char* dws = ws.take<char>(dws_bytes);
+  if (!emb || !head_ok || !d_fake || !d_t || !dws) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  AdvmilEmbedActs ea{};
+  ea.emb = emb; ea.y_pre = nullptr; ea.precision = a->precision;
+  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
+  ha.ab = nullptr;      // the G step asks D only for dL/dt: the gate activations are never read back
+  ha.emb = emb; ha.t = a->pred_g; ha.out = a->f_fake_g; ha.seed = 0; ha.train = 0; ha.precision = a->precision;
+  ha.workspace = dws; ha.workspace_bytes = dws_bytes;
+  ADVMIL_TRY(advmil_disc_head_fwd(&dp, bags, &ha, (void*)st));
+  // ---- loss (loss/utils.py:21-41,205-208) and backward: D hands back only dL/dt ----
+  ADVMIL_TRY(advmil_gen_loss(a->pred_g, a->t, a->e, a->visible, a->f_fake_g, nb, a->n_visible, a->n_fake, a->coef_gan,
+                             a->recon_alpha, a->recon_gamma, a->recon_norm, a->losses + 1, d_pred, d_fake, (void*)st));
+  ADVMIL_TRY(advmil_disc_head_bwd(&dp, bags, &ha, d_fake, nullptr, d_t, nullptr, 0, (void*)st));
+  launch_k(add_inplace_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, d_pred, d_t, nb);
+  ADVMIL_CHECK_LAUNCH();
+  return ADVMIL_OK;
+}
+
 }  // namespace advmil
 
 using namespace advmil;
 
-// persistent region (same layout in both calls): eval projection, virtual-bag offsets, and everything the G step's train
-// forward writes (it may run on the side stream while the D phase uses the scratch region)
+// persistent region (same layout in both calls): eval projection and everything the G step's train forward writes (it may
+// run on the side stream while the D phase uses the scratch region)
 struct Persist {
-  char* h_eval; int32_t* offs2; char* h; char* ab; GenBufs gb; char* gws; size_t gws_bytes;
+  char* h_eval; char* h; char* ab; GenBufs gb; char* gws; size_t gws_bytes;
 };
 static int take_persist(Workspace& ws, const AdvmilGenParams& gp, int rows, int nb, size_t es, Persist& P) {
   const size_t abw = gate_width(gp.h);
   P.h_eval = ws.take<char>((size_t)rows * gp.h * es);
-  P.offs2 = ws.take<int32_t>(2 * nb + 2);
   P.h = ws.take<char>((size_t)rows * gp.h * es);
   P.ab = ws.take<char>((size_t)rows * abw * es);
   const bool ok = take_gen(ws, gp, rows, nb, P.gb);
   P.gws_bytes = advmil_generator_workspace_bytes(&gp, rows, nb, 1);
   P.gws = ws.take<char>(P.gws_bytes);
-  if (!P.h_eval || !P.offs2 || !P.h || !P.ab || !ok || !P.gws) { set_error("adv_step: workspace too small (have %zu bytes)", ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  if (!P.h_eval || !P.h || !P.ab || !ok || !P.gws) { set_error("adv_step: workspace too small (have %zu bytes)", ws.cap); return ADVMIL_ERR_WORKSPACE; }
   return ADVMIL_OK;
 }
 static void fill_train_acts(const AdvmilStepArgs* a, const Persist& P, AdvmilGenActs& ga) {
@@ -123,16 +220,11 @@ static void fill_train_acts(const AdvmilStepArgs* a, const Persist& P, AdvmilGen
 extern "C" size_t advmil_adv_step_workspace_bytes(const AdvmilGenParams* g, const AdvmilDiscParams* d, int32_t rows,
                                                   int32_t bags, int32_t precision) {
   const size_t es = elem_bytes(elem_of_precision(precision));
-  const size_t R = rows / 16, nb = bags, abw = gate_width(g->h);
-  size_t persistent = 2 * align_up((size_t)rows * g->h * es, 256) + align_up((2 * nb + 2) * sizeof(int32_t), 256) +
-                      align_up((size_t)rows * abw * es, 256) + gen_bufs_bytes(*g, rows, nb) +
+  const size_t nb = bags, abw = gate_width(g->h);
+  size_t persistent = 2 * align_up((size_t)rows * g->h * es, 256) + align_up((size_t)rows * abw * es, 256) + gen_bufs_bytes(*g, rows, nb) +
                       advmil_generator_workspace_bytes(g, rows, bags, 1) + 2048;
-  size_t disc = gen_bufs_bytes(*g, rows, nb) + advmil_generator_workspace_bytes(g, rows, bags, 0) + 256 +
-                align_up(2 * R * d->d * sizeof(float), 256) + align_up((size_t)rows * d->d * es, 256) + head_bytes(*d, 2 * R, 2 * nb) +
-                align_up(2 * R * d->d * sizeof(float), 256) + 8 * 256 + 6 * nb * sizeof(float) +
-                advmil_disc_workspace_bytes(d, 2 * rows, 2 * bags, 1) + 256;
-  size_t gen = align_up(R * d->d * sizeof(float), 256) + head_bytes(*d, R, nb) + 8 * 256 + 4 * nb * sizeof(float) +
-               advmil_disc_workspace_bytes(d, rows, bags, 1) + 256;
+  size_t disc = gen_bufs_bytes(*g, rows, nb) + advmil_generator_workspace_bytes(g, rows, bags, 0) + 256 + disc_part_bytes(d, rows, nb, precision);
+  size_t gen = gen_part_bytes(d, rows, nb);
   return persistent + (disc > gen ? disc : gen) + 4096;
 }
 
@@ -151,15 +243,12 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   const AdvmilGenParams& gp = *a->gen;
   const AdvmilDiscParams& dp = *a->disc;
   const AdvmilBags* bags = a->bags;
-  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  const int rows = bags->rows, nb = bags->bags, d = dp.d;
   const size_t es = elem_bytes(elem_of_precision(a->precision));
-  const bool batched = a->n_real > 0.f;                 // no real pair anywhere: only the fake half runs
-  const int nbv = batched ? 2 * nb : nb, Rv = batched ? 2 * R : R;
   Workspace ws(a->workspace, a->workspace_bytes);
   Persist P;
   ADVMIL_TRY(take_persist(ws, gp, rows, nb, es, P));
   char* h_eval = P.h_eval;
-  int32_t* offs2 = P.offs2;
   std::lock_guard<std::mutex> side_lock(g_side_mu);
   SideState* side = nullptr;
   ADVMIL_TRY(side_get(&side));
@@ -180,10 +269,8 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   ga.seed = 0; ga.train = 0; ga.precision = a->precision; ga.workspace = gws; ga.workspace_bytes = gws_bytes;
   ga.h_drop_out = P.h; ga.seed_drop = a->seed_g; ga.mask_h_drop = a->g_mask_h;   // the G step's dropped projection, same pass
   // ---- shared region embedding (K5+K6), duplicated for the batched head ----
-  STEP_TAKE(emb2, float, (size_t)2 * R * d);
-  STEP_TAKE(y_pre, char, (size_t)rows * d * es);
-  AdvmilEmbedActs ea{};
-  ea.emb = emb2; ea.y_pre = y_pre; ea.precision = a->precision;
+  AdvmilEmbedActs ea;
+  ADVMIL_TRY(disc_embed(a, ws, false, ea, __func__, st));
   const bool fused = gp.C == dp.C && (dp.ksize == 0 || dp.ksize == 1) && proj_embed_supported(rows, gp.C, gp.h, d, a->precision);
   if (fused) {     // K1 and K5+K6 read the same x: one pass over stacked weights, then the generator forward skips K1
     for (int i = 0; i < nb; ++i)
@@ -192,7 +279,7 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
     Drop d2 = Drop::make(a->g_mask_h, a->seed_g, SITE_H, gp.p_backbone, 1, gp.h);
     { ProfScope ps(PROF_PROJ_EMBED, st);
       ADVMIL_TRY(proj_embed_fwd(bags->x, gp.W1, gp.b1, dp.Wc, dp.bc, dp.ln_g, dp.ln_b, rows, gp.C, gp.h, d, dp.ln_eps, h_eval, P.h, &d2,
-                                y_pre, emb2, st)); }
+                                ea.y_pre, ea.emb, st)); }
     ga.h_ready = 1; ga.h_drop_out = nullptr;
   }
   ADVMIL_TRY(advmil_generator_fwd(&gp, bags, &ga, stream));
@@ -208,39 +295,8 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
     ADVMIL_CHECK_CUDA(cudaEventRecord(side->done[slot], side->stream));
     side->pending_ws[slot] = a->workspace;
   }
-  // ---- batched head over the virtual bags [fake pairs | real pairs] ----
-  AdvmilHeadActs ha{};
-  if (!take_head(ws, dp, 2 * (size_t)R, 2 * (size_t)nb, ha)) { set_error("adv_step_disc: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
-  STEP_TAKE(d_emb2, float, (size_t)2 * R * d);
-  STEP_TAKE(t2, float, 2 * nb);
-  STEP_TAKE(d_out2, float, 2 * nb);
-  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, 2 * rows, 2 * nb, 1);
-  STEP_TAKE(dws, char, dws_bytes);
-  std::vector<int32_t> offs2_host(2 * nb + 1);
-  for (int i = 0; i <= nb; ++i) { offs2_host[i] = bags->offsets_host[i]; offs2_host[nb + i] = bags->offsets_host[i] + rows; }
-  launch_k(dup_offsets_kernel, dim3(cdiv(nb + 1, 128)), dim3(128), 0, st, bags->offsets, nb, rows, offs2);
-  ADVMIL_CHECK_LAUNCH();
-  launch_k(real_mask_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, a->e, a->visible, nb, a->real_mask);
-  ADVMIL_CHECK_LAUNCH();
-  ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2, a->pred_d, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  if (batched) {
-    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2 + nb, a->t, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(emb2 + (size_t)R * d, emb2, (size_t)R * d * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  }
-  AdvmilBags vb = *bags;
-  vb.offsets = offs2; vb.offsets_host = offs2_host.data(); vb.rows = batched ? 2 * rows : rows; vb.bags = nbv;
-  ha.emb = emb2; ha.t = t2; ha.out = a->f_fake_d;
-  ha.mask_fc1 = a->d_mask_fc1; ha.mask_ga = a->d_mask_ga; ha.mask_gs = a->d_mask_gs; ha.mask_fc2 = a->d_mask_fc2;
-  ha.seed = a->seed_d; ha.train = 1; ha.precision = a->precision; ha.workspace = dws; ha.workspace_bytes = dws_bytes;
-  ADVMIL_TRY(advmil_disc_head_fwd(&dp, &vb, &ha, stream));
-  // ---- loss (loss/utils.py:182-203) and backward ----
-  ADVMIL_TRY(advmil_disc_loss(a->f_fake_d + nb, a->f_fake_d, a->real_mask, nb, a->loss_d, a->n_real, a->n_fake, a->losses,
-                              d_out2 + nb, d_out2, stream));
-  ADVMIL_TRY(advmil_disc_head_bwd(&dp, &vb, &ha, d_out2, d_emb2, nullptr, a->disc_grads, 0, stream));
-  ea.workspace = dws; ea.workspace_bytes = dws_bytes;
-  ADVMIL_TRY(disc_embed_bwd_impl(&dp, bags, &ea, d_emb2, batched ? d_emb2 + (size_t)R * d : nullptr, a->disc_grads, 0, st));
-  (void)Rv;
-  return ADVMIL_OK;
+  // ---- batched head over the virtual bags [fake pairs | real pairs], loss and backward ----
+  return disc_rlip(a, ws, ea, __func__, st);
 }
 
 extern "C" int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream) {
@@ -248,9 +304,8 @@ extern "C" int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream) {
   ADVMIL_REQUIRE(a->gen_grads && a->pred_g && a->f_fake_g, "adv_step_gen: missing output buffers");
   cudaStream_t st = (cudaStream_t)stream;
   const AdvmilGenParams& gp = *a->gen;
-  const AdvmilDiscParams& dp = *a->disc;
   const AdvmilBags* bags = a->bags;
-  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  const int rows = bags->rows, nb = bags->bags;
   const size_t es = elem_bytes(elem_of_precision(a->precision));
   Workspace ws(a->workspace, a->workspace_bytes);
   Persist P;                                                  // h_eval was written by advmil_adv_step_disc on this workspace
@@ -270,28 +325,9 @@ extern "C" int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream) {
     side_lock.unlock();
     ADVMIL_TRY(advmil_generator_fwd(&gp, bags, &ga, stream));
   }
-  // ---- D(x, pred_g) with the updated discriminator, eval mode ----
-  STEP_TAKE(emb, float, (size_t)R * d);
-  AdvmilEmbedActs ea{};
-  ea.emb = emb; ea.y_pre = nullptr; ea.precision = a->precision;
-  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, stream));
-  AdvmilHeadActs ha{};
-  if (!take_head(ws, dp, R, nb, ha)) { set_error("adv_step_gen: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
+  // ---- D(x, pred_g) with the updated discriminator, G loss, dL/dpred_g ----
   STEP_TAKE(d_pred, float, nb);
-  STEP_TAKE(d_fake, float, nb);
-  STEP_TAKE(d_t, float, nb);
-  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, rows, nb, 1);
-  STEP_TAKE(dws, char, dws_bytes);
-  ha.ab = nullptr;      // the G step asks D only for dL/dt: the gate activations are never read back
-  ha.emb = emb; ha.t = a->pred_g; ha.out = a->f_fake_g; ha.seed = 0; ha.train = 0; ha.precision = a->precision;
-  ha.workspace = dws; ha.workspace_bytes = dws_bytes;
-  ADVMIL_TRY(advmil_disc_head_fwd(&dp, bags, &ha, stream));
-  // ---- loss (loss/utils.py:21-41,205-208) and backward: D hands back only dL/dt ----
-  ADVMIL_TRY(advmil_gen_loss(a->pred_g, a->t, a->e, a->visible, a->f_fake_g, nb, a->n_visible, a->n_fake, a->coef_gan,
-                             a->recon_alpha, a->recon_gamma, a->recon_norm, a->losses + 1, d_pred, d_fake, stream));
-  ADVMIL_TRY(advmil_disc_head_bwd(&dp, bags, &ha, d_fake, nullptr, d_t, nullptr, 0, stream));
-  launch_k(add_inplace_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, d_pred, d_t, nb);
-  ADVMIL_CHECK_LAUNCH();
+  ADVMIL_TRY(gen_rlip(a, ws, d_pred, __func__, st));
   return advmil_generator_bwd(&gp, bags, &ga, d_pred, a->gen_grads, stream);
 }
 
@@ -308,7 +344,6 @@ namespace advmil {
 struct EsatBufs {
   char* y_pre; float *emb, *qkv, *lse, *ctx, *s1, *x1, *f, *s2, *x2, *ab, *rep, *attn, *H, *H1, *pre;
   char* ews; size_t ews_bytes;
-  int32_t* offs2;
 };
 static size_t esat_acts_bytes(const AdvmilEsatParams& p, const AdvmilGenParams& h, size_t rows, size_t nb, size_t es) {
   const size_t R = rows / 16, d = p.d, abw = gate_width(p.d);
@@ -324,9 +359,8 @@ static int take_esat(Workspace& ws, const AdvmilEsatParams& p, const AdvmilGenPa
   const size_t e0 = advmil_esat_workspace_bytes(&p, &h, rows, nb, 0), e1 = advmil_esat_workspace_bytes(&p, &h, rows, nb, 1);
   b.ews_bytes = e0 > e1 ? e0 : e1;
   b.ews = ws.take<char>(b.ews_bytes);
-  b.offs2 = ws.take<int32_t>(2 * nb + 2);
   if (!b.y_pre || !b.emb || !b.qkv || !b.lse || !b.ctx || !b.s1 || !b.x1 || !b.f || !b.s2 || !b.x2 || !b.ab || !b.rep || !b.attn || !b.H ||
-      !b.H1 || !b.pre || !b.ews || !b.offs2) {
+      !b.H1 || !b.pre || !b.ews) {
     set_error("adv_step_esat: workspace too small (have %zu bytes)", ws.cap);
     return ADVMIL_ERR_WORKSPACE;
   }
@@ -348,19 +382,26 @@ static int esat_step_check(const AdvmilEsatStepArgs* a) {
   ADVMIL_REQUIRE(a->head->W0 && a->head->noise0 == 0, "adv_step_esat: needs the noise head with gen_noi_noise '0-1'");
   return ADVMIL_OK;
 }
+// the fields disc_rlip / gen_rlip read, as an AdvmilStepArgs view of the ESAT step's arguments (no injected D masks)
+static AdvmilStepArgs rlip_args(const AdvmilEsatStepArgs* a) {
+  AdvmilStepArgs v{};
+  v.disc = a->disc; v.disc_grads = a->disc_grads; v.bags = a->bags; v.t = a->t; v.e = a->e; v.visible = a->visible;
+  v.seed_d = a->seed_d; v.n_real = a->n_real; v.n_fake = a->n_fake; v.n_visible = a->n_visible;
+  v.loss_d = a->loss_d; v.coef_gan = a->coef_gan; v.recon_alpha = a->recon_alpha; v.recon_gamma = a->recon_gamma;
+  v.recon_norm = a->recon_norm; v.precision = a->precision;
+  v.losses = a->losses; v.pred_d = a->pred_d; v.f_fake_d = a->f_fake_d; v.real_mask = a->real_mask;
+  v.pred_g = a->pred_g; v.f_fake_g = a->f_fake_g;
+  return v;
+}
 }  // namespace advmil
 
 extern "C" size_t advmil_adv_step_esat_workspace_bytes(const AdvmilEsatParams* g, const AdvmilGenParams* head, const AdvmilDiscParams* d,
                                                        int32_t rows, int32_t bags, int32_t precision) {
   const size_t es = elem_bytes(elem_of_precision(precision));
-  const size_t R = rows / 16, nb = bags;
+  const size_t nb = bags;
   const size_t e0 = advmil_esat_workspace_bytes(g, head, rows, bags, 0), e1 = advmil_esat_workspace_bytes(g, head, rows, bags, 1);
-  size_t persistent = esat_acts_bytes(*g, *head, rows, nb, es) + (e0 > e1 ? e0 : e1) + 256 + align_up((2 * nb + 2) * sizeof(int32_t), 256);
-  size_t disc = align_up(2 * R * d->d * sizeof(float), 256) + align_up((size_t)rows * d->d * es, 256) + head_bytes(*d, 2 * R, 2 * nb) +
-                align_up(2 * R * d->d * sizeof(float), 256) + 8 * 256 + 6 * nb * sizeof(float) +
-                advmil_disc_workspace_bytes(d, 2 * rows, 2 * bags, 1) + 256;
-  size_t gen = align_up(R * d->d * sizeof(float), 256) + head_bytes(*d, R, nb) + 8 * 256 + 4 * nb * sizeof(float) +
-               advmil_disc_workspace_bytes(d, rows, bags, 1) + 256;
+  size_t persistent = esat_acts_bytes(*g, *head, rows, nb, es) + (e0 > e1 ? e0 : e1) + 256;
+  size_t disc = disc_part_bytes(d, rows, nb, precision), gen = gen_part_bytes(d, rows, nb);
   return persistent + (disc > gen ? disc : gen) + 4096;
 }
 
@@ -368,12 +409,9 @@ extern "C" int advmil_adv_step_esat_disc(const AdvmilEsatStepArgs* a, void* stre
   ADVMIL_TRY(esat_step_check(a));
   ADVMIL_REQUIRE(a->disc_grads && a->pred_d && a->f_fake_d && a->real_mask, "adv_step_esat_disc: missing output buffers");
   cudaStream_t st = (cudaStream_t)stream;
-  const AdvmilDiscParams& dp = *a->disc;
   const AdvmilBags* bags = a->bags;
-  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  const int rows = bags->rows, nb = bags->bags;
   const size_t es = elem_bytes(elem_of_precision(a->precision));
-  const bool batched = a->n_real > 0.f;
-  const int nbv = batched ? 2 * nb : nb;
   Workspace ws(a->workspace, a->workspace_bytes);
   EsatBufs B;
   ADVMIL_TRY(take_esat(ws, *a->esat, *a->head, rows, nb, es, B));
@@ -381,49 +419,19 @@ extern "C" int advmil_adv_step_esat_disc(const AdvmilEsatStepArgs* a, void* stre
   AdvmilEsatActs ea;
   fill_esat_acts(a, B, 0, ea);
   ADVMIL_TRY(advmil_esat_fwd(a->esat, a->head, bags, &ea, stream));
-  // ---- shared region embedding, duplicated for the batched head ----
-  STEP_TAKE(emb2, float, (size_t)2 * R * d);
-  STEP_TAKE(y_pre, char, (size_t)rows * d * es);
-  AdvmilEmbedActs da{};
-  da.emb = emb2; da.y_pre = y_pre; da.precision = a->precision;
-  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &da, stream));
-  AdvmilHeadActs ha{};
-  if (!take_head(ws, dp, 2 * (size_t)R, 2 * (size_t)nb, ha)) { set_error("adv_step_esat_disc: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
-  STEP_TAKE(d_emb2, float, (size_t)2 * R * d);
-  STEP_TAKE(t2, float, 2 * nb);
-  STEP_TAKE(d_out2, float, 2 * nb);
-  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, 2 * rows, 2 * nb, 1);
-  STEP_TAKE(dws, char, dws_bytes);
-  std::vector<int32_t> offs2_host(2 * nb + 1);
-  for (int i = 0; i <= nb; ++i) { offs2_host[i] = bags->offsets_host[i]; offs2_host[nb + i] = bags->offsets_host[i] + rows; }
-  launch_k(dup_offsets_kernel, dim3(cdiv(nb + 1, 128)), dim3(128), 0, st, bags->offsets, nb, rows, B.offs2);
-  ADVMIL_CHECK_LAUNCH();
-  launch_k(real_mask_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, a->e, a->visible, nb, a->real_mask);
-  ADVMIL_CHECK_LAUNCH();
-  ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2, a->pred_d, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  if (batched) {
-    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2 + nb, a->t, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(emb2 + (size_t)R * d, emb2, (size_t)R * d * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  }
-  AdvmilBags vb = *bags;
-  vb.offsets = B.offs2; vb.offsets_host = offs2_host.data(); vb.rows = batched ? 2 * rows : rows; vb.bags = nbv;
-  ha.emb = emb2; ha.t = t2; ha.out = a->f_fake_d;
-  ha.seed = a->seed_d; ha.train = 1; ha.precision = a->precision; ha.workspace = dws; ha.workspace_bytes = dws_bytes;
-  ADVMIL_TRY(advmil_disc_head_fwd(&dp, &vb, &ha, stream));
-  ADVMIL_TRY(advmil_disc_loss(a->f_fake_d + nb, a->f_fake_d, a->real_mask, nb, a->loss_d, a->n_real, a->n_fake, a->losses,
-                              d_out2 + nb, d_out2, stream));
-  ADVMIL_TRY(advmil_disc_head_bwd(&dp, &vb, &ha, d_out2, d_emb2, nullptr, a->disc_grads, 0, stream));
-  da.workspace = dws; da.workspace_bytes = dws_bytes;
-  return disc_embed_bwd_impl(&dp, bags, &da, d_emb2, batched ? d_emb2 + (size_t)R * d : nullptr, a->disc_grads, 0, st);
+  // ---- shared region embedding, batched head over [fake | real] pairs, D loss and backward ----
+  const AdvmilStepArgs v = rlip_args(a);
+  AdvmilEmbedActs da;
+  ADVMIL_TRY(disc_embed(&v, ws, true, da, __func__, st));
+  return disc_rlip(&v, ws, da, __func__, st);
 }
 
 extern "C" int advmil_adv_step_esat_gen(const AdvmilEsatStepArgs* a, void* stream) {
   ADVMIL_TRY(esat_step_check(a));
   ADVMIL_REQUIRE(a->esat_grads && a->head_grads && a->pred_g && a->f_fake_g, "adv_step_esat_gen: missing output buffers");
   cudaStream_t st = (cudaStream_t)stream;
-  const AdvmilDiscParams& dp = *a->disc;
   const AdvmilBags* bags = a->bags;
-  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
+  const int rows = bags->rows, nb = bags->bags;
   const size_t es = elem_bytes(elem_of_precision(a->precision));
   Workspace ws(a->workspace, a->workspace_bytes);
   EsatBufs B;                                      // y_pre / emb were written by advmil_adv_step_esat_disc on this workspace
@@ -432,27 +440,10 @@ extern "C" int advmil_adv_step_esat_gen(const AdvmilEsatStepArgs* a, void* strea
   AdvmilEsatActs ea;
   fill_esat_acts(a, B, 1, ea);
   ADVMIL_TRY(advmil_esat_fwd(a->esat, a->head, bags, &ea, stream));
-  // ---- D(x, pred_g) with the updated discriminator, eval mode ----
-  STEP_TAKE(emb, float, (size_t)R * d);
-  AdvmilEmbedActs da{};
-  da.emb = emb; da.y_pre = nullptr; da.precision = a->precision;
-  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &da, stream));
-  AdvmilHeadActs ha{};
-  if (!take_head(ws, dp, R, nb, ha)) { set_error("adv_step_esat_gen: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
+  // ---- D(x, pred_g) with the updated discriminator, G loss, dL/dpred_g ----
   STEP_TAKE(d_pred, float, nb);
-  STEP_TAKE(d_fake, float, nb);
-  STEP_TAKE(d_t, float, nb);
-  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, rows, nb, 1);
-  STEP_TAKE(dws, char, dws_bytes);
-  ha.ab = nullptr;
-  ha.emb = emb; ha.t = a->pred_g; ha.out = a->f_fake_g; ha.seed = 0; ha.train = 0; ha.precision = a->precision;
-  ha.workspace = dws; ha.workspace_bytes = dws_bytes;
-  ADVMIL_TRY(advmil_disc_head_fwd(&dp, bags, &ha, stream));
-  ADVMIL_TRY(advmil_gen_loss(a->pred_g, a->t, a->e, a->visible, a->f_fake_g, nb, a->n_visible, a->n_fake, a->coef_gan,
-                             a->recon_alpha, a->recon_gamma, a->recon_norm, a->losses + 1, d_pred, d_fake, stream));
-  ADVMIL_TRY(advmil_disc_head_bwd(&dp, bags, &ha, d_fake, nullptr, d_t, nullptr, 0, stream));
-  launch_k(add_inplace_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, d_pred, d_t, nb);
-  ADVMIL_CHECK_LAUNCH();
+  const AdvmilStepArgs v = rlip_args(a);
+  ADVMIL_TRY(gen_rlip(&v, ws, d_pred, __func__, st));
   esat_request_overlap(1);     // weight / bias gradients of the region-level layers on the backward side stream
   const int rc = advmil_esat_bwd(a->esat, a->head, bags, &ea, d_pred, a->esat_grads, a->head_grads, stream);
   esat_request_overlap(0);
@@ -524,86 +515,6 @@ static int cluster_step_check(const AdvmilClusterStepArgs* ca) {
                    "bags: bag %d has a length that is not a multiple of 16 (model/backbone_utils.py:65)", i);
   return ADVMIL_OK;
 }
-static size_t disc_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb, int precision) {
-  const size_t es = elem_bytes(elem_of_precision(precision)), R = rows / 16;
-  return align_up(2 * R * d->d * sizeof(float), 256) + align_up(rows * d->d * es, 256) + head_bytes(*d, 2 * R, 2 * nb) +
-         align_up(2 * R * d->d * sizeof(float), 256) + 8 * 256 + 6 * nb * sizeof(float) + align_up((2 * nb + 2) * sizeof(int32_t), 256) +
-         advmil_disc_workspace_bytes(d, 2 * rows, 2 * nb, 1) + 256;
-}
-static size_t gen_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb) {
-  const size_t R = rows / 16;
-  return align_up(R * d->d * sizeof(float), 256) + head_bytes(*d, R, nb) + 8 * 256 + 4 * nb * sizeof(float) +
-         advmil_disc_workspace_bytes(d, rows, nb, 1) + 256;
-}
-// D phase after pred_d exists: shared region embedding, batched head over [fake | real] pairs, D loss, D backward
-static int disc_rlip(const AdvmilStepArgs* a, Workspace& ws, cudaStream_t st) {
-  const AdvmilDiscParams& dp = *a->disc;
-  const AdvmilBags* bags = a->bags;
-  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
-  const size_t es = elem_bytes(elem_of_precision(a->precision));
-  const bool batched = a->n_real > 0.f;                 // no real pair anywhere: only the fake half runs
-  STEP_TAKE(emb2, float, (size_t)2 * R * d);
-  STEP_TAKE(y_pre, char, (size_t)rows * d * es);
-  AdvmilEmbedActs ea{};
-  ea.emb = emb2; ea.y_pre = y_pre; ea.precision = a->precision;
-  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
-  AdvmilHeadActs ha{};
-  if (!take_head(ws, dp, 2 * (size_t)R, 2 * (size_t)nb, ha)) { set_error("adv_step_cluster_disc: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
-  STEP_TAKE(d_emb2, float, (size_t)2 * R * d);
-  STEP_TAKE(t2, float, 2 * nb);
-  STEP_TAKE(d_out2, float, 2 * nb);
-  STEP_TAKE(offs2, int32_t, 2 * nb + 2);
-  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, 2 * rows, 2 * nb, 1);
-  STEP_TAKE(dws, char, dws_bytes);
-  std::vector<int32_t> offs2_host(2 * nb + 1);
-  for (int i = 0; i <= nb; ++i) { offs2_host[i] = bags->offsets_host[i]; offs2_host[nb + i] = bags->offsets_host[i] + rows; }
-  launch_k(dup_offsets_kernel, dim3(cdiv(nb + 1, 128)), dim3(128), 0, st, bags->offsets, nb, rows, offs2);
-  ADVMIL_CHECK_LAUNCH();
-  launch_k(real_mask_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, a->e, a->visible, nb, a->real_mask);
-  ADVMIL_CHECK_LAUNCH();
-  ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2, a->pred_d, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  if (batched) {
-    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(t2 + nb, a->t, nb * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    ADVMIL_CHECK_CUDA(cudaMemcpyAsync(emb2 + (size_t)R * d, emb2, (size_t)R * d * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  }
-  AdvmilBags vb = *bags;
-  vb.offsets = offs2; vb.offsets_host = offs2_host.data(); vb.rows = batched ? 2 * rows : rows; vb.bags = batched ? 2 * nb : nb;
-  ha.emb = emb2; ha.t = t2; ha.out = a->f_fake_d;
-  ha.mask_fc1 = a->d_mask_fc1; ha.mask_ga = a->d_mask_ga; ha.mask_gs = a->d_mask_gs; ha.mask_fc2 = a->d_mask_fc2;
-  ha.seed = a->seed_d; ha.train = 1; ha.precision = a->precision; ha.workspace = dws; ha.workspace_bytes = dws_bytes;
-  ADVMIL_TRY(advmil_disc_head_fwd(&dp, &vb, &ha, (void*)st));
-  ADVMIL_TRY(advmil_disc_loss(a->f_fake_d + nb, a->f_fake_d, a->real_mask, nb, a->loss_d, a->n_real, a->n_fake, a->losses,
-                              d_out2 + nb, d_out2, (void*)st));
-  ADVMIL_TRY(advmil_disc_head_bwd(&dp, &vb, &ha, d_out2, d_emb2, nullptr, a->disc_grads, 0, (void*)st));
-  ea.workspace = dws; ea.workspace_bytes = dws_bytes;
-  return disc_embed_bwd_impl(&dp, bags, &ea, d_emb2, batched ? d_emb2 + (size_t)R * d : nullptr, a->disc_grads, 0, st);
-}
-// G phase after pred_g exists: D(x, pred_g) in eval mode, G loss, and dL/dpred_g (recon + the adversarial term through D)
-static int gen_rlip(const AdvmilStepArgs* a, Workspace& ws, float* d_pred, cudaStream_t st) {
-  const AdvmilDiscParams& dp = *a->disc;
-  const AdvmilBags* bags = a->bags;
-  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
-  STEP_TAKE(emb, float, (size_t)R * d);
-  AdvmilEmbedActs ea{};
-  ea.emb = emb; ea.y_pre = nullptr; ea.precision = a->precision;
-  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
-  AdvmilHeadActs ha{};
-  if (!take_head(ws, dp, R, nb, ha)) { set_error("adv_step_cluster_gen: workspace too small"); return ADVMIL_ERR_WORKSPACE; }
-  STEP_TAKE(d_fake, float, nb);
-  STEP_TAKE(d_t, float, nb);
-  const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, rows, nb, 1);
-  STEP_TAKE(dws, char, dws_bytes);
-  ha.ab = nullptr;
-  ha.emb = emb; ha.t = a->pred_g; ha.out = a->f_fake_g; ha.seed = 0; ha.train = 0; ha.precision = a->precision;
-  ha.workspace = dws; ha.workspace_bytes = dws_bytes;
-  ADVMIL_TRY(advmil_disc_head_fwd(&dp, bags, &ha, (void*)st));
-  ADVMIL_TRY(advmil_gen_loss(a->pred_g, a->t, a->e, a->visible, a->f_fake_g, nb, a->n_visible, a->n_fake, a->coef_gan,
-                             a->recon_alpha, a->recon_gamma, a->recon_norm, a->losses + 1, d_pred, d_fake, (void*)st));
-  ADVMIL_TRY(advmil_disc_head_bwd(&dp, bags, &ha, d_fake, nullptr, d_t, nullptr, 0, (void*)st));
-  launch_k(add_inplace_kernel, dim3(cdiv(nb, 128)), dim3(128), 0, st, d_pred, d_t, nb);
-  ADVMIL_CHECK_LAUNCH();
-  return ADVMIL_OK;
-}
 }  // namespace advmil
 
 extern "C" size_t advmil_adv_step_cluster_workspace_bytes(const AdvmilGenParams* g, const AdvmilDiscParams* d, int32_t rows,
@@ -667,7 +578,9 @@ extern "C" int advmil_adv_step_cluster_disc(const AdvmilClusterStepArgs* ca, voi
   ga.pred = a->pred_d; ga.noise0 = nullptr; ga.noise1 = a->noise_d;
   ga.seed = 0; ga.train = 0; ga.precision = ADVMIL_FP32; ga.workspace = gws; ga.workspace_bytes = gws_bytes;
   ADVMIL_TRY(advmil_generator_fwd(&gp, &cb, &ga, stream));
-  return disc_rlip(a, ws, st);
+  AdvmilEmbedActs ea;
+  ADVMIL_TRY(disc_embed(a, ws, true, ea, __func__, st));
+  return disc_rlip(a, ws, ea, __func__, st);
 }
 
 extern "C" int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* ca, void* stream) {
@@ -699,7 +612,7 @@ extern "C" int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* ca, void
   ADVMIL_TRY(advmil_generator_fwd(&gp, &cb, &ga, stream));
   // ---- D(x, pred_g), G loss, dL/dpred_g ----
   STEP_TAKE(d_pred, float, nb);
-  ADVMIL_TRY(gen_rlip(a, ws, d_pred, st));
+  ADVMIL_TRY(gen_rlip(a, ws, d_pred, __func__, st));
   // ---- attention stage backward down to d_hc, then K9's backward and dWphi / dbphi ----
   STEP_TAKE(d_hc, float, (size_t)nbc * h);
   AdvmilGenGrads gg = *a->gen_grads;

@@ -132,6 +132,12 @@ class AdvStep(_DataParallelMixin):
         self.G = FlatParams(netG, self.gparams, weight_decay_rule=True)
         self.D = FlatParams(netD, self.dparams, weight_decay_rule=False)
         self.ggrads, self.dgrads = self.G.grads_for(self.gparams), self.D.grads_for(self.dparams)
+        self._init_hparams(lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
+                           process_group)
+
+    def _init_hparams(self, lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
+                      process_group):
+        """Optimiser, loss and precision settings of the C-fused steps; runs after self.G / self.D exist."""
         self.lr_g, self.lr_d, self.wd_g = lr_g, lr_d, weight_decay_g
         self.coef_gan, self.coef_l1 = coef_gan, coef_l1
         self.loss_d = {"bce": 0, "hinge": 1, "wasserstein": 2}[loss_d]
@@ -154,12 +160,80 @@ class AdvStep(_DataParallelMixin):
             self._c = (gp, dp, gg, dg)
         return self._c
 
-    def _workspace(self, lib, gp, dp, rows, nb, dev) -> torch.Tensor:
-        need = lib.advmil_adv_step_workspace_bytes(C.byref(gp), C.byref(dp), rows, nb, self.precision)
+    def _inputs(self, bags, t, e, visible, global_counts):
+        """The bags in this engine's precision, t / e / visible as flat device vectors, and the GLOBAL pair counts
+        (n_real, n_fake, n_visible): an all-reduce and one host sync unless the caller passes them."""
+        bags = bags.for_precision(self.precision)   # bf16 mode: bf16 features as packed by the loader, or one cast here
+        dev, nb = bags.x.device, bags.bags
+        t = t.reshape(-1).contiguous().float()
+        e = e.reshape(-1).contiguous().float()
+        visible = visible.reshape(-1).to(torch.uint8).contiguous()
+        if global_counts is None:
+            real_mask = ((e == 1) & (visible != 0))                      # model_handler.py:373-375
+            cnt = torch.stack([real_mask.sum(), torch.tensor(nb, device=dev), visible.sum()]).float()
+            self._allreduce(cnt)
+            counts = [float(v) for v in cnt.tolist()]
+        else:
+            counts = [float(v) for v in global_counts]
+        return bags, t, e, visible, counts
+
+    def _noise(self, nb, dev, noise_d, noise_g):
+        """Noise of the D phase's and of the G phase's generator pass, drawn in that order where not given."""
+        noise_d = (noise_d if noise_d is not None else self._draw(nb, dev)).contiguous().float()
+        noise_g = (noise_g if noise_g is not None else self._draw(nb, dev)).contiguous().float()
+        return noise_d, noise_g
+
+    def _workspace(self, need, dev) -> torch.Tensor:
+        """The step's workspace of at least `need` bytes: grow-only, so steady-state steps allocate nothing."""
         ws = getattr(self, "_ws", None)
         if ws is None or ws.numel() < need or ws.device != dev:
-            self._ws = ws = torch.empty(int(need * 1.05) + 4096, dtype=torch.uint8, device=dev)   # grow-only
+            self._ws = ws = torch.empty(int(need * 1.05) + 4096, dtype=torch.uint8, device=dev)
         return ws
+
+    @staticmethod
+    def _outputs(nb, dev) -> Dict:
+        f32 = dict(dtype=torch.float32, device=dev)
+        return {"losses": torch.zeros(8, **f32), "pred_d": torch.empty(nb, **f32), "pred_g": torch.empty(nb, **f32),
+                "f_d": torch.empty(2 * nb, **f32), "f_fake_g": torch.empty(nb, **f32),
+                "real_mask": torch.empty(nb, dtype=torch.uint8, device=dev)}
+
+    def _fill_args(self, a, bags, t, e, visible, noise_d, noise_g, counts, out, ws):
+        """The fields that StepArgs and EsatStepArgs share by name (the dropout seeds are drawn here: D's, then G's)."""
+        a.bags = C.pointer(bags.c())
+        a.t, a.e, a.visible = t.data_ptr(), e.data_ptr(), visible.data_ptr()
+        a.noise_d, a.noise_g = noise_d.data_ptr(), noise_g.data_ptr()
+        a.seed_d, a.seed_g = self._seed(), self._seed()
+        a.n_real, a.n_fake, a.n_visible = counts
+        a.loss_d = self.loss_d
+        a.recon_norm, a.recon_alpha, a.recon_gamma = self.recon
+        a.coef_gan, a.precision = self.coef_gan, self.precision
+        a.losses, a.pred_d, a.f_fake_d, a.real_mask = (out["losses"].data_ptr(), out["pred_d"].data_ptr(),
+                                                       out["f_d"].data_ptr(), out["real_mask"].data_ptr())
+        a.pred_g, a.f_fake_g = out["pred_g"].data_ptr(), out["f_fake_g"].data_ptr()
+        a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
+
+    def _update(self, lib, disc_fn: str, gen_fn: str, args, out, nb, n_real, keep) -> Dict:
+        """The two phases: the library's D call, D all-reduce and Adam, then its G call, L1 value, G all-reduce and Adam.
+        keep: the step's input tensors, alive until the stream is done with them."""
+        st = torch.cuda.current_stream().cuda_stream
+        # ---------------- D step: D.train / G.eval (model_handler.py:355-356) ----------------
+        check(getattr(lib, disc_fn)(C.byref(args), st), disc_fn)
+        self._allreduce(self.D.grad)
+        self.D.adam(self.lr_d)
+        # ---------------- G step: D.eval / G.train (model_handler.py:432-433) ----------------
+        check(getattr(lib, gen_fn)(C.byref(args), st), gen_fn)
+        if self.coef_l1 > 1e-8:
+            check(lib.advmil_abs_sum(self.G.flat.data_ptr(), self.G.total, out["losses"][4:].data_ptr(), st), "advmil_abs_sum")
+        self._allreduce(self.G.grad)
+        self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
+        out["f_fake_d"] = out["f_d"][:nb]
+        out["f_real"] = out["f_d"][nb:] if n_real > 0 else None
+        out["_keep"] = keep
+        # pred_g / noise_g / the masks are also touched by the library's side stream (the forked train forward): the engine
+        # keeps the step's tensors until the NEXT step has been issued, by which time the main stream has joined the side
+        # stream -- a caller that drops `out` early cannot hand their memory back to the allocator under the side stream
+        self._inflight = out
+        return out
 
     @staticmethod
     def _cat_masks(fake, real, keys):
@@ -171,74 +245,28 @@ class AdvStep(_DataParallelMixin):
 
     def step(self, bags: ops.PackedBags, t: torch.Tensor, e: torch.Tensor, visible: torch.Tensor,
              noise_d: Optional[torch.Tensor] = None, noise_g: Optional[torch.Tensor] = None,
-             masks_d_real=None, masks_d_fake=None, masks_g=None, global_counts=None, return_debug=False) -> Dict:
+             masks_d_real=None, masks_d_fake=None, masks_g=None, global_counts=None) -> Dict:
         """t, e: [bags] float32 device; visible: [bags] uint8 device (label_visible_mask).  noise_*: [bags, hid] device
         (drawn like utils/func.generate_noise when None).  Returns device tensors only (no host sync when
         global_counts is given).  Two C calls (advmil_adv_step_disc / _gen) issue the whole launch sequence."""
         lib = _lib.load()
-        st = torch.cuda.current_stream().cuda_stream
-        bags = bags.for_precision(self.precision)   # bf16 mode: bf16 features as packed by the loader, or one cast here
-        dev = bags.x.device
-        nb = bags.bags
-        G = self.netG
-        f32 = dict(dtype=torch.float32, device=dev)
-        t = t.reshape(-1).contiguous().float()
-        e = e.reshape(-1).contiguous().float()
-        visible = visible.reshape(-1).to(torch.uint8).contiguous()
-        if global_counts is None:
-            real_mask = ((e == 1) & (visible != 0))                      # model_handler.py:373-375
-            cnt = torch.stack([real_mask.sum(), torch.tensor(nb, device=dev), visible.sum()]).float()
-            self._allreduce(cnt)
-            n_real, n_fake, n_vis = [float(v) for v in cnt.tolist()]
-        else:
-            n_real, n_fake, n_vis = [float(v) for v in global_counts]
-        if noise_d is None:
-            noise_d = self._draw(nb, dev)
-        if noise_g is None:
-            noise_g = self._draw(nb, dev)
-        noise_d, noise_g = noise_d.contiguous().float(), noise_g.contiguous().float()
+        bags, t, e, visible, counts = self._inputs(bags, t, e, visible, global_counts)
+        dev, nb = bags.x.device, bags.bags
+        noise_d, noise_g = self._noise(nb, dev, noise_d, noise_g)
         gp, dp, gg, dg = self._structs()
-        ws = self._workspace(lib, gp, dp, bags.rows, nb, dev)
-        out = {"losses": torch.zeros(8, **f32), "pred_d": torch.empty(nb, **f32), "pred_g": torch.empty(nb, **f32),
-               "f_d": torch.empty(2 * nb, **f32), "f_fake_g": torch.empty(nb, **f32),
-               "real_mask": torch.empty(nb, dtype=torch.uint8, device=dev)}
+        ws = self._workspace(lib.advmil_adv_step_workspace_bytes(C.byref(gp), C.byref(dp), bags.rows, nb, self.precision), dev)
+        out = self._outputs(nb, dev)
         md = self._cat_masks(masks_d_fake, masks_d_real, ("fc1", "ga", "gs", "fc2"))
         mg = masks_g or {}
-        b = bags.c()
         a = _lib.StepArgs()
-        a.gen, a.disc, a.gen_grads, a.disc_grads, a.bags = C.pointer(gp), C.pointer(dp), C.pointer(gg), C.pointer(dg), C.pointer(b)
-        a.t, a.e, a.visible = t.data_ptr(), e.data_ptr(), visible.data_ptr()
-        a.noise_d, a.noise_g = noise_d.data_ptr(), noise_g.data_ptr()
+        a.gen, a.disc, a.gen_grads, a.disc_grads = C.pointer(gp), C.pointer(dp), C.pointer(gg), C.pointer(dg)
         for k in ("h", "a", "b", "rho", "mlp0"):
             setattr(a, "g_mask_" + k, ops._ptr(mg.get(k)))
         for k in ("fc1", "ga", "gs", "fc2"):
             setattr(a, "d_mask_" + k, ops._ptr(md.get(k)))
-        a.seed_d, a.seed_g = self._seed(), self._seed()
-        a.n_real, a.n_fake, a.n_visible, a.loss_d = n_real, n_fake, n_vis, self.loss_d
-        a.recon_norm, a.recon_alpha, a.recon_gamma = self.recon
-        a.coef_gan, a.precision = self.coef_gan, self.precision
-        a.losses, a.pred_d, a.f_fake_d, a.real_mask = (out["losses"].data_ptr(), out["pred_d"].data_ptr(),
-                                                       out["f_d"].data_ptr(), out["real_mask"].data_ptr())
-        a.pred_g, a.f_fake_g = out["pred_g"].data_ptr(), out["f_fake_g"].data_ptr()
-        a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
-        # ---------------- D step: D.train / G.eval (model_handler.py:355-356) ----------------
-        check(lib.advmil_adv_step_disc(C.byref(a), st), "advmil_adv_step_disc")
-        self._allreduce(self.D.grad)
-        self.D.adam(self.lr_d)
-        # ---------------- G step: D.eval / G.train (model_handler.py:432-433) ----------------
-        check(lib.advmil_adv_step_gen(C.byref(a), st), "advmil_adv_step_gen")
-        if self.coef_l1 > 1e-8:
-            check(lib.advmil_abs_sum(self.G.flat.data_ptr(), self.G.total, out["losses"][4:].data_ptr(), st), "advmil_abs_sum")
-        self._allreduce(self.G.grad)
-        self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
-        out["f_fake_d"] = out["f_d"][:nb]
-        out["f_real"] = out["f_d"][nb:] if n_real > 0 else None
-        out["_keep"] = (t, e, visible, noise_d, noise_g, md, mg, bags)     # inputs stay alive until the stream is done with them
-        # pred_g / noise_g / the masks are also touched by the library's side stream (the forked train forward): the engine
-        # keeps the step's tensors until the NEXT step has been issued, by which time the main stream has joined the side
-        # stream -- a caller that drops `out` early cannot hand their memory back to the allocator under the side stream
-        self._inflight = out
-        return out
+        self._fill_args(a, bags, t, e, visible, noise_d, noise_g, counts, out, ws)
+        return self._update(lib, "advmil_adv_step_disc", "advmil_adv_step_gen", a, out, nb, counts[0],
+                            (t, e, visible, noise_d, noise_g, md, mg, bags))
 
     def loss_dict(self, out) -> Dict[str, float]:
         """Host copy of the step's scalars (one sync): the values the handler prints (model_handler.py:413,486-494); under
@@ -270,13 +298,8 @@ class EsatAdvStep(AdvStep):
         self.D = FlatParams(netD, self.dparams, weight_decay_rule=False)
         self.egrads, self.hgrads, self.dgrads = self.G.grads_for(self.eparams), self.G.grads_for(self.hparams), self.D.grads_for(self.dparams)
         assert self.G.total == sum((t.numel() + 3) // 4 * 4 for t in self.eparams + self.hparams), "generator parameters outside the ESAT step"
-        self.lr_g, self.lr_d, self.wd_g = lr_g, lr_d, weight_decay_g
-        self.coef_gan, self.coef_l1 = coef_gan, coef_l1
-        self.loss_d = {"bce": 0, "hinge": 1, "wasserstein": 2}[loss_d]
-        self.recon = ({"l1": 0, "l2": 1}[recon_norm], recon_alpha, recon_gamma)
-        self.precision = ops.PRECISIONS[precision]
-        self._inflight = None
-        self._init_dp(process_group)
+        self._init_hparams(lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
+                           process_group)
 
     def _structs(self):
         if getattr(self, "_c", None) is None:
@@ -295,58 +318,21 @@ class EsatAdvStep(AdvStep):
     def step(self, bags: ops.PackedBags, t: torch.Tensor, e: torch.Tensor, visible: torch.Tensor,
              noise_d: Optional[torch.Tensor] = None, noise_g: Optional[torch.Tensor] = None, coord=None, global_counts=None) -> Dict:
         lib = _lib.load()
-        st = torch.cuda.current_stream().cuda_stream
-        bags = bags.for_precision(self.precision)
+        bags, t, e, visible, counts = self._inputs(bags, t, e, visible, global_counts)
         dev, nb = bags.x.device, bags.bags
-        f32 = dict(dtype=torch.float32, device=dev)
-        t = t.reshape(-1).contiguous().float()
-        e = e.reshape(-1).contiguous().float()
-        visible = visible.reshape(-1).to(torch.uint8).contiguous()
-        if global_counts is None:
-            real_mask = ((e == 1) & (visible != 0))
-            cnt = torch.stack([real_mask.sum(), torch.tensor(nb, device=dev), visible.sum()]).float()
-            self._allreduce(cnt)
-            n_real, n_fake, n_vis = [float(v) for v in cnt.tolist()]
-        else:
-            n_real, n_fake, n_vis = [float(v) for v in global_counts]
-        noise_d = (noise_d if noise_d is not None else self._draw(nb, dev)).contiguous().float()
-        noise_g = (noise_g if noise_g is not None else self._draw(nb, dev)).contiguous().float()
+        noise_d, noise_g = self._noise(nb, dev, noise_d, noise_g)
         pe = self.netG.backbone.positional(bags, coord)
         ep, hp, dp, eg, hg, dg = self._structs()
-        need = lib.advmil_adv_step_esat_workspace_bytes(C.byref(ep), C.byref(hp), C.byref(dp), bags.rows, nb, self.precision)
-        ws = getattr(self, "_ws", None)
-        if ws is None or ws.numel() < need or ws.device != dev:
-            self._ws = ws = torch.empty(int(need * 1.05) + 4096, dtype=torch.uint8, device=dev)      # grow-only
-        out = {"losses": torch.zeros(8, **f32), "pred_d": torch.empty(nb, **f32), "pred_g": torch.empty(nb, **f32),
-               "f_d": torch.empty(2 * nb, **f32), "f_fake_g": torch.empty(nb, **f32),
-               "real_mask": torch.empty(nb, dtype=torch.uint8, device=dev)}
-        b = bags.c()
+        ws = self._workspace(lib.advmil_adv_step_esat_workspace_bytes(C.byref(ep), C.byref(hp), C.byref(dp), bags.rows, nb,
+                                                                      self.precision), dev)
+        out = self._outputs(nb, dev)
         a = _lib.EsatStepArgs()
         a.esat, a.head, a.disc = C.pointer(ep), C.pointer(hp), C.pointer(dp)
-        a.esat_grads, a.head_grads, a.disc_grads, a.bags = C.pointer(eg), C.pointer(hg), C.pointer(dg), C.pointer(b)
-        a.t, a.e, a.visible = t.data_ptr(), e.data_ptr(), visible.data_ptr()
-        a.noise_d, a.noise_g, a.pe = noise_d.data_ptr(), noise_g.data_ptr(), ops._ptr(pe)
-        a.seed_d, a.seed_g = self._seed(), self._seed()
-        a.n_real, a.n_fake, a.n_visible, a.loss_d = n_real, n_fake, n_vis, self.loss_d
-        a.recon_norm, a.recon_alpha, a.recon_gamma = self.recon
-        a.coef_gan, a.precision = self.coef_gan, self.precision
-        a.losses, a.pred_d, a.f_fake_d, a.real_mask = (out["losses"].data_ptr(), out["pred_d"].data_ptr(),
-                                                       out["f_d"].data_ptr(), out["real_mask"].data_ptr())
-        a.pred_g, a.f_fake_g = out["pred_g"].data_ptr(), out["f_fake_g"].data_ptr()
-        a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
-        check(lib.advmil_adv_step_esat_disc(C.byref(a), st), "advmil_adv_step_esat_disc")
-        self._allreduce(self.D.grad)
-        self.D.adam(self.lr_d)
-        check(lib.advmil_adv_step_esat_gen(C.byref(a), st), "advmil_adv_step_esat_gen")
-        if self.coef_l1 > 1e-8:
-            check(lib.advmil_abs_sum(self.G.flat.data_ptr(), self.G.total, out["losses"][4:].data_ptr(), st), "advmil_abs_sum")
-        self._allreduce(self.G.grad)
-        self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
-        out["f_fake_d"] = out["f_d"][:nb]
-        out["f_real"] = out["f_d"][nb:] if n_real > 0 else None
-        out["_keep"] = (t, e, visible, noise_d, noise_g, pe, bags)
-        self._inflight = out
-        return out
+        a.esat_grads, a.head_grads, a.disc_grads = C.pointer(eg), C.pointer(hg), C.pointer(dg)
+        a.pe = ops._ptr(pe)
+        self._fill_args(a, bags, t, e, visible, noise_d, noise_g, counts, out, ws)
+        return self._update(lib, "advmil_adv_step_esat_disc", "advmil_adv_step_esat_gen", a, out, nb, counts[0],
+                            (t, e, visible, noise_d, noise_g, pe, bags))
 
 
 class ClusterAdvStep(AdvStep):
@@ -380,13 +366,8 @@ class ClusterAdvStep(AdvStep):
         self.dWphi, self.dbphi = self.G.grads_for([self.Wphi, self.bphi])
         covered = [t for t in self.gparams if t is not None] + [self.Wphi, self.bphi]
         assert self.G.total == sum((t.numel() + 3) // 4 * 4 for t in covered), "generator parameters outside the cluster step"
-        self.lr_g, self.lr_d, self.wd_g = lr_g, lr_d, weight_decay_g
-        self.coef_gan, self.coef_l1 = coef_gan, coef_l1
-        self.loss_d = {"bce": 0, "hinge": 1, "wasserstein": 2}[loss_d]
-        self.recon = ({"l1": 0, "l2": 1}[recon_norm], recon_alpha, recon_gamma)
-        self.precision = ops.PRECISIONS[precision]
-        self._inflight = None
-        self._init_dp(process_group)
+        self._init_hparams(lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
+                           process_group)
 
     def step(self, bags: ops.PackedBags, t: torch.Tensor, e: torch.Tensor, visible: torch.Tensor,
              noise_d: Optional[torch.Tensor] = None, noise_g: Optional[torch.Tensor] = None, ext=None,
@@ -395,69 +376,31 @@ class ClusterAdvStep(AdvStep):
         if ext is None:
             raise ValueError("ClusterAdvStep.step needs the cluster id of every row (ext)")
         lib = _lib.load()
-        st = torch.cuda.current_stream().cuda_stream
-        bags = bags.for_precision(self.precision)
+        bags, t, e, visible, counts = self._inputs(bags, t, e, visible, global_counts)
         dev, nb = bags.x.device, bags.bags
         cid = ext.reshape(-1)
         cid = (cid if cid.dtype == torch.int32 else cid.to(torch.int32)).contiguous()
         assert cid.numel() == bags.rows and cid.device == dev, "one cluster id per row, on the bags' device"
-        f32 = dict(dtype=torch.float32, device=dev)
-        t = t.reshape(-1).contiguous().float()
-        e = e.reshape(-1).contiguous().float()
-        visible = visible.reshape(-1).to(torch.uint8).contiguous()
-        if global_counts is None:
-            real_mask = ((e == 1) & (visible != 0))
-            cnt = torch.stack([real_mask.sum(), torch.tensor(nb, device=dev), visible.sum()]).float()
-            self._allreduce(cnt)
-            n_real, n_fake, n_vis = [float(v) for v in cnt.tolist()]
-        else:
-            n_real, n_fake, n_vis = [float(v) for v in global_counts]
-        noise_d = (noise_d if noise_d is not None else self._draw(nb, dev)).contiguous().float()
-        noise_g = (noise_g if noise_g is not None else self._draw(nb, dev)).contiguous().float()
+        noise_d, noise_g = self._noise(nb, dev, noise_d, noise_g)
         gp, dp, gg, dg = self._structs()
         ncl = self.netG.backbone.num_clusters
-        need = lib.advmil_adv_step_cluster_workspace_bytes(C.byref(gp), C.byref(dp), bags.rows, nb, ncl, self.precision)
-        ws = getattr(self, "_ws", None)
-        if ws is None or ws.numel() < need or ws.device != dev:
-            self._ws = ws = torch.empty(int(need * 1.05) + 4096, dtype=torch.uint8, device=dev)      # grow-only
-        out = {"losses": torch.zeros(8, **f32), "pred_d": torch.empty(nb, **f32), "pred_g": torch.empty(nb, **f32),
-               "f_d": torch.empty(2 * nb, **f32), "f_fake_g": torch.empty(nb, **f32),
-               "real_mask": torch.empty(nb, dtype=torch.uint8, device=dev)}
+        ws = self._workspace(lib.advmil_adv_step_cluster_workspace_bytes(C.byref(gp), C.byref(dp), bags.rows, nb, ncl,
+                                                                         self.precision), dev)
+        out = self._outputs(nb, dev)
         md = self._cat_masks(masks_d_fake, masks_d_real, ("fc1", "ga", "gs", "fc2"))
         mg = {k: v.contiguous() for k, v in (masks_g or {}).items()}
-        b = bags.c()
         ca = _lib.ClusterStepArgs()
         a = ca.base
-        a.gen, a.disc, a.gen_grads, a.disc_grads, a.bags = C.pointer(gp), C.pointer(dp), C.pointer(gg), C.pointer(dg), C.pointer(b)
-        a.t, a.e, a.visible = t.data_ptr(), e.data_ptr(), visible.data_ptr()
-        a.noise_d, a.noise_g = noise_d.data_ptr(), noise_g.data_ptr()
+        a.gen, a.disc, a.gen_grads, a.disc_grads = C.pointer(gp), C.pointer(dp), C.pointer(gg), C.pointer(dg)
         for k in ("h", "a", "b", "mlp0"):
             setattr(a, "g_mask_" + k, ops._ptr(mg.get(k)))
         for k in ("fc1", "ga", "gs", "fc2"):
             setattr(a, "d_mask_" + k, ops._ptr(md.get(k)))
-        a.seed_d, a.seed_g = self._seed(), self._seed()
-        a.n_real, a.n_fake, a.n_visible, a.loss_d = n_real, n_fake, n_vis, self.loss_d
-        a.recon_norm, a.recon_alpha, a.recon_gamma = self.recon
-        a.coef_gan, a.precision = self.coef_gan, self.precision
-        a.losses, a.pred_d, a.f_fake_d, a.real_mask = (out["losses"].data_ptr(), out["pred_d"].data_ptr(),
-                                                       out["f_d"].data_ptr(), out["real_mask"].data_ptr())
-        a.pred_g, a.f_fake_g = out["pred_g"].data_ptr(), out["f_fake_g"].data_ptr()
-        a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
+        self._fill_args(a, bags, t, e, visible, noise_d, noise_g, counts, out, ws)
         ca.Wphi, ca.bphi, ca.dWphi, ca.dbphi = self.Wphi.data_ptr(), self.bphi.data_ptr(), self.dWphi.data_ptr(), self.dbphi.data_ptr()
         ca.cid, ca.num_clusters = cid.data_ptr(), ncl
-        check(lib.advmil_adv_step_cluster_disc(C.byref(ca), st), "advmil_adv_step_cluster_disc")
-        self._allreduce(self.D.grad)
-        self.D.adam(self.lr_d)
-        check(lib.advmil_adv_step_cluster_gen(C.byref(ca), st), "advmil_adv_step_cluster_gen")
-        if self.coef_l1 > 1e-8:
-            check(lib.advmil_abs_sum(self.G.flat.data_ptr(), self.G.total, out["losses"][4:].data_ptr(), st), "advmil_abs_sum")
-        self._allreduce(self.G.grad)
-        self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
-        out["f_fake_d"] = out["f_d"][:nb]
-        out["f_real"] = out["f_d"][nb:] if n_real > 0 else None
-        out["_keep"] = (t, e, visible, noise_d, noise_g, md, mg, cid, bags)
-        self._inflight = out
-        return out
+        return self._update(lib, "advmil_adv_step_cluster_disc", "advmil_adv_step_cluster_gen", ca, out, nb, counts[0],
+                            (t, e, visible, noise_d, noise_g, md, mg, cid, bags))
 
 
 class ModuleAdvStep(_DataParallelMixin):
