@@ -266,7 +266,8 @@ ADVMIL_API int advmil_cluster_pool_bwd(const float* d_hc, const uint32_t* keep, 
 ADVMIL_API int advmil_linear_fwd(const void* x, const float* W, const float* b, int32_t rows, int32_t K, int32_t N, int32_t act,
                       float p_drop, const uint8_t* mask, uint64_t seed, int32_t site, int32_t train,
                       int32_t precision, void* y, void* stream);
-/* dX = dY W (optionally * (y_fwd>0)/(1-p) when relu_y != NULL), dW = dY^T X, db = colsum(dY); any output may be NULL */
+/* dX = dY W, dW = dY^T X, db = colsum(dY); any output may be NULL (dX needs W, dW needs X).  accumulate != 0 adds
+ * into dX, dW and db instead of overwriting them. */
 ADVMIL_API int advmil_linear_bwd(const void* dY, const void* X, const float* W, int32_t rows, int32_t K, int32_t N,
                       void* dX, float* dW, float* db, int32_t accumulate, int32_t precision,
                       void* workspace, size_t workspace_bytes, void* stream);
