@@ -282,8 +282,11 @@ extern "C" int advmil_disc_embed_fwd(const AdvmilDiscParams* p, const AdvmilBags
   ADVMIL_TRY(check_bags(bags, p->C, true, a->precision));
   ADVMIL_TRY(check_ksize(p));
   ProfScope ps(PROF_EMBED, (cudaStream_t)stream);
+  // the fp32 embedding at d = 256 writes y before its LayerNorm pass: into y_pre, or into the workspace when y_pre is not saved
+  const size_t y_bytes = (size_t)bags->rows * p->d * sizeof(float);
+  float* y_ws = (a->workspace && a->workspace_bytes >= y_bytes) ? (float*)a->workspace : nullptr;
   return region_embed_fwd(bags->x, p->Wc, p->bc, p->ln_g, p->ln_b, bags->rows, p->C, p->d, p->ln_eps, a->y_pre, a->emb,
-                          a->precision, (cudaStream_t)stream, disc_ksize(p));
+                          a->precision, (cudaStream_t)stream, disc_ksize(p), y_ws);
 }
 
 namespace advmil {

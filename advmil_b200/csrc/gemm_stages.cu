@@ -54,9 +54,9 @@ int gated_score_fwd(const void* v, const float* Wp, const float* bp, const float
 }
 
 int region_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta, int rows,
-                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st, int ksize) {
+                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st, int ksize, float* y_ws) {
   ADVMIL_REQUIRE(rows % 16 == 0, "region_embed: rows %d not a multiple of 16 (backbone_utils.py:65)", rows);
-  ADVMIL_REQUIRE(d <= 128 && d % 4 == 0 && C % 4 == 0, "region_embed: d=%d (<=128, %%4) C=%d (%%4) unsupported", d, C);
+  ADVMIL_REQUIRE(((d <= 128 && d % 4 == 0) || d == 256) && C % 4 == 0, "region_embed: d=%d (<=128 and %%4, or 256) C=%d (%%4) unsupported", d, C);
   ADVMIL_REQUIRE(ksize == 1 || C % 16 == 0, "region_embed: the 3x3 embedding needs C %% 16 == 0 (C=%d)", C);
   // rejected here rather than in the backward: bf16 runs only on tcgen05, and the 3x3 weight gradient tiles its 9 C columns
   // by 128 or 256 without straddling a tap
@@ -67,6 +67,23 @@ int region_embed_fwd(const void* x, const float* Wc, const float* bc, const floa
     return ksize == 3 ? tc_conv3_embed_fwd(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, precision, st)
                       : tc_region_embed_fwd(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, precision, st);
   ADVMIL_REQUIRE(precision != ADVMIL_BF16, kBf16Shape, "region_embed_fwd", rows, C, d);
+  if (d > 128) {
+    // EpiLNPool needs the whole row in one 128-column tile: y = x Wc^T + bc first, then LayerNorm + ReLU + region mean
+    // per row (the same two passes as the ESAT patch embedding)
+    float* y = y_pre ? (float*)y_pre : y_ws;
+    ADVMIL_REQUIRE(y, "region_embed: the fp32 embedding at d=%d needs y_pre or %d x %d floats of workspace", d, rows, d);
+    EpiLinear lin{y, d, bc, 0, Drop::make(nullptr, 0, 0, 0.f, 0, 0), d};
+    if (ksize == 3) {
+      const float* Wk;
+      ADVMIL_TRY(conv3_weight_f32(Wc, d, C, st, &Wk));
+      GemmArgs g{(const float*)x, Wk, rows, d, 9 * C, C, 9 * C, 9 * C};
+      ADVMIL_TRY((launch_gemm<true, true, EpiLinear, Conv3LoaderA>(g, lin, 1, st)));
+    } else {
+      GemmArgs g{(const float*)x, Wc, rows, d, C, C, C, C};
+      ADVMIL_TRY((launch_gemm<true, true>(g, lin, 1, st)));
+    }
+    return ln_relu_mean16_fwd(y, gamma, beta, rows, d, eps, nullptr, emb, ELEM_F32, st);
+  }
   EpiLNPool epi{(float*)y_pre, emb, bc, gamma, beta, d, eps};
   if (ksize == 3) {
     const float* Wk;

@@ -153,7 +153,9 @@ template <int ES, int BLOCK_N, int EPI, bool X3 = false> struct RowCfg {
   static constexpr int STAGE_BYTES = (X3 ? 2 : 1) * (A_STAGE_BYTES + B_STAGE_BYTES);
   static constexpr int TMA_BYTES = A_STAGE_BYTES + (X3 ? 2 : 1) * B_STAGE_BYTES;     // what TMA delivers per stage
   // bf16 staging: 32 rows x 64 bytes, XOR-swizzled (2 KB per warp); fp32 staging: 32 x 36 floats; LN: full 128-column rows
-  static constexpr int STG_FLOATS_PER_WARP = (EPI == EPI_LN) ? 32 * STG_LD_LN : ((ES == 2 && EPI != EPI_PE && EPI != EPI_POOL) ? 32 * 64 / 4 : 32 * STG_LD);
+  // (the 64- and 256-column LN epilogues work chunk by chunk and stage 32 columns)
+  static constexpr int STG_FLOATS_PER_WARP = (EPI == EPI_LN) ? (BLOCK_N == 128 ? 32 * STG_LD_LN : 32 * STG_LD)
+                                                             : ((ES == 2 && EPI != EPI_PE && EPI != EPI_POOL) ? 32 * 64 / 4 : 32 * STG_LD);
   // gate: per 32-pair chunk 32 tanh biases | 32 sigmoid biases | 32 w_c (4 / NSUB chunks per warp);
   // proj+embed: conv bias | gamma | beta (128 each); cluster pool: per-cluster column sums of the warp's two 16-row halves
   static constexpr int COEF_FLOATS_PER_WARP = (EPI == EPI_GATE) ? 384 / NSUB : (EPI == EPI_PE) ? 384 : (EPI == EPI_POOL) ? 2 * 16 * 32 : 0;
@@ -1034,6 +1036,70 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           asm volatile("bar.sync %0, 64;" ::"r"(1 + wq * 2 + blk) : "memory");     // the two warps of (quarter, block)
           if (!(sub & 1) && m_row < M) ea.part[(size_t)(nt * 2 + blk) * M + m_row] = partial + slot[lane];
         }
+      } else if constexpr (EPI == EPI_LN && BLOCK_N != 128) {
+        // BLOCK_N == d == 64 or 256: three sweeps over this row's TMEM columns (sum -> mean, squared deviations -> rstd,
+        // normalise + store), one 32-column chunk in registers at a time.  A 256-float row would not fit the register file
+        // the 128-column variant below already fills.  The accumulator stays allocated for the three sweeps.
+        constexpr int NCH = BLOCK_N / 32;
+        const bool rowok = m_row < M;
+        auto ld_y = [&](int ch, float (&v)[32]) {
+          ld_acc(ch * 32, v);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) {
+            float y = v[i] + __ldg(ea.bias + ch * 32 + i);
+            if constexpr (sizeof(T) == 2) y = __bfloat162float(__float2bfloat16_rn(y));      // y_pre is bf16: see below
+            v[i] = y;
+          }
+        };
+        float ssum = 0.f;
+#pragma unroll 1
+        for (int ch = 0; ch < NCH; ++ch) {
+          float v[32];
+          ld_y(ch, v);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) ssum += v[i];
+        }
+        const float mean = ssum * (1.0f / BLOCK_N);
+        float qsum = 0.f;
+#pragma unroll 1
+        for (int ch = 0; ch < NCH; ++ch) {
+          float v[32];
+          ld_y(ch, v);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) { const float c = v[i] - mean; qsum = fmaf(c, c, qsum); }
+        }
+        const float rstd = rsqrtf(qsum * (1.0f / BLOCK_N) + ea.eps);
+#pragma unroll 1
+        for (int ch = 0; ch < NCH; ++ch) {
+          float v[32];
+          ld_y(ch, v);
+          if (ch == NCH - 1) { release_acc(&tempty[acc]); }
+          if (ea.y_pre) {
+            if constexpr (sizeof(T) == 2) {
+              store_rows_bf16(reinterpret_cast<uint8_t*>(stg), v, reinterpret_cast<bf16*>(ea.y_pre), BLOCK_N, m_base, M, ch * 32, lane);
+            } else {
+              stage_chunk(stg, STG_LD, 0, v, lane);
+              __syncwarp();
+              store_staged<T, 32>(stg, STG_LD, reinterpret_cast<T*>(ea.y_pre), BLOCK_N, m_base, M, ch * 32, lane);
+              __syncwarp();
+            }
+          }
+#pragma unroll
+          for (int i = 0; i < 32; ++i)
+            v[i] = rowok ? fmaxf(fmaf((v[i] - mean) * rstd, __ldg(ea.gamma + ch * 32 + i), __ldg(ea.beta + ch * 32 + i)), 0.f) : 0.f;
+          stage_chunk(stg, STG_LD, 0, v, lane);
+          __syncwarp();
+          const int rg = lane >> 4, c2 = (lane & 15) * 2;      // two 16-row regions per warp, two columns per lane
+          float a0 = 0.f, a1 = 0.f;
+#pragma unroll
+          for (int r = 0; r < 16; ++r) {
+            const float2 t2 = *reinterpret_cast<const float2*>(stg + (rg * 16 + r) * STG_LD + c2);
+            a0 += t2.x; a1 += t2.y;
+          }
+          const int m = m_base + rg * 16;
+          if (m < M) *reinterpret_cast<float2*>(ea.emb + (size_t)(m >> 4) * BLOCK_N + ch * 32 + c2) = make_float2(a0 * 0.0625f, a1 * 0.0625f);
+          __syncwarp();
+        }
       } else if constexpr (EPI == EPI_LN) {
         // BLOCK_N == 128 == d: the whole row lives in this thread's registers
         float v[128];
@@ -1509,7 +1575,21 @@ int tc_gated_score_fwd(const void* v, const float* Wp, const float* bp, const fl
   return gate_score_finish(part, gate_width(D) / 128, rows, bc, s, st);
 }
 
-bool tc_embed_supported(int rows, int C, int d, int dt) { return rows_ok(rows, dt) && C % kblk_of(dt) == 0 && d == 128; }
+// d = 64 / 128 / 256: one tile holds the whole row that LayerNorm needs (a 256-column split-tf32 tile has room for two
+// stages: see RowCfg)
+bool tc_embed_supported(int rows, int C, int d, int dt) {
+  return rows_ok(rows, dt) && C % kblk_of(dt) == 0 && (d == 64 || d == 128 || d == 256);
+}
+template <typename T, bool X3 = false, bool CONV = false>
+static int launch_embed(const T* x, const T* W, int rows, int K, int d, const RowEpi& ea, cudaStream_t st, const T* Wlo = nullptr) {
+  switch (d) {
+    case 64: return launch_rows<T, 64, EPI_LN, true, X3, CONV>(x, W, rows, K, d, ea, st, Wlo);
+    case 128: return launch_rows<T, 128, EPI_LN, true, X3, CONV>(x, W, rows, K, d, ea, st, Wlo);
+    case 256: return launch_rows<T, 256, EPI_LN, true, X3, CONV>(x, W, rows, K, d, ea, st, Wlo);
+  }
+  set_error("tc: region embedding width d=%d unsupported (64, 128 or 256)", d);
+  return ADVMIL_ERR_INVALID;
+}
 
 template <typename T>
 static int tc_embed_t(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta, int rows, int C,
@@ -1518,7 +1598,7 @@ static int tc_embed_t(const void* x, const float* Wc, const float* bc, const flo
   ADVMIL_TRY(weight_operand<T>(Wc, (size_t)d * C, WS_EMBED, st, &Wt));
   RowEpi ea{};
   ea.bias = bc; ea.y_pre = y_pre; ea.emb = emb; ea.gamma = gamma; ea.beta = beta; ea.eps = eps;
-  return launch_rows<T, 128, EPI_LN, true>((const T*)x, Wt, rows, C, d, ea, st);
+  return launch_embed<T>((const T*)x, Wt, rows, C, d, ea, st);
 }
 int tc_region_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta,
                         int rows, int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st) {
@@ -1528,7 +1608,7 @@ int tc_region_embed_fwd(const void* x, const float* Wc, const float* bc, const f
     ADVMIL_TRY(weight_split(Wc, (size_t)d * C, WS_EMBED, st, &Wh, &Wl));
     RowEpi ea{};
     ea.bias = bc; ea.y_pre = y_pre; ea.emb = emb; ea.gamma = gamma; ea.beta = beta; ea.eps = eps;
-    return launch_rows<float, 128, EPI_LN, true, true>((const float*)x, Wh, rows, C, d, ea, st, Wl);
+    return launch_embed<float, true>((const float*)x, Wh, rows, C, d, ea, st, Wl);
   }
   return tc_embed_t<float>(x, Wc, bc, gamma, beta, rows, C, d, eps, y_pre, emb, st);
 }
@@ -1576,7 +1656,7 @@ static int tc_conv3_embed_t(const void* x, const float* Wc, const float* bc, con
   ADVMIL_TRY(conv3_operand<T>(Wc, d, C, X3, st, &Wt, &Wl));
   RowEpi ea{};
   ea.bias = bc; ea.y_pre = y_pre; ea.emb = emb; ea.gamma = gamma; ea.beta = beta; ea.eps = eps;
-  return launch_rows<T, 128, EPI_LN, true, X3, true>((const T*)x, Wt, rows, 9 * C, d, ea, st, Wl);
+  return launch_embed<T, X3, true>((const T*)x, Wt, rows, 9 * C, d, ea, st, Wl);
 }
 int tc_conv3_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta,
                        int rows, int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st) {

@@ -3,7 +3,7 @@
 //   fi  = f1 F1b^T + b                            EmbedXLayer.fc1.3     (the "instance embeddings", quirk A.4#2)
 //   a,b = tanh(fi Pg^T + b), sigmoid(fi Ps^T + b) GAPool gate           (reference model/backbone_utils.py:47-56)
 //   rep = sum_j drop(a_j) drop(b_j) Pc_j                                (bias and softmax: seg_softmax_pool_fwd)
-// over R = rows / 16 regions of width d = 128.  These are 49 152 multiply-adds per region: far too little to fill the
+// over R = rows / 16 regions of width d = 64, 128 or 256 (128: 49 152 multiply-adds per region): far too little to fill the
 // tensor pipe kernel by kernel (round 1: four launches of 10-25 us, tensor pipe 2-10 %, a quarter of the step for 0.2 % of
 // its FLOPs).  One CTA owns 32 or 64 regions and walks the three contractions with the intermediates in shared memory; the
 // weights (192 KB, L2-resident) stream through a double-buffered stage.  The chain is fp32-grade in EVERY precision mode (no
@@ -26,25 +26,31 @@
 // of the SAME columns, so that a thread holds both halves of each (tanh_j, sigmoid_j) pair in matching fragment slots.
 // Measured (ncu, B200): 84 us for 32768 regions with <WM, KC> = <1, 16> (4 CTAs per SM), 46 us for 16384 regions with <2, 32>
 // (2 CTAs per SM); legacy tensor pipe 43-47 % busy, HMMA.1688.F32.TF32 at ~10.6 cycles per instruction and sub-core.
+// Other widths: phase 1 has d / 2 columns (d / 64 n-tiles per warp); phase 2 runs its d columns in groups of at most 128
+// (4 n-tiles per warp, as at d = 128: the accumulators of a 256-column phase would not fit beside the fragments); the gate
+// has d / 64 blocks.  Weight stages hold at most 128 rows at every width.
 #include "stages.cuh"
 
 namespace advmil {
 
 namespace {
 
-constexpr int CH_D = 128, CH_DH = 64;
-
 namespace mm {
-constexpr int LDA = CH_D + 4, LDF = CH_DH + 4, WROWS = 128;
+constexpr int WROWS = 128;
+// D = region width (64, 128 or 256), DH = D / 2.
 // WM = warp rows per CTA (a warp owns 32 regions): 64 regions / 256 threads or 32 regions / 128 threads; KC = K extent of a
 // weight stage.  Smaller CTAs balance better over the 148 SMs (16384 regions = 110.7 per SM) and decouple the phases of the
 // CTAs that share an SM (one CTA's epilogue runs under another's MMAs).
-template <int WM, int KC>
+template <int D, int WM, int KC>
 struct Cfg {
+  static constexpr int DH = D / 2, LDA = D + 4, LDF = DH + 4;
   static constexpr int TM = 32 * WM, THREADS = 128 * WM, LDW = KC + 4;
-  static constexpr int NC1 = CH_D / KC, NC2 = CH_DH / KC, NCHUNK = 3 * NC1 + NC2;
-  static constexpr size_t SMEM_FLOATS = (size_t)TM * LDA + (size_t)TM * LDF + 2 * (size_t)WROWS * LDW + 2 * 4 * TM;
+  static constexpr int W2 = D < 128 ? D : 128, G2 = D / W2;      // phase 2: G2 column groups of W2 columns
+  static constexpr int NB = D / 64;                               // gate blocks of 64 (tanh, sigmoid) pairs
+  static constexpr int NC1 = D / KC, NC2 = DH / KC, NCHUNK = NC1 + G2 * NC2 + NB * NC1;
+  static constexpr size_t SMEM_FLOATS = (size_t)TM * LDA + (size_t)TM * LDF + 2 * (size_t)WROWS * LDW + (size_t)NB * 4 * TM;
   static constexpr int MIN_CTAS = WM == 2 ? 2 : 4;
+  static_assert(NC2 >= 1 && DH <= WROWS, "unsupported chain width");
 };
 
 __device__ __forceinline__ void split3(float x, uint32_t& hi, uint32_t& lo) {
@@ -121,16 +127,17 @@ __device__ __forceinline__ void zero_acc(float (&a)[2][NT][4], float (&b)[2][NT]
       for (int e = 0; e < 4; ++e) { a[i][j][e] = 0.f; b[i][j][e] = 0.f; }
 }
 
-template <int WM, int KC>
-__global__ void __launch_bounds__(Cfg<WM, KC>::THREADS, Cfg<WM, KC>::MIN_CTAS)
+template <int D, int WM, int KC>
+__global__ void __launch_bounds__(Cfg<D, WM, KC>::THREADS, Cfg<D, WM, KC>::MIN_CTAS)
 rlip_chain_mma_kernel(const float* __restrict__ emb, const float* __restrict__ F1a_w, const float* __restrict__ F1a_b,
                       const float* __restrict__ F1b_w, const float* __restrict__ F1b_b, const float* __restrict__ Pg_w,
                       const float* __restrict__ Pg_b, const float* __restrict__ Ps_w, const float* __restrict__ Ps_b,
                       const float* __restrict__ Pc_w, int R, Drop dfc1, Drop dga, Drop dgs, float* __restrict__ f1,
                       float* __restrict__ fi, float* __restrict__ ab, float* __restrict__ part) {
   pdl_prologue();
-  using C = Cfg<WM, KC>;
-  constexpr int D = CH_D, DH = CH_DH, ABW = 2 * CH_D, TM = C::TM, THREADS = C::THREADS, LDW = C::LDW, NC1 = C::NC1, NC2 = C::NC2;
+  using C = Cfg<D, WM, KC>;
+  constexpr int DH = C::DH, ABW = 2 * D, TM = C::TM, THREADS = C::THREADS, LDW = C::LDW, NC1 = C::NC1, NC2 = C::NC2;
+  constexpr int LDA = C::LDA, LDF = C::LDF, W2 = C::W2, NT1 = DH / 32, NT2 = W2 / 32;
   extern __shared__ __align__(16) float smem[];
   float* actA = smem;                                   // [TM][LDA]: emb, later fi
   float* f1A = actA + (size_t)TM * LDA;                 // [TM][LDF]
@@ -141,13 +148,17 @@ rlip_chain_mma_kernel(const float* __restrict__ emb, const float* __restrict__ F
   const int m0 = blockIdx.x * TM;
   const int rbase = wm * 32;                            // this warp's first row of the tile
 
-  // weight chunk q of the schedule: F1a (NC1 chunks of K = 128), F1b (NC2, K = 64), gate block 0 (NC1), gate block 1 (NC1)
+  // weight chunk q of the schedule: F1a (NC1 chunks of K = D), F1b (G2 column groups of NC2 chunks, K = DH), then the
+  // NB gate blocks (NC1 chunks each)
   auto issue_chunk = [&](int q) {
     float* stage = wst + (size_t)(q & 1) * WROWS * LDW;
-    if (q < NC1) load_w_chunk<KC, THREADS, 64>(stage, F1a_w, nullptr, D, q * KC, tid);
-    else if (q < NC1 + NC2) load_w_chunk<KC, THREADS, 128>(stage, F1b_w, F1b_w + (size_t)64 * DH, DH, (q - NC1) * KC, tid);
-    else {
-      const int c = (q - NC1 - NC2) / NC1, kq = (q - NC1 - NC2) % NC1;
+    if (q < NC1) load_w_chunk<KC, THREADS, DH>(stage, F1a_w, DH > 64 ? F1a_w + (size_t)64 * D : nullptr, D, q * KC, tid);
+    else if (q < NC1 + C::G2 * NC2) {
+      const int grp = C::G2 == 1 ? 0 : (q - NC1) / NC2, kq = C::G2 == 1 ? q - NC1 : (q - NC1) % NC2;
+      const float* W0 = F1b_w + (size_t)grp * W2 * DH;
+      load_w_chunk<KC, THREADS, W2>(stage, W0, W0 + (size_t)64 * DH, DH, kq * KC, tid);
+    } else {
+      const int c = (q - NC1 - C::G2 * NC2) / NC1, kq = (q - NC1 - C::G2 * NC2) % NC1;
       load_w_chunk<KC, THREADS, 128>(stage, Pg_w + (size_t)c * 64 * D, Ps_w + (size_t)c * 64 * D, D, kq * KC, tid);
     }
     cp_async_commit();
@@ -162,24 +173,26 @@ rlip_chain_mma_kernel(const float* __restrict__ emb, const float* __restrict__ F
 
   // ---- emb tile (row-major, zero beyond R) + first weight chunk ----
   for (int i = tid; i < TM * (D / 4); i += THREADS) {
-    const int r = i >> 5, c4 = i & 31;
+    const int r = i / (D / 4), c4 = i % (D / 4);
     if (m0 + r < R) cp_async16(actA + (size_t)r * LDA + 4 * c4, emb + (size_t)(m0 + r) * D + 4 * c4);
     else *reinterpret_cast<float4*>(actA + (size_t)r * LDA + 4 * c4) = make_float4(0.f, 0.f, 0.f, 0.f);
   }
   issue_chunk(0);
 
-  // ---- phase 1: f1 = dropout(relu(emb F1a^T + b)), 64 columns: 2 n-tiles per warp ----
+  // ---- phase 1: f1 = dropout(relu(emb F1a^T + b)), DH columns: NT1 n-tiles per warp ----
   {
-    float accm[2][2][4], accs[2][2][4];
-    zero_acc<2>(accm, accs);
-    const int nrow[2] = {wn * 16, wn * 16 + 8};
+    float accm[2][NT1][4], accs[2][NT1][4];
+    zero_acc<NT1>(accm, accs);
+    int nrow[NT1];
+#pragma unroll
+    for (int nt = 0; nt < NT1; ++nt) nrow[nt] = wn * (DH / 4) + nt * 8;
 #pragma unroll 1
     for (int q = 0; q < NC1; ++q) {
       const float* Ws = advance(q);
-      mma_chunk<2, KC>(accm, accs, actA + (size_t)rbase * LDA, LDA, q * KC, Ws, nrow, g, t);
+      mma_chunk<NT1, KC>(accm, accs, actA + (size_t)rbase * LDA, LDA, q * KC, Ws, nrow, g, t);
     }
 #pragma unroll
-    for (int nt = 0; nt < 2; ++nt) {
+    for (int nt = 0; nt < NT1; ++nt) {
       const int n = nrow[nt] + 2 * t;
       const float2 bv = *reinterpret_cast<const float2*>(F1a_b + n);
 #pragma unroll
@@ -201,28 +214,36 @@ rlip_chain_mma_kernel(const float* __restrict__ emb, const float* __restrict__ F
     }
   }
 
+  // ---- phase 2: fi = f1 F1b^T + b, D columns in G2 groups of W2: NT2 n-tiles per warp; fi replaces emb in shared memory.
+  //      With 4 n-tiles per warp the accumulators are those of phase 3 ----
   float accm[2][4][4], accs[2][4][4];
-  // ---- phase 2: fi = f1 F1b^T + b, 128 columns: 4 n-tiles per warp; fi replaces emb in shared memory ----
-  {
-    zero_acc<4>(accm, accs);
-    const int nrow[4] = {wn * 32, wn * 32 + 8, wn * 32 + 16, wn * 32 + 24};
+  float am1[2][NT2 == 4 ? 1 : NT2][4], as1[2][NT2 == 4 ? 1 : NT2][4];
+  auto& am = *reinterpret_cast<float (*)[2][NT2][4]>(NT2 == 4 ? (void*)accm : (void*)am1);
+  auto& as = *reinterpret_cast<float (*)[2][NT2][4]>(NT2 == 4 ? (void*)accs : (void*)as1);
 #pragma unroll 1
-    for (int q = NC1; q < NC1 + NC2; ++q) {
+  for (int grp = 0; grp < C::G2; ++grp) {
+    zero_acc<NT2>(am, as);
+    int nrow[NT2];
+#pragma unroll
+    for (int nt = 0; nt < NT2; ++nt) nrow[nt] = wn * (W2 / 4) + nt * 8;
+    const int q0 = NC1 + grp * NC2;
+#pragma unroll 1
+    for (int q = q0; q < q0 + NC2; ++q) {
       const float* Ws = advance(q);
-      mma_chunk<4, KC>(accm, accs, f1A + (size_t)rbase * LDF, LDF, (q - NC1) * KC, Ws, nrow, g, t);
+      mma_chunk<NT2, KC>(am, as, f1A + (size_t)rbase * LDF, LDF, (q - q0) * KC, Ws, nrow, g, t);
     }
     // every warp has finished reading emb (phase 1) before any thread got past the barriers of this phase
 #pragma unroll
-    for (int nt = 0; nt < 4; ++nt) {
-      const int n = nrow[nt] + 2 * t;
+    for (int nt = 0; nt < NT2; ++nt) {
+      const int n = grp * W2 + nrow[nt] + 2 * t;
       const float2 bv = *reinterpret_cast<const float2*>(F1b_b + n);
 #pragma unroll
       for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
         for (int hh = 0; hh < 2; ++hh) {
           const int row = rbase + mt * 16 + g + 8 * hh, m = m0 + row;
-          const float v0 = accm[mt][nt][2 * hh] + accs[mt][nt][2 * hh] + bv.x;
-          const float v1 = accm[mt][nt][2 * hh + 1] + accs[mt][nt][2 * hh + 1] + bv.y;
+          const float v0 = am[mt][nt][2 * hh] + as[mt][nt][2 * hh] + bv.x;
+          const float v1 = am[mt][nt][2 * hh + 1] + as[mt][nt][2 * hh + 1] + bv.y;
           if (m < R) *reinterpret_cast<float2*>(fi + (size_t)m * D + n) = make_float2(v0, v1);
           *reinterpret_cast<float2*>(actA + (size_t)row * LDA + n) = make_float2(v0, v1);
         }
@@ -236,7 +257,7 @@ rlip_chain_mma_kernel(const float* __restrict__ emb, const float* __restrict__ F
   for (int c = 0; c < D / 64; ++c) {
     zero_acc<4>(accm, accs);
     const int nrow[4] = {wn * 16, wn * 16 + 8, 64 + wn * 16, 64 + wn * 16 + 8};
-    const int q0 = NC1 + NC2 + c * NC1;
+    const int q0 = NC1 + C::G2 * NC2 + c * NC1;
 #pragma unroll 1
     for (int q = q0; q < q0 + NC1; ++q) {
       const float* Ws = advance(q);
@@ -289,26 +310,27 @@ rlip_chain_mma_kernel(const float* __restrict__ emb, const float* __restrict__ F
       }
   }
   __syncthreads();
-  if (tid < 2 * TM) {
+  static_assert(C::NB * TM <= THREADS, "one thread per (gate block, region)");
+  if (tid < C::NB * TM) {
     const int c = tid / TM, row = tid % TM, m = m0 + row;
     const float* rp = red + (size_t)c * 4 * TM + row;
     if (m < R) part[(size_t)c * R + m] = (rp[0] + rp[TM]) + (rp[2 * TM] + rp[3 * TM]);
   }
 }
 
-template <int WM, int KC>
+template <int D, int WM, int KC>
 static int launch_chain_mma(const float* emb, const AdvmilDiscParams& p, int R, const Drop& dfc1, const Drop& dga, const Drop& dgs,
                             float* f1, float* fi, float* ab, float* part, cudaStream_t st) {
-  using C = Cfg<WM, KC>;
+  using C = Cfg<D, WM, KC>;
   const size_t smem = C::SMEM_FLOATS * sizeof(float);
   static bool attr_set[64] = {};
   int dev = 0;
   ADVMIL_CHECK_CUDA(cudaGetDevice(&dev));
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(rlip_chain_mma_kernel<WM, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(rlip_chain_mma_kernel<D, WM, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
   }
-  launch_k(rlip_chain_mma_kernel<WM, KC>, dim3(cdiv(R, C::TM)), dim3(C::THREADS), smem, st, emb, p.F1a_w, p.F1a_b, p.F1b_w, p.F1b_b,
+  launch_k(rlip_chain_mma_kernel<D, WM, KC>, dim3(cdiv(R, C::TM)), dim3(C::THREADS), smem, st, emb, p.F1a_w, p.F1a_b, p.F1b_w, p.F1b_b,
            p.Pg_w, p.Pg_b, p.Ps_w, p.Ps_b, p.Pc_w, R, dfc1, dga, dgs, f1, fi, ab, part);
   ADVMIL_CHECK_LAUNCH();
   return ADVMIL_OK;
@@ -317,18 +339,25 @@ static int launch_chain_mma(const float* emb, const AdvmilDiscParams& p, int R, 
 
 }  // namespace
 
-bool rlip_chain_supported(int d) { return d == CH_D; }
+bool rlip_chain_supported(int d) { return d == 64 || d == 128 || d == 256; }
 
 int rlip_chain_fwd(const float* emb, const AdvmilDiscParams& p, int R, const Drop& dfc1, const Drop& dga, const Drop& dgs,
                    float* f1, float* fi, float* ab, float* part, cudaStream_t st) {
-  ADVMIL_REQUIRE(p.d == CH_D, "rlip_chain_fwd: d=%d unsupported", p.d);
+  ADVMIL_REQUIRE(rlip_chain_supported(p.d), "rlip_chain_fwd: d=%d unsupported (64, 128 or 256)", p.d);
   if (R == 0) return ADVMIL_OK;
   // 64-region CTAs while they fit one wave of 2 CTAs per SM (R = 16384: 46 us against 49 us), 32-region CTAs with 16-deep
   // weight stages (4 CTAs per SM) beyond that (the batched real + fake launch, 2R = 32768: 86 us against 91 us)
   static int sms = 0;
   if (!sms) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); if (sms <= 0) sms = 148; }
-  if (cdiv(R, 64) <= 2 * sms) return mm::launch_chain_mma<2, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
-  return mm::launch_chain_mma<1, 16>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
+  // d = 64: the same choice with 32-deep stages (a 16-deep stage of the 32-row F1a chunk does not divide over 256 threads);
+  // d = 256: 32-region CTAs only (a 64-region CTA needs 138 KB of shared memory: one per SM)
+  if (p.d == 64) {
+    if (cdiv(R, 64) <= 2 * sms) return mm::launch_chain_mma<64, 2, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
+    return mm::launch_chain_mma<64, 1, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
+  }
+  if (p.d == 256) return mm::launch_chain_mma<256, 1, 16>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
+  if (cdiv(R, 64) <= 2 * sms) return mm::launch_chain_mma<128, 2, 32>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
+  return mm::launch_chain_mma<128, 1, 16>(emb, p, R, dfc1, dga, dgs, f1, fi, ab, part, st);
 }
 
 }  // namespace advmil

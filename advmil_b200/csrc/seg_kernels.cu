@@ -719,10 +719,11 @@ int pool_gate_bwd(const void* v, const float* w, const float* z, const float* dz
 // =============================================================================================
 // K5/K6 backward per row: region mean (1/16), ReLU, LayerNorm (biased variance, eps) -> d_y
 // =============================================================================================
-template <int VPL>  // values per lane: d <= 32*VPL
+// T = element type of y_pre / d_y (fp32, or bf16 at d = 64 and 256; d = 128 has its own kernel below)
+template <typename T, int VPL>  // values per lane: d <= 32*VPL
 __global__ void __launch_bounds__(256) ln_pool_bwd_kernel(
-    const float* __restrict__ y_pre, const float* __restrict__ d_emb, const float* __restrict__ d_emb2,
-    const float* __restrict__ gamma, const float* __restrict__ beta, int rows, int d, float eps, float* __restrict__ d_y,
+    const T* __restrict__ y_pre, const float* __restrict__ d_emb, const float* __restrict__ d_emb2,
+    const float* __restrict__ gamma, const float* __restrict__ beta, int rows, int d, float eps, T* __restrict__ d_y,
     float* __restrict__ part /*[chunks][3][d]*/) {
   pdl_prologue();
   extern __shared__ float sm[];  // [8 warps][3][d]
@@ -743,7 +744,7 @@ __global__ void __launch_bounds__(256) ln_pool_bwd_kernel(
     float y[VPL];
     float s = 0.f;
 #pragma unroll
-    for (int k = 0; k < VPL; ++k) { int c = lane + 32 * k; y[k] = c < d ? y_pre[row * d + c] : 0.f; s += y[k]; }
+    for (int k = 0; k < VPL; ++k) { int c = lane + 32 * k; y[k] = c < d ? ld1(y_pre + row * d + c) : 0.f; s += y[k]; }
     float mean = warp_sum(s) * inv_d;
     float q = 0.f;
 #pragma unroll
@@ -772,7 +773,7 @@ __global__ void __launch_bounds__(256) ln_pool_bwd_kernel(
       int c = lane + 32 * k;
       if (c < d) {
         float dy = rstd * (dxh[k] - m1 - xh[k] * m2);
-        d_y[row * d + c] = dy;
+        st1(d_y + row * d + c, dy);
         pbias[k] += dy;
       }
     }
@@ -918,15 +919,19 @@ int ln_pool_bwd(const void* y_pre, const float* d_emb, const float* d_emb2, cons
                 int d, float eps, void* d_y, float* dgamma, float* dbeta, float* dbias, int accumulate, float* ws, int dt,
                 cudaStream_t st) {
   ADVMIL_REQUIRE(d <= 256, "ln_pool_bwd: d %d > 256 unsupported", d);
-  ADVMIL_REQUIRE(dt == ELEM_F32 || d == 128, "ln_pool_bwd: the bf16 mode supports d == 128 only (d=%d)", d);
+  ADVMIL_REQUIRE(dt == ELEM_F32 || d == 64 || d == 128 || d == 256, "ln_pool_bwd: the bf16 mode supports d = 64, 128 and 256 only (d=%d)", d);
   int chunks = row_chunks(rows);
   size_t smem = (size_t)8 * 3 * d * sizeof(float);
   if (d == 128 && dt == ELEM_BF16)      // 96 registers (32 bytes of spills), 5 CTAs per SM: 58 -> 56 us
     launch_k(ln_pool_bwd128_kernel<bf16, 5>, dim3(chunks), dim3(128), 0, st, (const bf16*)y_pre, d_emb, d_emb2, gamma, beta, rows, eps, (bf16*)d_y, ws);
   else if (d == 128)
     launch_k(ln_pool_bwd128_kernel<float, 4>, dim3(chunks), dim3(128), 0, st, (const float*)y_pre, d_emb, d_emb2, gamma, beta, rows, eps, (float*)d_y, ws);
-  else if (d <= 128) launch_k(ln_pool_bwd_kernel<4>, dim3(chunks), dim3(256), smem, st, (const float*)y_pre, d_emb, d_emb2, gamma, beta, rows, d, eps, (float*)d_y, ws);
-  else launch_k(ln_pool_bwd_kernel<8>, dim3(chunks), dim3(256), smem, st, (const float*)y_pre, d_emb, d_emb2, gamma, beta, rows, d, eps, (float*)d_y, ws);
+  else if (dt == ELEM_BF16 && d == 64)
+    launch_k(ln_pool_bwd_kernel<bf16, 2>, dim3(chunks), dim3(256), smem, st, (const bf16*)y_pre, d_emb, d_emb2, gamma, beta, rows, d, eps, (bf16*)d_y, ws);
+  else if (dt == ELEM_BF16)
+    launch_k(ln_pool_bwd_kernel<bf16, 8>, dim3(chunks), dim3(256), smem, st, (const bf16*)y_pre, d_emb, d_emb2, gamma, beta, rows, d, eps, (bf16*)d_y, ws);
+  else if (d <= 128) launch_k(ln_pool_bwd_kernel<float, 4>, dim3(chunks), dim3(256), smem, st, (const float*)y_pre, d_emb, d_emb2, gamma, beta, rows, d, eps, (float*)d_y, ws);
+  else launch_k(ln_pool_bwd_kernel<float, 8>, dim3(chunks), dim3(256), smem, st, (const float*)y_pre, d_emb, d_emb2, gamma, beta, rows, d, eps, (float*)d_y, ws);
   ADVMIL_CHECK_LAUNCH();
   ReduceSeg segs[3] = {{ws, 3 * d, d, dgamma, accumulate}, {ws + d, 3 * d, d, dbeta, accumulate}, {ws + 2 * d, 3 * d, d, dbias, accumulate}};
   return reduce_rows_multi(segs, 3, chunks, st);

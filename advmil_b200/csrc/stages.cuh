@@ -43,9 +43,12 @@ int gated_score_fwd(const void* v, const float* Wp, const float* bp, const float
                     int D, const Drop& da, const Drop& db, void* ab, float* s, float* part_ws, int precision,
                     cudaStream_t st);
 // ksize 1: y = x Wc^T + bc (Wc [d, C]); ksize 3: y = 3x3 convolution, zero padded, inside every 4x4 region of 16 rows
-// (Wc [d, C, 3, 3], the Conv2d layout)
+// (Wc [d, C, 3, 3], the Conv2d layout).  d <= 128 (%4) or d == 256; the bf16 mode runs d = 64, 128 and 256 only.
+// y_ws: rows x d floats of scratch for the FFMA path at d = 256 when y_pre is NULL (the LayerNorm there runs as a
+// second pass over y; at every other width the statistics are taken in the GEMM's epilogue)
 int region_embed_fwd(const void* x, const float* Wc, const float* bc, const float* gamma, const float* beta, int rows,
-                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st, int ksize = 1);
+                     int C, int d, float eps, void* y_pre, float* emb, int precision, cudaStream_t st, int ksize = 1,
+                     float* y_ws = nullptr);
 // dX[rows,Nx] = (dY[rows,Ny] . W[Ny,Nx] + pool terms) * relu'  (W row-major [Ny, Nx])
 struct BwdDataExtras {
   const float* w = nullptr; const float* dz = nullptr; const float* dmean = nullptr;
@@ -83,7 +86,8 @@ int cluster_pool_bwd(const float* d_hc, const uint32_t* keep, const int32_t* cid
                      int rows, int bags, int h, int ncl, int precision, void* d_hx, cudaStream_t st);
 
 // ---- rlip_chain.cu ----------------------------------------------------------------------------
-// fc1 MLP + GAPool gate of the RLIP head over R regions in one FFMA kernel (d == 128): writes f1 [R, d/2], fi [R, d],
+// fc1 MLP + GAPool gate of the RLIP head over R regions in one split-tf32 mma.sync kernel (d = 64, 128 or 256): writes
+// f1 [R, d/2], fi [R, d],
 // ab [R, 2d] packed (optional) and the per-64-pair partial logits part [d/64][R] (finished by seg_softmax_pool_fwd)
 bool rlip_chain_supported(int d);
 int rlip_chain_fwd(const float* emb, const AdvmilDiscParams& p, int R, const Drop& dfc1, const Drop& dga, const Drop& dgs,

@@ -174,6 +174,7 @@ static int gen_rlip(const AdvmilStepArgs* a, Workspace& ws, float* d_pred, const
   if (!emb || !head_ok || !d_fake || !d_t || !dws) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
   AdvmilEmbedActs ea{};
   ea.emb = emb; ea.y_pre = nullptr; ea.precision = a->precision;
+  ea.workspace = dws; ea.workspace_bytes = dws_bytes;      // the head forward below reuses it
   ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
   ha.ab = nullptr;      // the G step asks D only for dL/dt: the gate activations are never read back
   ha.emb = emb; ha.t = a->pred_g; ha.out = a->f_fake_g; ha.seed = 0; ha.train = 0; ha.precision = a->precision;

@@ -474,7 +474,11 @@ def disc_embed_forward(cfg: DiscConfig, params, bags: PackedBags, precision: int
             "y_pre": torch.empty(bags.rows, cfg.d, dtype=act_dtype(precision), device=dev) if save else None,
             "precision": int(precision)}
     p = cfg.c(params)
-    a = EmbedActs(acts["emb"].data_ptr(), _ptr(acts["y_pre"]), int(precision), None, 0)
+    # the exact-fp32 FFMA embedding at d = 256 (fp32 mode; tf32 / tf32x3 below one 128-row tile or at C % 32 != 0) runs its
+    # LayerNorm as a second pass over y: scratch for y when y_pre is not kept
+    ffma = int(precision) == FP32 or (int(precision) != BF16 and (bags.rows < 128 or cfg.C % 32 != 0))
+    ws = torch.empty(bags.rows * cfg.d * 4, dtype=torch.uint8, device=dev) if not save and cfg.d > 128 and ffma else None
+    a = EmbedActs(acts["emb"].data_ptr(), _ptr(acts["y_pre"]), int(precision), _ptr(ws), 0 if ws is None else ws.numel())
     b = bags.c()
     check(lib.advmil_disc_embed_fwd(C.byref(p), C.byref(b), C.byref(a), _stream()), "advmil_disc_embed_fwd")
     return acts

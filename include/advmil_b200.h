@@ -148,6 +148,9 @@ typedef struct AdvmilEmbedActs {      /* K5+K6: region embedding */
   float* emb;    /* [rows/16, d] */
   void* y_pre;   /* T [rows, d] pre-LayerNorm projection, NULL = not saved (no D-param backward) */
   int32_t precision;
+  /* workspace: required by advmil_disc_embed_bwd (advmil_disc_workspace_bytes(p, rows, bags, 1) bytes).  The forward reads
+   * it only on the exact-fp32 FFMA path at d = 256 with y_pre == NULL (fp32 mode, or tf32 / tf32x3 below 128 rows), where
+   * it needs rows * d * 4 bytes for y before the LayerNorm pass; the backward size above covers that. */
   void* workspace; size_t workspace_bytes;
 } AdvmilEmbedActs;
 
