@@ -164,6 +164,7 @@ SYMBOLS = {
     "advmil_adv_step_workspace_bytes": (_sz, [_P(GenParams), _P(DiscParams), _i32, _i32, _i32]),
     "advmil_adv_step_disc": (C.c_int, [_P(StepArgs), _vp]),
     "advmil_adv_step_gen": (C.c_int, [_P(StepArgs), _vp]),
+    "advmil_adv_step_gen_next": (C.c_int, [_P(StepArgs), _vp]),
     "advmil_seg_pool_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "advmil_region_index_map": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),
     "advmil_region_of_rows": (C.c_int, [_i32, _i32, _vp, _vp]),
@@ -178,9 +179,11 @@ SYMBOLS = {
     "advmil_adv_step_esat_workspace_bytes": (_sz, [_P(EsatParams), _P(GenParams), _P(DiscParams), _i32, _i32, _i32]),
     "advmil_adv_step_esat_disc": (C.c_int, [_P(EsatStepArgs), _vp]),
     "advmil_adv_step_esat_gen": (C.c_int, [_P(EsatStepArgs), _vp]),
+    "advmil_adv_step_esat_gen_next": (C.c_int, [_P(EsatStepArgs), _vp]),
     "advmil_adv_step_cluster_workspace_bytes": (_sz, [_P(GenParams), _P(DiscParams), _i32, _i32, _i32, _i32]),
     "advmil_adv_step_cluster_disc": (C.c_int, [_P(ClusterStepArgs), _vp]),
     "advmil_adv_step_cluster_gen": (C.c_int, [_P(ClusterStepArgs), _vp]),
+    "advmil_adv_step_cluster_gen_next": (C.c_int, [_P(ClusterStepArgs), _vp]),
     "advmil_cluster_pool_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
     "advmil_cluster_pool_fwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _P(C.c_int32), _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp,
                                           _vp, _sz, _vp]),

@@ -1,5 +1,7 @@
 // Fused adversarial step: the launch sequence of one D update + one G update (model/model_handler.py:349-498) issued from
-// C in two host calls (advmil_adv_step_disc / advmil_adv_step_gen) over one caller-owned workspace.
+// C in two host calls (advmil_adv_step_disc / advmil_adv_step_gen) over one caller-owned workspace.  gen_updates > 1 (more
+// G updates per D update, model/model_handler.py:328-335): advmil_adv_step_gen_next runs each further G update on the same
+// workspace; the G phase is one function (gen_phase) with a `first` flag.
 //
 //  * real and fake pairs of the D step share one region-embedding pass and run through ONE batched RLIP head pass: the
 //    head sees 2 x bags "virtual bags" (fake pairs first, then real pairs) over a duplicated [2R, d] embedding;
@@ -101,9 +103,11 @@ static size_t disc_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb,
 }
 static size_t gen_part_bytes(const AdvmilDiscParams* d, size_t rows, size_t nb) {
   const size_t R = rows / 16;
-  return align_up(R * d->d * sizeof(float), 256) + head_bytes(*d, R, nb) + 8 * 256 + 4 * nb * sizeof(float) +
-         advmil_disc_workspace_bytes(d, rows, nb, 1) + 256;
+  return head_bytes(*d, R, nb) + 8 * 256 + 4 * nb * sizeof(float) + advmil_disc_workspace_bytes(d, rows, nb, 1) + 256;
 }
+// D's region embedding of x for the G phase, [R, d] fp32: a persistent slot of every step's workspace.  D does not change
+// between the G updates of one step, so the first G update writes it and the later ones read it back.
+static size_t gen_emb_bytes(const AdvmilDiscParams* d, size_t rows) { return align_up(rows / 16 * d->d * sizeof(float), 256); }
 // D phase, region embedding: ea.emb has room for the [2R, d] copy that disc_rlip duplicates for the batched head.  With
 // run == false the caller writes ea.emb / ea.y_pre itself (the ABMIL step: fused with its projection, or after its forward).
 static int disc_embed(const AdvmilStepArgs* a, Workspace& ws, bool run, AdvmilEmbedActs& ea, const char* who, cudaStream_t st) {
@@ -159,23 +163,26 @@ static int disc_rlip(const AdvmilStepArgs* a, Workspace& ws, AdvmilEmbedActs& ea
   return disc_embed_bwd_impl(&dp, bags, &ea, d_emb2, batched ? d_emb2 + (size_t)R * d : nullptr, a->disc_grads, 0, st);
 }
 // G phase after pred_g exists: D(x, pred_g) with the updated discriminator in eval mode, G loss, and dL/dpred_g (recon +
-// the adversarial term through D) into d_pred [bags]
-static int gen_rlip(const AdvmilStepArgs* a, Workspace& ws, float* d_pred, const char* who, cudaStream_t st) {
+// the adversarial term through D) into d_pred [bags].  emb: the persistent [R, d] slot of D's region embedding, computed
+// here unless emb_ready (a later G update of the same step).
+static int gen_rlip(const AdvmilStepArgs* a, Workspace& ws, float* emb, bool emb_ready, float* d_pred, const char* who,
+                    cudaStream_t st) {
   const AdvmilDiscParams& dp = *a->disc;
   const AdvmilBags* bags = a->bags;
-  const int rows = bags->rows, nb = bags->bags, R = rows / 16, d = dp.d;
-  float* emb = ws.take<float>((size_t)R * d);
+  const int rows = bags->rows, nb = bags->bags, R = rows / 16;
   AdvmilHeadActs ha{};
   const bool head_ok = take_head(ws, dp, R, nb, ha);
   float* d_fake = ws.take<float>(nb);
   float* d_t = ws.take<float>(nb);
   const size_t dws_bytes = advmil_disc_workspace_bytes(&dp, rows, nb, 1);
   char* dws = ws.take<char>(dws_bytes);
-  if (!emb || !head_ok || !d_fake || !d_t || !dws) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
-  AdvmilEmbedActs ea{};
-  ea.emb = emb; ea.y_pre = nullptr; ea.precision = a->precision;
-  ea.workspace = dws; ea.workspace_bytes = dws_bytes;      // the head forward below reuses it
-  ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
+  if (!head_ok || !d_fake || !d_t || !dws) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  if (!emb_ready) {
+    AdvmilEmbedActs ea{};
+    ea.emb = emb; ea.y_pre = nullptr; ea.precision = a->precision;
+    ea.workspace = dws; ea.workspace_bytes = dws_bytes;      // the head forward below reuses it
+    ADVMIL_TRY(advmil_disc_embed_fwd(&dp, bags, &ea, (void*)st));
+  }
   ha.ab = nullptr;      // the G step asks D only for dL/dt: the gate activations are never read back
   ha.emb = emb; ha.t = a->pred_g; ha.out = a->f_fake_g; ha.seed = 0; ha.train = 0; ha.precision = a->precision;
   ha.workspace = dws; ha.workspace_bytes = dws_bytes;
@@ -193,12 +200,12 @@ static int gen_rlip(const AdvmilStepArgs* a, Workspace& ws, float* d_pred, const
 
 using namespace advmil;
 
-// persistent region (same layout in both calls): eval projection and everything the G step's train forward writes (it may
-// run on the side stream while the D phase uses the scratch region)
+// persistent region (same layout in every call): eval projection and everything the G step's train forward writes (it may
+// run on the side stream while the D phase uses the scratch region), and D's region embedding for the G phase
 struct Persist {
-  char* h_eval; char* h; char* ab; GenBufs gb; char* gws; size_t gws_bytes;
+  char* h_eval; char* h; char* ab; GenBufs gb; char* gws; size_t gws_bytes; float* demb;
 };
-static int take_persist(Workspace& ws, const AdvmilGenParams& gp, int rows, int nb, size_t es, Persist& P) {
+static int take_persist(Workspace& ws, const AdvmilGenParams& gp, const AdvmilDiscParams& dp, int rows, int nb, size_t es, Persist& P) {
   const size_t abw = gate_width(gp.h);
   P.h_eval = ws.take<char>((size_t)rows * gp.h * es);
   P.h = ws.take<char>((size_t)rows * gp.h * es);
@@ -206,7 +213,8 @@ static int take_persist(Workspace& ws, const AdvmilGenParams& gp, int rows, int 
   const bool ok = take_gen(ws, gp, rows, nb, P.gb);
   P.gws_bytes = advmil_generator_workspace_bytes(&gp, rows, nb, 1);
   P.gws = ws.take<char>(P.gws_bytes);
-  if (!P.h_eval || !P.h || !P.ab || !ok || !P.gws) { set_error("adv_step: workspace too small (have %zu bytes)", ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  P.demb = ws.take<float>((size_t)(rows / 16) * dp.d);
+  if (!P.h_eval || !P.h || !P.ab || !ok || !P.gws || !P.demb) { set_error("adv_step: workspace too small (have %zu bytes)", ws.cap); return ADVMIL_ERR_WORKSPACE; }
   return ADVMIL_OK;
 }
 static void fill_train_acts(const AdvmilStepArgs* a, const Persist& P, AdvmilGenActs& ga) {
@@ -223,7 +231,7 @@ extern "C" size_t advmil_adv_step_workspace_bytes(const AdvmilGenParams* g, cons
   const size_t es = elem_bytes(elem_of_precision(precision));
   const size_t nb = bags, abw = gate_width(g->h);
   size_t persistent = 2 * align_up((size_t)rows * g->h * es, 256) + align_up((size_t)rows * abw * es, 256) + gen_bufs_bytes(*g, rows, nb) +
-                      advmil_generator_workspace_bytes(g, rows, bags, 1) + 2048;
+                      advmil_generator_workspace_bytes(g, rows, bags, 1) + gen_emb_bytes(d, rows) + 2048;
   size_t disc = gen_bufs_bytes(*g, rows, nb) + advmil_generator_workspace_bytes(g, rows, bags, 0) + 256 + disc_part_bytes(d, rows, nb, precision);
   size_t gen = gen_part_bytes(d, rows, nb);
   return persistent + (disc > gen ? disc : gen) + 4096;
@@ -248,7 +256,7 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   const size_t es = elem_bytes(elem_of_precision(a->precision));
   Workspace ws(a->workspace, a->workspace_bytes);
   Persist P;
-  ADVMIL_TRY(take_persist(ws, gp, rows, nb, es, P));
+  ADVMIL_TRY(take_persist(ws, gp, dp, rows, nb, es, P));
   char* h_eval = P.h_eval;
   std::lock_guard<std::mutex> side_lock(g_side_mu);
   SideState* side = nullptr;
@@ -300,20 +308,22 @@ extern "C" int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream) {
   return disc_rlip(a, ws, ea, __func__, st);
 }
 
-extern "C" int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream) {
+// One G update (model_handler.py:432-498 up to the caller's Adam step).  first: the update after the D phase, which reuses
+// the dropped projection of the disc call (side stream or not); a later update recomputes K1 from G's current parameters.
+static int gen_phase(const AdvmilStepArgs* a, bool first, const char* who, cudaStream_t st) {
   ADVMIL_TRY(step_check(a));
-  ADVMIL_REQUIRE(a->gen_grads && a->pred_g && a->f_fake_g, "adv_step_gen: missing output buffers");
-  cudaStream_t st = (cudaStream_t)stream;
+  ADVMIL_REQUIRE(a->gen_grads && a->pred_g && a->f_fake_g, "%s: missing output buffers", who);
   const AdvmilGenParams& gp = *a->gen;
   const AdvmilBags* bags = a->bags;
   const int rows = bags->rows, nb = bags->bags;
   const size_t es = elem_bytes(elem_of_precision(a->precision));
   Workspace ws(a->workspace, a->workspace_bytes);
   Persist P;                                                  // h_eval was written by advmil_adv_step_disc on this workspace
-  ADVMIL_TRY(take_persist(ws, gp, rows, nb, es, P));
-  // ---- generator, train mode, on the cached eval projection: join the side stream, or run it here ----
+  ADVMIL_TRY(take_persist(ws, gp, *a->disc, rows, nb, es, P));
+  // ---- generator, train mode: join the side stream's forward on the cached eval projection, or run it here ----
   AdvmilGenActs ga;
   fill_train_acts(a, P, ga);
+  if (!first) ga.h_ready = 0;        // K1 with this update's dropout: G's parameters moved at the previous update
   std::unique_lock<std::mutex> side_lock(g_side_mu);
   SideState* side = nullptr;
   ADVMIL_TRY(side_get(&side));
@@ -321,15 +331,21 @@ extern "C" int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream) {
   if (slot >= 0) {
     ADVMIL_CHECK_CUDA(cudaStreamWaitEvent(st, side->done[slot], 0));
     side->pending_ws[slot] = nullptr;
-    side_lock.unlock();
-  } else {
-    side_lock.unlock();
-    ADVMIL_TRY(advmil_generator_fwd(&gp, bags, &ga, stream));
   }
+  side_lock.unlock();
+  if (slot < 0 || !first) ADVMIL_TRY(advmil_generator_fwd(&gp, bags, &ga, (void*)st));
   // ---- D(x, pred_g) with the updated discriminator, G loss, dL/dpred_g ----
-  STEP_TAKE(d_pred, float, nb);
-  ADVMIL_TRY(gen_rlip(a, ws, d_pred, __func__, st));
-  return advmil_generator_bwd(&gp, bags, &ga, d_pred, a->gen_grads, stream);
+  float* d_pred = ws.take<float>(nb);
+  if (!d_pred) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  ADVMIL_TRY(gen_rlip(a, ws, P.demb, !first, d_pred, who, st));
+  return advmil_generator_bwd(&gp, bags, &ga, d_pred, a->gen_grads, (void*)st);
+}
+
+extern "C" int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream) {
+  return gen_phase(a, true, __func__, (cudaStream_t)stream);
+}
+extern "C" int advmil_adv_step_gen_next(const AdvmilStepArgs* a, void* stream) {
+  return gen_phase(a, false, __func__, (cudaStream_t)stream);
 }
 
 
@@ -345,12 +361,14 @@ namespace advmil {
 struct EsatBufs {
   char* y_pre; float *emb, *qkv, *lse, *ctx, *s1, *x1, *f, *s2, *x2, *ab, *rep, *attn, *H, *H1, *pre;
   char* ews; size_t ews_bytes;
+  float* demb;      // D's region embedding for the G phase
 };
 static size_t esat_acts_bytes(const AdvmilEsatParams& p, const AdvmilGenParams& h, size_t rows, size_t nb, size_t es) {
   const size_t R = rows / 16, d = p.d, abw = gate_width(p.d);
   return align_up(rows * d * es, 256) + (R * (d * 9 + p.ff + abw + 2) + (size_t)p.nhead * R + nb * (d + h.hid + 1)) * sizeof(float) + 20 * 256;
 }
-static int take_esat(Workspace& ws, const AdvmilEsatParams& p, const AdvmilGenParams& h, int rows, int nb, size_t es, EsatBufs& b) {
+static int take_esat(Workspace& ws, const AdvmilEsatParams& p, const AdvmilGenParams& h, const AdvmilDiscParams& dp, int rows, int nb,
+                     size_t es, EsatBufs& b) {
   const size_t R = rows / 16, d = p.d, abw = gate_width(p.d);
   b.y_pre = ws.take<char>((size_t)rows * d * es);
   b.emb = ws.take<float>(R * d); b.qkv = ws.take<float>(R * 3 * d); b.lse = ws.take<float>((size_t)p.nhead * R); b.ctx = ws.take<float>(R * d);
@@ -360,8 +378,9 @@ static int take_esat(Workspace& ws, const AdvmilEsatParams& p, const AdvmilGenPa
   const size_t e0 = advmil_esat_workspace_bytes(&p, &h, rows, nb, 0), e1 = advmil_esat_workspace_bytes(&p, &h, rows, nb, 1);
   b.ews_bytes = e0 > e1 ? e0 : e1;
   b.ews = ws.take<char>(b.ews_bytes);
+  b.demb = ws.take<float>(R * dp.d);
   if (!b.y_pre || !b.emb || !b.qkv || !b.lse || !b.ctx || !b.s1 || !b.x1 || !b.f || !b.s2 || !b.x2 || !b.ab || !b.rep || !b.attn || !b.H ||
-      !b.H1 || !b.pre || !b.ews) {
+      !b.H1 || !b.pre || !b.ews || !b.demb) {
     set_error("adv_step_esat: workspace too small (have %zu bytes)", ws.cap);
     return ADVMIL_ERR_WORKSPACE;
   }
@@ -401,7 +420,7 @@ extern "C" size_t advmil_adv_step_esat_workspace_bytes(const AdvmilEsatParams* g
   const size_t es = elem_bytes(elem_of_precision(precision));
   const size_t nb = bags;
   const size_t e0 = advmil_esat_workspace_bytes(g, head, rows, bags, 0), e1 = advmil_esat_workspace_bytes(g, head, rows, bags, 1);
-  size_t persistent = esat_acts_bytes(*g, *head, rows, nb, es) + (e0 > e1 ? e0 : e1) + 256;
+  size_t persistent = esat_acts_bytes(*g, *head, rows, nb, es) + (e0 > e1 ? e0 : e1) + gen_emb_bytes(d, rows) + 512;
   size_t disc = disc_part_bytes(d, rows, nb, precision), gen = gen_part_bytes(d, rows, nb);
   return persistent + (disc > gen ? disc : gen) + 4096;
 }
@@ -415,7 +434,7 @@ extern "C" int advmil_adv_step_esat_disc(const AdvmilEsatStepArgs* a, void* stre
   const size_t es = elem_bytes(elem_of_precision(a->precision));
   Workspace ws(a->workspace, a->workspace_bytes);
   EsatBufs B;
-  ADVMIL_TRY(take_esat(ws, *a->esat, *a->head, rows, nb, es, B));
+  ADVMIL_TRY(take_esat(ws, *a->esat, *a->head, *a->disc, rows, nb, es, B));
   // ---- generator, eval mode, detached (model_handler.py:383-387) ----
   AdvmilEsatActs ea;
   fill_esat_acts(a, B, 0, ea);
@@ -427,28 +446,38 @@ extern "C" int advmil_adv_step_esat_disc(const AdvmilEsatStepArgs* a, void* stre
   return disc_rlip(&v, ws, da, __func__, st);
 }
 
-extern "C" int advmil_adv_step_esat_gen(const AdvmilEsatStepArgs* a, void* stream) {
+// One G update; first: the update after the D phase, on the patch embedding of the disc call's eval pass.  A later update
+// recomputes the embedding from G's current parameters (emb_ready = 0).
+static int esat_gen_phase(const AdvmilEsatStepArgs* a, bool first, const char* who, cudaStream_t st) {
   ADVMIL_TRY(esat_step_check(a));
-  ADVMIL_REQUIRE(a->esat_grads && a->head_grads && a->pred_g && a->f_fake_g, "adv_step_esat_gen: missing output buffers");
-  cudaStream_t st = (cudaStream_t)stream;
+  ADVMIL_REQUIRE(a->esat_grads && a->head_grads && a->pred_g && a->f_fake_g, "%s: missing output buffers", who);
   const AdvmilBags* bags = a->bags;
   const int rows = bags->rows, nb = bags->bags;
   const size_t es = elem_bytes(elem_of_precision(a->precision));
   Workspace ws(a->workspace, a->workspace_bytes);
   EsatBufs B;                                      // y_pre / emb were written by advmil_adv_step_esat_disc on this workspace
-  ADVMIL_TRY(take_esat(ws, *a->esat, *a->head, rows, nb, es, B));
-  // ---- generator, train mode, on the cached patch embedding ----
+  ADVMIL_TRY(take_esat(ws, *a->esat, *a->head, *a->disc, rows, nb, es, B));
+  // ---- generator, train mode ----
   AdvmilEsatActs ea;
   fill_esat_acts(a, B, 1, ea);
-  ADVMIL_TRY(advmil_esat_fwd(a->esat, a->head, bags, &ea, stream));
+  ea.emb_ready = first;
+  ADVMIL_TRY(advmil_esat_fwd(a->esat, a->head, bags, &ea, (void*)st));
   // ---- D(x, pred_g) with the updated discriminator, G loss, dL/dpred_g ----
-  STEP_TAKE(d_pred, float, nb);
+  float* d_pred = ws.take<float>(nb);
+  if (!d_pred) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
   const AdvmilStepArgs v = rlip_args(a);
-  ADVMIL_TRY(gen_rlip(&v, ws, d_pred, __func__, st));
+  ADVMIL_TRY(gen_rlip(&v, ws, B.demb, !first, d_pred, who, st));
   esat_request_overlap(1);     // weight / bias gradients of the region-level layers on the backward side stream
-  const int rc = advmil_esat_bwd(a->esat, a->head, bags, &ea, d_pred, a->esat_grads, a->head_grads, stream);
+  const int rc = advmil_esat_bwd(a->esat, a->head, bags, &ea, d_pred, a->esat_grads, a->head_grads, (void*)st);
   esat_request_overlap(0);
   return rc;
+}
+
+extern "C" int advmil_adv_step_esat_gen(const AdvmilEsatStepArgs* a, void* stream) {
+  return esat_gen_phase(a, true, __func__, (cudaStream_t)stream);
+}
+extern "C" int advmil_adv_step_esat_gen_next(const AdvmilEsatStepArgs* a, void* stream) {
+  return esat_gen_phase(a, false, __func__, (cudaStream_t)stream);
 }
 
 
@@ -470,7 +499,7 @@ __global__ void iota_scaled_kernel(int n, int step, int32_t* __restrict__ out) {
   if (i <= n) out[i] = i * step;
 }
 
-struct ClusterBufs { float* hc; int32_t* counts; uint32_t* keep; char* hx; int32_t* hoffs; };
+struct ClusterBufs { float* hc; int32_t* counts; uint32_t* keep; char* hx; int32_t* hoffs; float* demb; };
 static size_t cluster_persist_bytes(int rows, int nb, int C, int h, int ncl, int precision) {
   const size_t nbc = (size_t)nb * ncl;
   const size_t act = cluster_pool_fused(rows, C, h, precision) ? (size_t)rows * (h / 32) * sizeof(uint32_t)
@@ -478,7 +507,7 @@ static size_t cluster_persist_bytes(int rows, int nb, int C, int h, int ncl, int
   return align_up(nbc * h * sizeof(float), 256) + align_up(nbc * sizeof(int32_t), 256) + align_up(act, 256) +
          align_up((nb + 1) * sizeof(int32_t), 256) + 4 * 256;
 }
-static int take_cluster(Workspace& ws, int rows, int nb, int C, int h, int ncl, int precision, ClusterBufs& B) {
+static int take_cluster(Workspace& ws, const AdvmilDiscParams& dp, int rows, int nb, int C, int h, int ncl, int precision, ClusterBufs& B) {
   const size_t nbc = (size_t)nb * ncl;
   B = ClusterBufs{};
   B.hc = ws.take<float>(nbc * h);
@@ -486,7 +515,8 @@ static int take_cluster(Workspace& ws, int rows, int nb, int C, int h, int ncl, 
   if (cluster_pool_fused(rows, C, h, precision)) B.keep = ws.take<uint32_t>((size_t)rows * (h / 32));
   else B.hx = ws.take<char>((size_t)rows * h * elem_bytes(elem_of_precision(precision)));
   B.hoffs = ws.take<int32_t>(nb + 1);
-  if (!B.hc || !B.counts || !(B.keep || B.hx) || !B.hoffs) { set_error("adv_step_cluster: workspace too small (have %zu bytes)", ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  B.demb = ws.take<float>((size_t)(rows / 16) * dp.d);
+  if (!B.hc || !B.counts || !(B.keep || B.hx) || !B.hoffs || !B.demb) { set_error("adv_step_cluster: workspace too small (have %zu bytes)", ws.cap); return ADVMIL_ERR_WORKSPACE; }
   return ADVMIL_OK;
 }
 // packed view of hc: num_clusters fp32 rows of width h per bag
@@ -497,6 +527,30 @@ static AdvmilBags cluster_bags(const ClusterBufs& B, int nb, int ncl, int h, std
   cb.x = B.hc; cb.offsets = B.hoffs; cb.offsets_host = offs_host.data();
   cb.rows = nb * ncl; cb.bags = nb; cb.C = h; cb.max_bag_rows = ncl; cb.elem = ELEM_F32;
   return cb;
+}
+// K9: hc, counts and the backward's ReLU keep bits (or relu(x Wphi^T + b) itself) into the persistent region, from the
+// current Wphi / bphi.  Its partials come from the scratch region.
+static size_t cluster_k9_bytes(int rows, int nb, int C, int h, int ncl, int precision) {
+  return cluster_pool_fused(rows, C, h, precision) ? align_up(cluster_pool_ws_floats(rows, nb, h, ncl) * sizeof(float), 256)
+                                                   : advmil_segment_mean_workspace_bytes(rows, nb, h, ncl) + 256;
+}
+static int cluster_k9(const AdvmilClusterStepArgs* ca, Workspace& ws, const ClusterBufs& B, const char* who, cudaStream_t st) {
+  const AdvmilBags* bags = ca->base.bags;
+  const int rows = bags->rows, nb = bags->bags, C = bags->C, h = ca->base.gen->h, ncl = ca->num_clusters, prec = ca->base.precision;
+  if (cluster_pool_fused(rows, C, h, prec)) {
+    float* part = ws.take<float>(cluster_pool_ws_floats(rows, nb, h, ncl));
+    if (!part) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
+    ProfScope ps(PROF_PROJ_SEGMEAN, st);
+    return cluster_pool_fwd(bags->x, ca->Wphi, ca->bphi, ca->cid, bags->offsets, bags->offsets_host, rows, nb, C, h, ncl, prec,
+                            B.hc, B.counts, B.keep, part, st);
+  }
+  const size_t sm_bytes = advmil_segment_mean_workspace_bytes(rows, nb, h, ncl);
+  char* smws = ws.take<char>(sm_bytes);
+  if (!smws) { set_error("%s: workspace too small (have %zu bytes)", who, ws.cap); return ADVMIL_ERR_WORKSPACE; }
+  Drop none = Drop::make(nullptr, 0, 0, 0.f, 0, 0);
+  { ProfScope ps(PROF_PROJ, st); ADVMIL_TRY(linear_fwd(bags->x, ca->Wphi, ca->bphi, rows, C, h, 1, none, B.hx, prec, st)); }
+  return advmil_segment_mean_by_id_fwd(B.hx, elem_of_precision(prec), ca->cid, bags->offsets, bags->offsets_host, rows, nb, h, ncl,
+                                       B.hc, B.counts, smws, sm_bytes, (void*)st);
 }
 static int cluster_step_check(const AdvmilClusterStepArgs* ca) {
   ADVMIL_REQUIRE(ca, "adv_step_cluster: null argument");
@@ -523,13 +577,11 @@ extern "C" size_t advmil_adv_step_cluster_workspace_bytes(const AdvmilGenParams*
   const int C = d->C, h = g->h, ncl = num_clusters;
   const size_t nb = bags, nbc = nb * ncl, abw = gate_width(h);
   const size_t es = elem_bytes(elem_of_precision(precision));
-  const bool fused = cluster_pool_fused(rows, C, h, precision);
-  const size_t persistent = cluster_persist_bytes(rows, bags, C, h, ncl, precision);
-  const size_t k9 = fused ? align_up(cluster_pool_ws_floats(rows, bags, h, ncl) * sizeof(float), 256)
-                          : advmil_segment_mean_workspace_bytes(rows, bags, h, ncl) + 256;
+  const size_t persistent = cluster_persist_bytes(rows, bags, C, h, ncl, precision) + gen_emb_bytes(d, rows);
+  const size_t k9 = cluster_k9_bytes(rows, bags, C, h, ncl, precision);      // the disc phase, and every G update after the first
   const size_t disc = k9 + gen_bufs_bytes(*g, nbc, nb) + align_up(nbc * h * sizeof(float), 256) +
                       advmil_generator_workspace_bytes(g, (int)nbc, bags, 0) + 256 + disc_part_bytes(d, rows, nb, precision);
-  const size_t gen = gen_bufs_bytes(*g, nbc, nb) + align_up(nbc * h * sizeof(float), 256) + align_up(nbc * abw * sizeof(float), 256) +
+  const size_t gen = k9 + gen_bufs_bytes(*g, nbc, nb) + align_up(nbc * h * sizeof(float), 256) + align_up(nbc * abw * sizeof(float), 256) +
                      advmil_generator_workspace_bytes(g, (int)nbc, bags, 1) + 256 + align_up(nb * sizeof(float), 256) +
                      align_up(nbc * h * sizeof(float), 256) + align_up((size_t)rows * h * es, 256) +
                      align_up(bwd_weight_ws_floats(rows, h, C) * sizeof(float), 256) + align_up((size_t)row_chunks(rows) * h * sizeof(float), 256) +
@@ -549,21 +601,9 @@ extern "C" int advmil_adv_step_cluster_disc(const AdvmilClusterStepArgs* ca, voi
   ADVMIL_REQUIRE(C == a->disc->C && bags->elem == elem_of_precision(prec), "adv_step_cluster_disc: x width %d / element type do not match", C);
   Workspace ws(a->workspace, a->workspace_bytes);
   ClusterBufs B;
-  ADVMIL_TRY(take_cluster(ws, rows, nb, C, h, ncl, prec, B));
-  // ---- K9 once per step: hc, counts and the backward's ReLU mask stay in the persistent region ----
-  if (cluster_pool_fused(rows, C, h, prec)) {
-    STEP_TAKE(part, float, cluster_pool_ws_floats(rows, nb, h, ncl));
-    ProfScope ps(PROF_PROJ_SEGMEAN, st);
-    ADVMIL_TRY(cluster_pool_fwd(bags->x, ca->Wphi, ca->bphi, ca->cid, bags->offsets, bags->offsets_host, rows, nb, C, h, ncl, prec,
-                                B.hc, B.counts, B.keep, part, st));
-  } else {
-    const size_t sm_bytes = advmil_segment_mean_workspace_bytes(rows, nb, h, ncl);
-    STEP_TAKE(smws, char, sm_bytes);
-    Drop none = Drop::make(nullptr, 0, 0, 0.f, 0, 0);
-    { ProfScope ps(PROF_PROJ, st); ADVMIL_TRY(linear_fwd(bags->x, ca->Wphi, ca->bphi, rows, C, h, 1, none, B.hx, prec, st)); }
-    ADVMIL_TRY(advmil_segment_mean_by_id_fwd(B.hx, elem_of_precision(prec), ca->cid, bags->offsets, bags->offsets_host, rows, nb, h, ncl,
-                                             B.hc, B.counts, smws, sm_bytes, stream));
-  }
+  ADVMIL_TRY(take_cluster(ws, *a->disc, rows, nb, C, h, ncl, prec, B));
+  // ---- K9: hc, counts and the backward's ReLU mask stay in the persistent region for the first G update ----
+  ADVMIL_TRY(cluster_k9(ca, ws, B, __func__, st));
   launch_k(iota_scaled_kernel, dim3(cdiv(nb + 1, 128)), dim3(128), 0, st, nb, ncl, B.hoffs);
   ADVMIL_CHECK_LAUNCH();
   // ---- attention stage, eval mode, detached (model_handler.py:383-387) ----
@@ -584,18 +624,21 @@ extern "C" int advmil_adv_step_cluster_disc(const AdvmilClusterStepArgs* ca, voi
   return disc_rlip(a, ws, ea, __func__, st);
 }
 
-extern "C" int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* ca, void* stream) {
+// One G update; first: the update after the D phase, on the hc of the disc call's K9.  A later update runs K9 again from
+// G's current Wphi / bphi.
+static int cluster_gen_phase(const AdvmilClusterStepArgs* ca, bool first, const char* who, cudaStream_t st) {
   ADVMIL_TRY(cluster_step_check(ca));
   const AdvmilStepArgs* a = &ca->base;
-  ADVMIL_REQUIRE(a->gen_grads && a->pred_g && a->f_fake_g && a->noise_g && ca->dWphi && ca->dbphi, "adv_step_cluster_gen: missing buffers");
-  cudaStream_t st = (cudaStream_t)stream;
+  ADVMIL_REQUIRE(a->gen_grads && a->pred_g && a->f_fake_g && a->noise_g && ca->dWphi && ca->dbphi, "%s: missing buffers", who);
+  void* stream = (void*)st;
   const AdvmilGenParams& gp = *a->gen;
   const AdvmilBags* bags = a->bags;
   const int rows = bags->rows, nb = bags->bags, C = bags->C, h = gp.h, ncl = ca->num_clusters, nbc = nb * ncl;
   const int prec = a->precision, dt = elem_of_precision(prec);
   Workspace ws(a->workspace, a->workspace_bytes);
   ClusterBufs B;                                    // hc / counts / keep bits were written by advmil_adv_step_cluster_disc
-  ADVMIL_TRY(take_cluster(ws, rows, nb, C, h, ncl, prec, B));
+  ADVMIL_TRY(take_cluster(ws, *a->disc, rows, nb, C, h, ncl, prec, B));
+  if (!first) ADVMIL_TRY(cluster_k9(ca, ws, B, who, st));
   // ---- attention stage, train mode, on the same hc ----
   std::vector<int32_t> hoffs_host;
   const AdvmilBags cb = cluster_bags(B, nb, ncl, h, hoffs_host);
@@ -613,7 +656,7 @@ extern "C" int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* ca, void
   ADVMIL_TRY(advmil_generator_fwd(&gp, &cb, &ga, stream));
   // ---- D(x, pred_g), G loss, dL/dpred_g ----
   STEP_TAKE(d_pred, float, nb);
-  ADVMIL_TRY(gen_rlip(a, ws, d_pred, __func__, st));
+  ADVMIL_TRY(gen_rlip(a, ws, B.demb, !first, d_pred, who, st));
   // ---- attention stage backward down to d_hc, then K9's backward and dWphi / dbphi ----
   STEP_TAKE(d_hc, float, (size_t)nbc * h);
   AdvmilGenGrads gg = *a->gen_grads;
@@ -631,4 +674,11 @@ extern "C" int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* ca, void
   STEP_TAKE(csws, float, (size_t)row_chunks(rows) * h);
   { ProfScope ps(PROF_COLSUM, st); ADVMIL_TRY(colsum(d_hx, dt, rows, h, h, ca->dbphi, 0, csws, st)); }
   return ADVMIL_OK;
+}
+
+extern "C" int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* ca, void* stream) {
+  return cluster_gen_phase(ca, true, __func__, (cudaStream_t)stream);
+}
+extern "C" int advmil_adv_step_cluster_gen_next(const AdvmilClusterStepArgs* ca, void* stream) {
+  return cluster_gen_phase(ca, false, __func__, (cudaStream_t)stream);
 }

@@ -1,5 +1,6 @@
-"""Fused adversarial step over packed bags: one D update + one G update, the semantics of
-MyHandler._update_disc + _update_gen (reference model/model_handler.py:349-498), without the handler's redundant work:
+"""Fused adversarial step over packed bags: one D update + `gen_updates` G updates, the semantics of
+MyHandler._update_disc + gen_updates x _update_gen (reference model/model_handler.py:328-335,349-498), without the
+handler's redundant work:
 
   * the D-step generator forward (eval) and the G-step generator forward (train) share the x.W1^T projection
     (G's parameters do not change in between; dropout is applied to the cached eval activations);
@@ -83,6 +84,25 @@ class _DataParallelMixin:
     draws its generator noise from its own CPU generator, so shards do not repeat each other's masks and noise (a single
     process keeps the default generator: the reference's stream, utils/func.py:154-164)."""
 
+    def _init_gen_updates(self, gen_updates):
+        """G updates per D update (config key `gen_updates`, model/model_handler.py:328-335)."""
+        if isinstance(gen_updates, bool) or not isinstance(gen_updates, int) or gen_updates < 1:
+            raise ValueError(f"gen_updates must be an integer >= 1, got {gen_updates!r}")
+        self.gen_updates = gen_updates
+
+    def _per_update(self, v, what):
+        """One value per G update: `v` itself when gen_updates == 1, else a sequence of gen_updates values (None: [None] * k)."""
+        k = self.gen_updates
+        if v is None:
+            return [None] * k
+        if isinstance(v, (list, tuple)):
+            if len(v) != k:
+                raise ValueError(f"{what}: {len(v)} values for gen_updates={k}")
+            return list(v)
+        if k != 1:
+            raise ValueError(f"{what}: gen_updates={k} needs a sequence of {k} values, one per G update")
+        return [v]
+
     def _init_dp(self, process_group):
         self.pg = process_group
         self.world, self.rank = 1, 0
@@ -118,7 +138,7 @@ class _DataParallelMixin:
 class AdvStep(_DataParallelMixin):
     def __init__(self, netG, netD, lr_g=8e-5, lr_d=8e-5, weight_decay_g=5e-4, coef_gan=0.004, coef_l1=1e-5,
                  loss_d="bce", recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32",
-                 process_group=None):
+                 process_group=None, gen_updates=1):
         if netG.backbone.kind != "abmil":
             other = {"cluster": "ClusterAdvStep", "patch": "EsatAdvStep"}.get(netG.backbone.kind, "ModuleAdvStep")
             raise NotImplementedError(f"AdvStep is the C-fused step of the ABMIL generator; use {other} for bcb_mode "
@@ -133,11 +153,12 @@ class AdvStep(_DataParallelMixin):
         self.D = FlatParams(netD, self.dparams, weight_decay_rule=False)
         self.ggrads, self.dgrads = self.G.grads_for(self.gparams), self.D.grads_for(self.dparams)
         self._init_hparams(lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
-                           process_group)
+                           process_group, gen_updates)
 
     def _init_hparams(self, lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
-                      process_group):
-        """Optimiser, loss and precision settings of the C-fused steps; runs after self.G / self.D exist."""
+                      process_group, gen_updates):
+        """Optimiser, loss, precision and schedule settings of the C-fused steps; runs after self.G / self.D exist."""
+        self._init_gen_updates(gen_updates)
         self.lr_g, self.lr_d, self.wd_g = lr_g, lr_d, weight_decay_g
         self.coef_gan, self.coef_l1 = coef_gan, coef_l1
         self.loss_d = {"bce": 0, "hinge": 1, "wasserstein": 2}[loss_d]
@@ -178,9 +199,10 @@ class AdvStep(_DataParallelMixin):
         return bags, t, e, visible, counts
 
     def _noise(self, nb, dev, noise_d, noise_g):
-        """Noise of the D phase's and of the G phase's generator pass, drawn in that order where not given."""
+        """Noise of the D phase's generator pass and of every G update's pass (a list), drawn in that order where not given."""
+        noise_g = self._per_update(noise_g, "noise_g")
         noise_d = (noise_d if noise_d is not None else self._draw(nb, dev)).contiguous().float()
-        noise_g = (noise_g if noise_g is not None else self._draw(nb, dev)).contiguous().float()
+        noise_g = [(n if n is not None else self._draw(nb, dev)).contiguous().float() for n in noise_g]
         return noise_d, noise_g
 
     def _workspace(self, need, dev) -> torch.Tensor:
@@ -190,15 +212,23 @@ class AdvStep(_DataParallelMixin):
             self._ws = ws = torch.empty(int(need * 1.05) + 4096, dtype=torch.uint8, device=dev)
         return ws
 
-    @staticmethod
-    def _outputs(nb, dev) -> Dict:
+    def _outputs(self, nb, dev):
+        """The step's output tensors, and lbuf [gen_updates, 8]: row u holds the loss slots of G update u.  `losses` (the
+        layout of the C ABI: D loss, then the G terms) is the last row, which the D phase writes too.  With gen_updates > 1,
+        gen_losses [gen_updates, 4]: t_reg, gen, t_reg + coef_gan * gen and sum|W_G| of every G update (with one update
+        those are losses[1:5], and the outputs are those of a one-update step as before)."""
         f32 = dict(dtype=torch.float32, device=dev)
-        return {"losses": torch.zeros(8, **f32), "pred_d": torch.empty(nb, **f32), "pred_g": torch.empty(nb, **f32),
-                "f_d": torch.empty(2 * nb, **f32), "f_fake_g": torch.empty(nb, **f32),
-                "real_mask": torch.empty(nb, dtype=torch.uint8, device=dev)}
+        lbuf = torch.zeros(self.gen_updates, 8, **f32)
+        out = {"losses": lbuf[-1], "pred_d": torch.empty(nb, **f32), "pred_g": torch.empty(nb, **f32),
+               "f_d": torch.empty(2 * nb, **f32), "f_fake_g": torch.empty(nb, **f32),
+               "real_mask": torch.empty(nb, dtype=torch.uint8, device=dev)}
+        if self.gen_updates > 1:
+            out["gen_losses"] = lbuf[:, 1:5]
+        return out, lbuf
 
     def _fill_args(self, a, bags, t, e, visible, noise_d, noise_g, counts, out, ws):
-        """The fields that StepArgs and EsatStepArgs share by name (the dropout seeds are drawn here: D's, then G's)."""
+        """The fields that StepArgs and EsatStepArgs share by name (the dropout seeds are drawn here: D's, then the first G
+        update's; noise_g: the first G update's noise)."""
         a.bags = C.pointer(bags.c())
         a.t, a.e, a.visible = t.data_ptr(), e.data_ptr(), visible.data_ptr()
         a.noise_d, a.noise_g = noise_d.data_ptr(), noise_g.data_ptr()
@@ -212,20 +242,28 @@ class AdvStep(_DataParallelMixin):
         a.pred_g, a.f_fake_g = out["pred_g"].data_ptr(), out["f_fake_g"].data_ptr()
         a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
 
-    def _update(self, lib, disc_fn: str, gen_fn: str, args, out, nb, n_real, keep) -> Dict:
-        """The two phases: the library's D call, D all-reduce and Adam, then its G call, L1 value, G all-reduce and Adam.
-        keep: the step's input tensors, alive until the stream is done with them."""
+    def _update(self, lib, disc_fn: str, gen_fn: str, args, a, gen_fields, out, lbuf, nb, n_real, keep) -> Dict:
+        """The library's D call, D all-reduce and Adam, then per G update its G call (`gen_fn`, then `gen_fn`_next), L1 value,
+        G all-reduce and Adam.  a: the AdvmilStepArgs-like fields of `args`; gen_fields: per G update, the fields of `a` that
+        update sets (its noise and injected masks).  keep: the step's input tensors, alive until the stream is done with them."""
         st = torch.cuda.current_stream().cuda_stream
         # ---------------- D step: D.train / G.eval (model_handler.py:355-356) ----------------
         check(getattr(lib, disc_fn)(C.byref(args), st), disc_fn)
         self._allreduce(self.D.grad)
         self.D.adam(self.lr_d)
-        # ---------------- G step: D.eval / G.train (model_handler.py:432-433) ----------------
-        check(getattr(lib, gen_fn)(C.byref(args), st), gen_fn)
-        if self.coef_l1 > 1e-8:
-            check(lib.advmil_abs_sum(self.G.flat.data_ptr(), self.G.total, out["losses"][4:].data_ptr(), st), "advmil_abs_sum")
-        self._allreduce(self.G.grad)
-        self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
+        # ---------------- G steps: D.eval / G.train (model_handler.py:432-433), gen_updates times ----------------
+        for u, fields in enumerate(gen_fields):
+            fn = gen_fn if u == 0 else gen_fn + "_next"
+            if u > 0:
+                for name, v in fields.items():
+                    setattr(a, name, v)
+                a.seed_g = self._seed()
+            a.losses = lbuf[u].data_ptr()
+            check(getattr(lib, fn)(C.byref(args), st), fn)
+            if self.coef_l1 > 1e-8:
+                check(lib.advmil_abs_sum(self.G.flat.data_ptr(), self.G.total, lbuf[u][4:].data_ptr(), st), "advmil_abs_sum")
+            self._allreduce(self.G.grad)
+            self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
         out["f_fake_d"] = out["f_d"][:nb]
         out["f_real"] = out["f_d"][nb:] if n_real > 0 else None
         out["_keep"] = keep
@@ -234,6 +272,12 @@ class AdvStep(_DataParallelMixin):
         # stream -- a caller that drops `out` early cannot hand their memory back to the allocator under the side stream
         self._inflight = out
         return out
+
+    @staticmethod
+    def _gen_fields(noise_g, masks_g, keys):
+        """Per G update: the AdvmilStepArgs fields of its noise and of its injected masks (over `keys`)."""
+        return [dict({"noise_g": n.data_ptr()}, **{"g_mask_" + k: ops._ptr((m or {}).get(k)) for k in keys})
+                for n, m in zip(noise_g, masks_g)]
 
     @staticmethod
     def _cat_masks(fake, real, keys):
@@ -247,26 +291,29 @@ class AdvStep(_DataParallelMixin):
              noise_d: Optional[torch.Tensor] = None, noise_g: Optional[torch.Tensor] = None,
              masks_d_real=None, masks_d_fake=None, masks_g=None, global_counts=None) -> Dict:
         """t, e: [bags] float32 device; visible: [bags] uint8 device (label_visible_mask).  noise_*: [bags, hid] device
-        (drawn like utils/func.generate_noise when None).  Returns device tensors only (no host sync when
-        global_counts is given).  Two C calls (advmil_adv_step_disc / _gen) issue the whole launch sequence."""
+        (drawn like utils/func.generate_noise when None: noise_d, then one draw per G update).  noise_g and masks_g: one
+        value, or a sequence of gen_updates values (one per G update).  Returns device tensors only (no host sync when
+        global_counts is given); losses / pred_g / f_fake_g are those of the last G update; with gen_updates > 1,
+        gen_losses [gen_updates, 4] holds every update's.  One C call per phase (advmil_adv_step_disc / _gen / _gen_next) issues the launch sequence."""
         lib = _lib.load()
         bags, t, e, visible, counts = self._inputs(bags, t, e, visible, global_counts)
         dev, nb = bags.x.device, bags.bags
+        mgs = [m or {} for m in self._per_update(masks_g, "masks_g")]
         noise_d, noise_g = self._noise(nb, dev, noise_d, noise_g)
         gp, dp, gg, dg = self._structs()
         ws = self._workspace(lib.advmil_adv_step_workspace_bytes(C.byref(gp), C.byref(dp), bags.rows, nb, self.precision), dev)
-        out = self._outputs(nb, dev)
+        out, lbuf = self._outputs(nb, dev)
         md = self._cat_masks(masks_d_fake, masks_d_real, ("fc1", "ga", "gs", "fc2"))
-        mg = masks_g or {}
         a = _lib.StepArgs()
         a.gen, a.disc, a.gen_grads, a.disc_grads = C.pointer(gp), C.pointer(dp), C.pointer(gg), C.pointer(dg)
-        for k in ("h", "a", "b", "rho", "mlp0"):
-            setattr(a, "g_mask_" + k, ops._ptr(mg.get(k)))
+        fields = self._gen_fields(noise_g, mgs, ("h", "a", "b", "rho", "mlp0"))
+        for name, v in fields[0].items():
+            setattr(a, name, v)
         for k in ("fc1", "ga", "gs", "fc2"):
             setattr(a, "d_mask_" + k, ops._ptr(md.get(k)))
-        self._fill_args(a, bags, t, e, visible, noise_d, noise_g, counts, out, ws)
-        return self._update(lib, "advmil_adv_step_disc", "advmil_adv_step_gen", a, out, nb, counts[0],
-                            (t, e, visible, noise_d, noise_g, md, mg, bags))
+        self._fill_args(a, bags, t, e, visible, noise_d, noise_g[0], counts, out, ws)
+        return self._update(lib, "advmil_adv_step_disc", "advmil_adv_step_gen", a, a, fields, out, lbuf, nb, counts[0],
+                            (t, e, visible, noise_d, noise_g, md, mgs, bags))
 
     def loss_dict(self, out) -> Dict[str, float]:
         """Host copy of the step's scalars (one sync): the values the handler prints (model_handler.py:413,486-494); under
@@ -285,7 +332,8 @@ class EsatAdvStep(AdvStep):
     embedding, or None (what the handler passes, model_handler.py:613)."""
 
     def __init__(self, netG, netD, lr_g=8e-5, lr_d=8e-5, weight_decay_g=5e-4, coef_gan=0.004, coef_l1=1e-5,
-                 loss_d="bce", recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32", process_group=None):
+                 loss_d="bce", recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32", process_group=None,
+                 gen_updates=1):
         if netG.backbone.kind != "patch":
             raise NotImplementedError(f"EsatAdvStep is the C-fused step of the ESAT generator, got bcb_mode '{netG.backbone.kind}'")
         if list(netG.noise) != [0, 1]:
@@ -299,7 +347,7 @@ class EsatAdvStep(AdvStep):
         self.egrads, self.hgrads, self.dgrads = self.G.grads_for(self.eparams), self.G.grads_for(self.hparams), self.D.grads_for(self.dparams)
         assert self.G.total == sum((t.numel() + 3) // 4 * 4 for t in self.eparams + self.hparams), "generator parameters outside the ESAT step"
         self._init_hparams(lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
-                           process_group)
+                           process_group, gen_updates)
 
     def _structs(self):
         if getattr(self, "_c", None) is None:
@@ -325,13 +373,14 @@ class EsatAdvStep(AdvStep):
         ep, hp, dp, eg, hg, dg = self._structs()
         ws = self._workspace(lib.advmil_adv_step_esat_workspace_bytes(C.byref(ep), C.byref(hp), C.byref(dp), bags.rows, nb,
                                                                       self.precision), dev)
-        out = self._outputs(nb, dev)
+        out, lbuf = self._outputs(nb, dev)
         a = _lib.EsatStepArgs()
         a.esat, a.head, a.disc = C.pointer(ep), C.pointer(hp), C.pointer(dp)
         a.esat_grads, a.head_grads, a.disc_grads = C.pointer(eg), C.pointer(hg), C.pointer(dg)
         a.pe = ops._ptr(pe)
-        self._fill_args(a, bags, t, e, visible, noise_d, noise_g, counts, out, ws)
-        return self._update(lib, "advmil_adv_step_esat_disc", "advmil_adv_step_esat_gen", a, out, nb, counts[0],
+        self._fill_args(a, bags, t, e, visible, noise_d, noise_g[0], counts, out, ws)
+        return self._update(lib, "advmil_adv_step_esat_disc", "advmil_adv_step_esat_gen", a, a,
+                            self._gen_fields(noise_g, [None] * len(noise_g), ()), out, lbuf, nb, counts[0],
                             (t, e, visible, noise_d, noise_g, pe, bags))
 
 
@@ -345,7 +394,8 @@ class ClusterAdvStep(AdvStep):
     injected generator masks are over the attention stage's [bags * num_clusters, h] rows, as in `ModuleAdvStep`."""
 
     def __init__(self, netG, netD, lr_g=8e-5, lr_d=8e-5, weight_decay_g=5e-4, coef_gan=0.004, coef_l1=1e-5,
-                 loss_d="bce", recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32", process_group=None):
+                 loss_d="bce", recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32", process_group=None,
+                 gen_updates=1):
         bb = netG.backbone
         if bb.kind != "cluster":
             raise NotImplementedError(f"ClusterAdvStep is the C-fused step of the DeepAttMISL generator, got bcb_mode '{bb.kind}': "
@@ -367,7 +417,7 @@ class ClusterAdvStep(AdvStep):
         covered = [t for t in self.gparams if t is not None] + [self.Wphi, self.bphi]
         assert self.G.total == sum((t.numel() + 3) // 4 * 4 for t in covered), "generator parameters outside the cluster step"
         self._init_hparams(lr_g, lr_d, weight_decay_g, coef_gan, coef_l1, loss_d, recon_norm, recon_alpha, recon_gamma, precision,
-                           process_group)
+                           process_group, gen_updates)
 
     def step(self, bags: ops.PackedBags, t: torch.Tensor, e: torch.Tensor, visible: torch.Tensor,
              noise_d: Optional[torch.Tensor] = None, noise_g: Optional[torch.Tensor] = None, ext=None,
@@ -381,38 +431,40 @@ class ClusterAdvStep(AdvStep):
         cid = ext.reshape(-1)
         cid = (cid if cid.dtype == torch.int32 else cid.to(torch.int32)).contiguous()
         assert cid.numel() == bags.rows and cid.device == dev, "one cluster id per row, on the bags' device"
+        mgs = [{k: v.contiguous() for k, v in (m or {}).items()} for m in self._per_update(masks_g, "masks_g")]
         noise_d, noise_g = self._noise(nb, dev, noise_d, noise_g)
         gp, dp, gg, dg = self._structs()
         ncl = self.netG.backbone.num_clusters
         ws = self._workspace(lib.advmil_adv_step_cluster_workspace_bytes(C.byref(gp), C.byref(dp), bags.rows, nb, ncl,
                                                                          self.precision), dev)
-        out = self._outputs(nb, dev)
+        out, lbuf = self._outputs(nb, dev)
         md = self._cat_masks(masks_d_fake, masks_d_real, ("fc1", "ga", "gs", "fc2"))
-        mg = {k: v.contiguous() for k, v in (masks_g or {}).items()}
         ca = _lib.ClusterStepArgs()
         a = ca.base
         a.gen, a.disc, a.gen_grads, a.disc_grads = C.pointer(gp), C.pointer(dp), C.pointer(gg), C.pointer(dg)
-        for k in ("h", "a", "b", "mlp0"):
-            setattr(a, "g_mask_" + k, ops._ptr(mg.get(k)))
+        fields = self._gen_fields(noise_g, mgs, ("h", "a", "b", "mlp0"))
+        for name, v in fields[0].items():
+            setattr(a, name, v)
         for k in ("fc1", "ga", "gs", "fc2"):
             setattr(a, "d_mask_" + k, ops._ptr(md.get(k)))
-        self._fill_args(a, bags, t, e, visible, noise_d, noise_g, counts, out, ws)
+        self._fill_args(a, bags, t, e, visible, noise_d, noise_g[0], counts, out, ws)
         ca.Wphi, ca.bphi, ca.dWphi, ca.dbphi = self.Wphi.data_ptr(), self.bphi.data_ptr(), self.dWphi.data_ptr(), self.dbphi.data_ptr()
         ca.cid, ca.num_clusters = cid.data_ptr(), ncl
-        return self._update(lib, "advmil_adv_step_cluster_disc", "advmil_adv_step_cluster_gen", ca, out, nb, counts[0],
-                            (t, e, visible, noise_d, noise_g, md, mg, cid, bags))
+        return self._update(lib, "advmil_adv_step_cluster_disc", "advmil_adv_step_cluster_gen", ca, a, fields, out, lbuf, nb, counts[0],
+                            (t, e, visible, noise_d, noise_g, md, mgs, cid, bags))
 
 
 class ModuleAdvStep(_DataParallelMixin):
-    """One D update + one G update over packed bags for any built generator backbone (ABMIL, DeepAttMISL, ESAT), composed from
+    """One D update + `gen_updates` G updates over packed bags for any built generator backbone (ABMIL, DeepAttMISL, ESAT), composed from
     the modules' packed forwards and their autograd Functions: the same step semantics as `AdvStep`
     (model/model_handler.py:349-498; global-count loss normalisation, flat parameter buffers, one all-reduce and one fused
     Adam launch per network, L1 and weight decay inside the Adam kernel) without the ABMIL-specific cross-phase sharing
     of `advmil_adv_step_disc/gen`.  Used for `bcb_mode: patch`; `AdvStep` remains the path for the ABMIL benchmark."""
 
     def __init__(self, netG, netD, lr_g=8e-5, lr_d=8e-5, weight_decay_g=5e-4, coef_gan=0.004, coef_l1=1e-5, loss_d="bce",
-                 recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32", process_group=None):
+                 recon_norm="l1", recon_alpha=0.0, recon_gamma=0.0, precision="fp32", process_group=None, gen_updates=1):
         assert recon_norm in ("l1", "l2"), recon_norm          # loss/utils.py:21-41
+        self._init_gen_updates(gen_updates)
         self.recon_norm = recon_norm
         self.netG, self.netD = netG, netD
         self.gparams = [p for p in netG.parameters()]
@@ -496,8 +548,9 @@ class ModuleAdvStep(_DataParallelMixin):
             n_real, n_fake, n_vis = [float(v) for v in cnt.tolist()]
         else:
             n_real, n_fake, n_vis = [float(v) for v in global_counts]
+        noise_g, masks_g = self._per_update(noise_g, "noise_g"), self._per_update(masks_g, "masks_g")
         nz_d = [None, noise_d if noise_d is not None else self._draw(nb, dev)]
-        nz_g = [None, noise_g if noise_g is not None else self._draw(nb, dev)]
+        nz_g = [[None, n if n is not None else self._draw(nb, dev)] for n in noise_g]
         # ---------------- D step: D.train / G.eval (model_handler.py:355-356) ----------------
         self._set_training(self._dmods, True)
         self._set_training(self._gmods, False)
@@ -517,36 +570,44 @@ class ModuleAdvStep(_DataParallelMixin):
         dis_loss.backward()
         self._allreduce(self.D.grad)
         self.D.adam(self.lr_d)
-        # ---------------- G step: D.eval / G.train (model_handler.py:432-433) ----------------
+        # ---------------- G steps: D.eval / G.train (model_handler.py:432-433), gen_updates times ----------------
         self._set_training(self._dmods, False)
         self._set_training(self._gmods, True)
-        self.G.grad.zero_()
         for p in self.dparams:
             p.requires_grad_(False)         # D only hands dL/dt back to G
+        gen_losses = []
         try:
-            G._inject_masks = masks_g
-            pred_g = self._generate(bags, nz_g, ext, coord, reuse=shared)
-            f_g = D.forward_packed(bags, pred_g).reshape(-1)
-            gen_loss = -f_g.sum() / n_fake                                        # fake_generator_loss (loss/utils.py:205-208)
-            pg = pred_g.reshape(-1)
-            lo = e * torch.abs(pg - t)                                            # recon_loss (loss/utils.py:21-41)
-            lc = (1.0 - e) * torch.relu(self.recon_gamma - (pg - t))
-            if self.recon_norm == "l2":
-                lo, lc = lo * lo, lc * lc
-            t_reg = (vis.float() * ((1.0 - self.recon_alpha) * (lo + lc) + self.recon_alpha * lo)).sum() / max(n_vis, 1.0)
-            total = t_reg + self.coef_gan * gen_loss
-            total.backward()
+            for u in range(self.gen_updates):
+                self.G.grad.zero_()
+                G._inject_masks = masks_g[u]
+                pred_g = self._generate(bags, nz_g[u], ext, coord, reuse=shared if u == 0 else None)
+                shared = sink = None        # the patch embedding of the D step's pass serves the first update only
+                f_g = D.forward_packed(bags, pred_g).reshape(-1)
+                gen_loss = -f_g.sum() / n_fake                                    # fake_generator_loss (loss/utils.py:205-208)
+                pg = pred_g.reshape(-1)
+                lo = e * torch.abs(pg - t)                                        # recon_loss (loss/utils.py:21-41)
+                lc = (1.0 - e) * torch.relu(self.recon_gamma - (pg - t))
+                if self.recon_norm == "l2":
+                    lo, lc = lo * lo, lc * lc
+                t_reg = (vis.float() * ((1.0 - self.recon_alpha) * (lo + lc) + self.recon_alpha * lo)).sum() / max(n_vis, 1.0)
+                total = t_reg + self.coef_gan * gen_loss
+                total.backward()
+                self._allreduce(self.G.grad)
+                l1 = self.G.flat.abs().sum() if self.coef_l1 > 1e-8 else None    # value only; its gradient is in the Adam kernel
+                self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
+                gen_losses.append((t_reg.detach(), gen_loss.detach(), total.detach(), l1))
         finally:
             for p in self.dparams:
                 p.requires_grad_(True)
-        shared = sink = None                # do not keep the step's activations alive
-        self._allreduce(self.G.grad)
-        l1 = self.G.flat.abs().sum() if self.coef_l1 > 1e-8 else None             # value only; its gradient is in the Adam kernel
-        self.G.adam(self.lr_g, weight_decay=self.wd_g, l1_coef=self.coef_l1 if self.coef_l1 > 1e-8 else 0.0)
-        return {"dis_loss": dis_loss.detach(), "gen_loss": gen_loss.detach(), "t_reg_loss": t_reg.detach(),
-                "gen_total_loss": total.detach() + (self.coef_l1 * l1 if l1 is not None else 0.0),
-                "pred_d": pred_d.reshape(-1), "pred_g": pred_g.detach().reshape(-1), "f_fake_d": f_fake.detach(),
-                "f_real": None if f_real is None else f_real.detach(), "f_fake_g": f_g.detach()}
+        t_reg, gen_loss, total, l1 = gen_losses[-1]
+        out = {"dis_loss": dis_loss.detach(), "gen_loss": gen_loss, "t_reg_loss": t_reg,
+               "gen_total_loss": total + (self.coef_l1 * l1 if l1 is not None else 0.0),
+               "pred_d": pred_d.reshape(-1), "pred_g": pred_g.detach().reshape(-1), "f_fake_d": f_fake.detach(),
+               "f_real": None if f_real is None else f_real.detach(), "f_fake_g": f_g.detach()}
+        if self.gen_updates > 1:      # as in AdvStep: [gen_updates, 4] t_reg, gen, t_reg + coef_gan * gen, sum|W_G|
+            out["gen_losses"] = torch.stack([torch.stack([a, b, c, torch.zeros_like(c) if d is None else d])
+                                             for a, b, c, d in gen_losses])
+        return out
 
 
 @torch.no_grad()

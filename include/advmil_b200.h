@@ -343,7 +343,11 @@ ADVMIL_API int advmil_cindex_counts_f64(const double* t, const double* e, const 
  *      region embedding; D loss (loss/utils.py:182-203) with GLOBAL pair counts; writes all 24 D gradients.
  *  advmil_adv_step_gen:  D.eval / G.train (:432-433), D already updated by the caller.  Re-uses the eval projection of the
  *      disc phase (kept in the workspace: call both phases with the SAME workspace), new dropout draw; G loss = recon +
- *      coef_gan * (-mean f_fake) (:478-484; the L1 term lives in advmil_adam_step); writes all 14 G gradients.          */
+ *      coef_gan * (-mean f_fake) (:478-484; the L1 term lives in advmil_adam_step); writes all 14 G gradients.
+ *  advmil_adv_step_gen_next: one more G update of the same step (gen_updates > 1, model_handler.py:328-335), called after
+ *      advmil_adv_step_gen and the caller's G Adam step, on the same workspace.  The caller sets that update's noise_g,
+ *      seed_g, g_mask_*, pred_g, f_fake_g and losses.  K1 is recomputed from G's current parameters; D's region embedding
+ *      of x is read back from the workspace (advmil_adv_step_gen left it there: D does not change between G updates).   */
 typedef struct AdvmilStepArgs {
   const AdvmilGenParams* gen; const AdvmilDiscParams* disc;
   AdvmilGenGrads* gen_grads; AdvmilDiscGrads* disc_grads;
@@ -373,6 +377,7 @@ ADVMIL_API size_t advmil_adv_step_workspace_bytes(const AdvmilGenParams* gen, co
                                        int32_t bags, int32_t precision);
 ADVMIL_API int advmil_adv_step_disc(const AdvmilStepArgs* a, void* stream);
 ADVMIL_API int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream);
+ADVMIL_API int advmil_adv_step_gen_next(const AdvmilStepArgs* a, void* stream);
 
 /* ---- the same two-phase step for the DeepAttMISL generator (bcb_mode `cluster`, model/backbone.py:89-123) with the RLIP
  *      discriminator.  The disc phase runs K9 (advmil_cluster_pool_fwd) once and keeps hc, counts and the ReLU keep bits in
@@ -384,7 +389,9 @@ ADVMIL_API int advmil_adv_step_gen(const AdvmilStepArgs* a, void* stream);
  *      single tcgen05 pass in ADVMIL_TF32 / _TF32X3 / _BF16 wherever that pass covers the shape; elsewhere (ADVMIL_FP32,
  *      and fp32 features with fewer than 128 rows) the step composes advmil_linear_fwd and advmil_segment_mean_by_id_fwd,
  *      reported under the ADVMIL_PROF_PROJ tag instead of the K9 tag.  Every bag length a
- *      multiple of 16, 1 <= num_clusters <= 16, noise0 == 0, ksize-1 discriminator: else ADVMIL_ERR_INVALID. */
+ *      multiple of 16, 1 <= num_clusters <= 16, noise0 == 0, ksize-1 discriminator: else ADVMIL_ERR_INVALID.
+ *      advmil_adv_step_cluster_gen_next: one more G update, as advmil_adv_step_gen_next; it runs K9 again from the updated
+ *      Wphi / bphi (rewriting hc, the counts and the keep bits in the workspace). */
 typedef struct AdvmilClusterStepArgs {
   AdvmilStepArgs base;
   const float *Wphi, *bphi;            /* backbone.phis.0 [h, C(,1,1)], [h] */
@@ -396,6 +403,7 @@ ADVMIL_API size_t advmil_adv_step_cluster_workspace_bytes(const AdvmilGenParams*
                                                           int32_t bags, int32_t num_clusters, int32_t precision);
 ADVMIL_API int advmil_adv_step_cluster_disc(const AdvmilClusterStepArgs* a, void* stream);
 ADVMIL_API int advmil_adv_step_cluster_gen(const AdvmilClusterStepArgs* a, void* stream);
+ADVMIL_API int advmil_adv_step_cluster_gen_next(const AdvmilClusterStepArgs* a, void* stream);
 
 /* ---- ESAT backbone: DualTrans_HS (model/backbone.py:171-196) as load_backbone('patch', dims) builds it (:31-35):
  *      AVGPoolPatchEmbedding(C -> d, scale 4, ksize 1; model/backbone_utils.py:129-168) -> optional sincos positional
@@ -472,7 +480,8 @@ ADVMIL_API int advmil_sincos_pe(const int64_t* coord, const int32_t* offsets /* 
 /* ---- the fused adversarial step for the ESAT generator (the launch sequence of step.ModuleAdvStep issued from C; same
  *      semantics, outputs and loss layout as advmil_adv_step_disc / _gen; in-kernel dropout only).  pe: optional [R, d]
  *      positional embedding (advmil_sincos_pe).  The two calls share one workspace: the D phase's eval pass leaves the patch
- *      embedding of the bags in it for the G phase's train pass. */
+ *      embedding of the bags in it for the G phase's train pass.  advmil_adv_step_esat_gen_next: one more G update, as
+ *      advmil_adv_step_gen_next; it recomputes the patch embedding from the updated parameters. */
 typedef struct AdvmilEsatStepArgs {
   const AdvmilEsatParams* esat; const AdvmilGenParams* head; const AdvmilDiscParams* disc;
   AdvmilEsatGrads* esat_grads; AdvmilGenGrads* head_grads; AdvmilDiscGrads* disc_grads;
@@ -492,6 +501,7 @@ ADVMIL_API size_t advmil_adv_step_esat_workspace_bytes(const AdvmilEsatParams* e
                                             int32_t rows, int32_t bags, int32_t precision);
 ADVMIL_API int advmil_adv_step_esat_disc(const AdvmilEsatStepArgs* a, void* stream);
 ADVMIL_API int advmil_adv_step_esat_gen(const AdvmilEsatStepArgs* a, void* stream);
+ADVMIL_API int advmil_adv_step_esat_gen_next(const AdvmilEsatStepArgs* a, void* stream);
 
 /* ---- ESAT self-attention, stage level (nn.MultiheadAttention inside the encoder layer, model/backbone_utils.py:112-127):
  *      qkv [R, 3d] fp32 (the packed in-projection), region offsets [bags+1] on the device and on the host, -> ctx [R, d],
