@@ -662,6 +662,9 @@ __global__ void __launch_bounds__(1024) abs_sum_kernel(const float* __restrict__
 // K9: DeepAttMISL cluster pooling (model/backbone.py:105-117): per (bag, cluster) mean of rows
 // =============================================================================================
 constexpr int CL_CH = 128;
+constexpr int CL_MAX = 64;                            // most clusters per bag
+// the partial kernel's static shared memory (cnt_s, cid_s): it counts against the 48 KB a block may use without opting in
+constexpr size_t SEG_MEAN_STATIC_SMEM = (CL_MAX + CL_CH) * sizeof(int);
 template <typename T>
 __global__ void __launch_bounds__(256) seg_mean_id_partial_kernel(const T* __restrict__ v,
                                                                   const int32_t* __restrict__ cid,
@@ -670,7 +673,7 @@ __global__ void __launch_bounds__(256) seg_mean_id_partial_kernel(const T* __res
                                                                   int32_t* __restrict__ part_cnt) {
   pdl_prologue();
   extern __shared__ float sm[];  // [ncl][width] sums
-  __shared__ int cnt_s[64];
+  __shared__ int cnt_s[CL_MAX];
   __shared__ int cid_s[CL_CH];
   int b = blockIdx.y, chunk = blockIdx.x;
   int beg = offsets[b] + chunk * CL_CH, end = min(offsets[b + 1], beg + CL_CH);
@@ -812,7 +815,7 @@ extern "C" int advmil_segment_mean_by_id_fwd(const void* v, int32_t elem, const 
                                              const int32_t* offsets_host, int32_t rows, int32_t bags, int32_t width,
                                              int32_t num_clusters, float* out, int32_t* counts, void* workspace,
                                              size_t workspace_bytes, void* stream) {
-  ADVMIL_REQUIRE(num_clusters > 0 && num_clusters <= 64 && width > 0, "segment_mean_by_id: bad arguments");
+  ADVMIL_REQUIRE(num_clusters > 0 && num_clusters <= CL_MAX && width > 0, "segment_mean_by_id: bad arguments");
   ADVMIL_REQUIRE((size_t)num_clusters * width * sizeof(float) <= 96 * 1024, "segment_mean_by_id: clusters*width too large");
   cudaStream_t st = (cudaStream_t)stream;
   size_t nparts = (size_t)rows / CL_CH + bags + 1;
@@ -824,7 +827,7 @@ extern "C" int advmil_segment_mean_by_id_fwd(const void* v, int32_t elem, const 
   for (int b = 0; b < bags; ++b) maxlen = max(maxlen, offsets_host[b + 1] - offsets_host[b]);
   int maxchunks = max(1, cdiv(maxlen, CL_CH));
   size_t smem = (size_t)num_clusters * width * sizeof(float);
-  if (smem > 48 * 1024) {
+  if (smem + SEG_MEAN_STATIC_SMEM > 48 * 1024) {
     ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(seg_mean_id_partial_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ADVMIL_CHECK_CUDA(cudaFuncSetAttribute(seg_mean_id_partial_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   }
